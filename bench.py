@@ -6,10 +6,14 @@
 
 A "step" is one env step of the whole batch: BASELINE.json configs[1] — cooperative
 navigation, 3 agents, 16384 envs per GPU, random discrete actions — in the production
-precision (fp32).  `value` is device-resident throughput (actions already in HBM, outputs
-written to a rotating 25-slot rollout buffer larger than L2, 25 steps per CUDA-graph
-launch).  `e2e` is the same metric through the numpy-facing drop-in (`GraphVecEnv.step`):
+precision (fp32).  `value` is device-resident throughput over exactly K timed steps (actions
+already in HBM, outputs written to a rotating 25-slot rollout buffer larger than L2, 25 steps
+per fused launch).  `e2e` is the same metric through the numpy-facing drop-in (`GraphVecEnv.step`):
 host actions in, host outputs out, both copies inside the timed region.
+
+`--dump-outputs DIR` writes what the last timed step computed (the nine outputs of rank 0's envs)
+as DIR/<name>.npy.  The inputs are seeded and the warm-up and timed steps run from the reset state,
+so two builds run with the same arguments can be compared output for output.
 
 IMPORTANT LABEL: the GS-MARL env sources are withheld (reference readme.md:1), so the
 model is the declared one of SPEC.md with the UNVERIFIED constants of
@@ -141,6 +145,33 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(outputs, out_dir, limit=DUMP_LIMIT_BYTES):
+    """Write each output (leading dimension: envs) as out_dir/<name>.npy: real outputs in their own
+    precision, integer ones as float64 (exact; adj as its unsigned bit masks).  If all of them would
+    take more than `limit` bytes, every file holds the same fixed, seeded sample of env rows, and
+    env_index.npy says which."""
+    import numpy as np
+    arrays = {}
+    for k, v in outputs.items():
+        a = v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v)
+        if k == "adj":
+            a = a.view(np.uint32)
+        arrays[k] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    n_envs = len(next(iter(arrays.values())))
+    per_env = sum(a.nbytes for a in arrays.values()) // n_envs
+    if per_env * n_envs > limit:
+        keep = (limit - 4096 * (len(arrays) + 1)) // (per_env + 8)      # room for the .npy headers and the index
+        idx = np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def ncu_traffic():
@@ -327,7 +358,7 @@ def run_gpu(args):
     ring_bytes = sum(v.numel() * v.element_size() for v in ring.values())
 
     import ctypes as C
-    from bench_util import RolloutRegion, time_rollouts
+    from bench_util import GRAPH_CHUNK_STEPS, RolloutRegion, time_rollouts
     from gs_marl_b200.environment import StreamShardedEnv
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     # The timed region drives S contiguous sub-shards of this GPU's envs, each its own handle on
@@ -336,32 +367,38 @@ def run_gpu(args):
     S = max(1, args.streams)
     sh_env = StreamShardedEnv(cfg, args.envs, n_streams=S, device=local, env_offset=rank * args.envs, seed=1)
     sh_env.reset()
+    start_state, start_episode = sh_env.get_state(), sh_env.get_episode()
 
-    # ---- THE timed region: K env steps = fused T-step launches on the S shard streams, captured in
-    # ONE CUDA graph (fork / join inside) and replayed `repeats` times back to back so that the
-    # region lasts >= --region-ms whatever K is; envs are re-drawn in-kernel every EPISODE_LEN
+    # ---- THE timed region: exactly K env steps = fused T-step launches on the S shard streams,
+    # captured in a CUDA graph (fork / join inside); envs are re-drawn in-kernel every EPISODE_LEN
     # steps (state and episode counters persist across replays); all nine outputs are written.
-    region = RolloutRegion(sh_env, acts, ring, K, T, auto_reset=True)
-    warm_units = max(1, -(-max(W, 3) // (region.regions_per_unit * K)))
-    for _ in range(warm_units):
+    region = RolloutRegion(sh_env, acts, ring, K, T, auto_reset=True, pack=False)
+    # untimed pre-run: loads the modules and brings the clocks up.  The clock sampler was started
+    # first thing in this function; on a busy host (8 ranks, 8 nvidia-smi processes) its first sample
+    # can take seconds: keep the GPU under load until it reports (bounded)
+    for _ in range(max(1, GRAPH_CHUNK_STEPS // K)):
         region.replay_unit()
     torch.cuda.synchronize()
-    # the clock sampler was started first thing in this function; on a busy host (8 ranks, 8 nvidia-smi
-    # processes) its first sample can take seconds: keep the GPU under load until it reports (bounded)
     t_wait = time.time()
     while not sampler.lines and time.time() - t_wait < 15.0:
         region.replay_unit()
         torch.cuda.synchronize()
-    units = torch.tensor([region.calibrate(args.region_ms)], dtype=torch.int64, device=dev)
-    if world > 1:
-        dist.all_reduce(units, op=dist.ReduceOp.MAX)           # every rank runs the same work
-    units = int(units.item())
+    # the pre-run ran for a time-dependent number of steps: start again from the reset state, so that
+    # every run computes the same steps (--dump-outputs compares builds output for output)
+    sh_env.set_state(*start_state)
+    sh_env.set_episode(start_episode)
     barrier()
     wall0 = time.time()
-    ms, repeats = region.run(units)
+    # warm-up: ceil(max(W, 256) / K) replays of the K-step region, enqueued right before the timed one so
+    # that the GPU is still busy with them when the first event is recorded (no launch gap inside the events)
+    for _ in range(-(-max(W, 256) // K)):
+        region.replay_unit()
+    ms, repeats = region.run(1)
     barrier()
     wall1 = time.time()
     clocks = sampler.stop(wall0, wall1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs({k: ring[k][region.last_slot] for k in sh_env.OUTPUTS}, args.dump_outputs)
     launches = repeats * region.launches_per_region
     bytes_region = region.bytes_per_region(cfg)
 
@@ -481,8 +518,8 @@ def run_gpu(args):
         peak, peak_src = measured_peak()
         achieved = bytes_region * repeats / (ms * 1e-3) / 1e9
         per_step_bytes = cfg.bytes_per_agent_step() * agents     # state r/w charged every step (r1 accounting)
-        region_desc = (f"{region.copies} K-step region(s) per CUDA graph" if K <= 2500 else
-                       "CUDA graphs of 2500-step chunks")
+        region_desc = ("one CUDA graph" if K <= GRAPH_CHUNK_STEPS else
+                       f"CUDA graphs of {GRAPH_CHUNK_STEPS}-step chunks")
 
         def variant(r):
             return {"step_us": r["step_us"], "achieved": r["achieved"], "frac": r["achieved"] / peak}
@@ -500,10 +537,10 @@ def run_gpu(args):
                 "launch": f"fused launches of min({T}, remaining) steps (gsm_rollout); {S} contiguous env sub-shards of "
                           f"{args.envs // S} envs, one handle + one CUDA stream each, all writing the same rollout "
                           f"buffer (gsm_set_slot_envs)",
-                "timed_region": f"the K = {K}-step region is captured in a CUDA graph ({region_desc}; shard streams fork "
-                                f"and join inside the graph) and replayed back to back: repeats = {repeats} regions in "
-                                f"{ms:.1f} ms between two CUDA events; ms_per_step = region time / (repeats * K); no "
-                                "host launch inside the events",
+                "timed_region": f"exactly K = {K} steps, captured in {region_desc} (shard streams fork and join inside "
+                                f"the graph) and replayed once between two CUDA events, right behind the warm-up "
+                                f"(ceil(max(W, 256) / K) replays from the reset state): {ms:.3f} ms; ms_per_step = "
+                                "region time / K; no host launch inside the events",
                 "streams": S},
             "env_steps_per_s": value / N_AGENTS,
             "clocks": clocks,
@@ -793,8 +830,10 @@ def closed_loop(env, cfg, n_steps, dev):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100000)
+    ap.add_argument("--steps", type=int, default=100000, help="env steps in the timed region")
     ap.add_argument("--warmup", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0's envs) as DIR/<name>.npy")
     ap.add_argument("--large-envs", type=int, default=1048576,
                     help="extra roofline line at a GPU-saturating env count (0 = skip)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -807,7 +846,8 @@ def main():
     ap.add_argument("--collect-streams", type=int, default=1,
                     help="env sub-shards (streams) of the fused closed loop: one shard's actor overlaps another's env step")
     ap.add_argument("--region-ms", type=float, default=300.0,
-                    help="minimum length of the timed region: the K-step region is replayed until it lasts this long")
+                    help="minimum length of the side measurements (variants of the headline, large batch; "
+                         "capped at 60 ms): their K-step regions are replayed until they last this long")
     ap.add_argument("--configs", type=int, default=1, help="1: add the BASELINE configs[2..4] block to the line")
     ap.add_argument("--config-ms", type=float, default=60.0, help="timed length per entry of the configs block")
     ap.add_argument("--config5-steps", type=int, default=100)
@@ -815,7 +855,11 @@ def main():
     ap.add_argument("--ref-budget", type=float, default=90.0, help="(ignored: the reference arm always runs the full workload)")
     ap.add_argument("--no-cpu", action="store_true")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU arm's timed path")
         run_reference(args)
     else:
         run_gpu(args)

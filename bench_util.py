@@ -26,13 +26,14 @@ class RolloutRegion:
       head, join at its tail; consecutive launches of one shard are chained on its stream, shards
       are not joined in between),
     * K <= GRAPH_CHUNK_STEPS: the graph holds c = GRAPH_CHUNK_STEPS // K copies of the K-step
-      region (one replay = c regions); larger K: a GRAPH_CHUNK_STEPS graph replayed K // chunk
-      times plus one graph with the remainder.
+      region (one replay = c regions; c = 1 with pack=False, so that one unit is exactly K
+      steps); larger K: a GRAPH_CHUNK_STEPS graph replayed K // chunk times plus one graph with
+      the remainder.
     State persists across launches and replays, so with auto-reset on, every env is re-drawn
     in-kernel every `episode_length` steps whatever K and T are: no work is skipped.
     """
 
-    def __init__(self, env, acts, ring, K, T, auto_reset=True):
+    def __init__(self, env, acts, ring, K, T, auto_reset=True, pack=True):
         self.env, self.K, self.T = env, int(K), int(T)
         self.sharded = hasattr(env, "shards")
         self.dev = env.device
@@ -53,9 +54,10 @@ class RolloutRegion:
             self.launch_steps.append(m)
             d += m
         if self.K <= GRAPH_CHUNK_STEPS:
-            self.copies = max(1, GRAPH_CHUNK_STEPS // self.K)
+            self.copies = max(1, GRAPH_CHUNK_STEPS // self.K) if pack else 1
             self.plan = [(self._capture([self.K] * self.copies), 1)]      # (graph, replays per unit)
             self.regions_per_unit = self.copies
+            last_segment = self.K
         else:
             q, r = divmod(self.K, GRAPH_CHUNK_STEPS)
             self.copies = 1
@@ -63,6 +65,9 @@ class RolloutRegion:
             if r:
                 self.plan.append((self._capture([r]), 1))
             self.regions_per_unit = 1
+            last_segment = r or GRAPH_CHUNK_STEPS
+        # every fused launch writes ring slots 0, 1, ...: the last step of a unit lands here
+        self.last_slot = (last_segment - 1) % self.T
 
     def _enqueue(self, n_steps, streams):
         done = 0
