@@ -84,6 +84,22 @@ class GsmPolicyIO(C.Structure):
     ]
 
 
+class GsmPolicyEvalIO(C.Structure):
+    """gsm_policy_eval_io: DEVICE pointers; `params` is the parameters_to_vector(actor) vector."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("n_actions", C.c_int32),
+        ("params", C.c_void_p), ("obs", C.c_void_p), ("nbr_feat", C.c_void_p), ("nbr_cnt", C.c_void_p),
+        ("actions", C.c_void_p), ("rows", C.c_void_p),
+        ("logp", C.c_void_p), ("entropy", C.c_void_p), ("values", C.c_void_p),
+        ("n_rows", C.c_int64), ("max_nbrs", C.c_int32), ("reserved", C.c_int32),
+    ]
+
+
+def policy_n_params(n_actions: int) -> int:
+    """GSM_POLICY_N_PARAMS: length of the learner's parameter vector."""
+    return 961 + 129 * n_actions + 2 * (2 * GSM_POLICY_HIDDEN + 1)
+
+
 _H = C.c_void_p  # gsm_env*
 _IO = C.POINTER(GsmStepIO)
 
@@ -117,6 +133,10 @@ SYMBOLS = {
                           C.c_void_p]),
     "gsm_policy_act": (C.c_int, [C.POINTER(GsmPolicyWeights), C.POINTER(GsmPolicyIO), C.c_int, C.c_void_p]),
     "gsm_policy_last_error": (C.c_char_p, []),
+    "gsm_policy_evaluate": (C.c_int, [C.POINTER(GsmPolicyEvalIO), C.c_int, C.c_void_p]),
+    "gsm_policy_backward_workspace": (C.c_int64, [C.c_int64, C.c_int32]),
+    "gsm_policy_backward": (C.c_int, [C.POINTER(GsmPolicyEvalIO), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gsm_gae": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int64,
                           C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gsm_collect": (C.c_int, [_H, C.POINTER(GsmPolicyWeights), C.c_int32, _IO, C.c_void_p, C.c_void_p,

@@ -302,6 +302,385 @@ __global__ void __launch_bounds__(256) gae_kernel(const __grid_constant__ GaePar
   }
 }
 
+// ---- learner pass (SPEC.md §12): evaluate_actions forward and backward -------------------------
+// The lineage's evaluate_actions (SOURCES.txt:8, withheld) over the declared actor: per row the
+// log-prob of a GIVEN action, the entropy of softmax(z) and the two critics, and the gradient of
+//   L = sum_i d_logp[i] logp[i] + d_entropy[i] entropy[i] + d_values[i] . values[i]
+// with respect to the parameter vector (torch parameters_to_vector order, a DEVICE vector that an
+// optimiser changes every step: it cannot travel in the parameter space like gsm_policy_weights, so
+// every block copies it to shared memory).
+//
+// Forward (policy_eval_kernel): thread per row, the operation order of graph_actor_kernel — the same
+// fmaf chains over j (FFMA2 halves are independent fma.rn, so scalar fmaf rounds identically), the
+// rows folded in row order through the same online softmax — so logp and values are bit-identical
+// to what gsm_policy_act / gsm_collect wrote.  One row per thread instead of the actor's flattened
+// row items: simpler, divergent on nbr_cnt, and the learner pass is not the collect loop's hot path.
+//
+// Backward (policy_backward_kernel), with h = [e; g], g = sum_r a_r m_r, Z = [z; v], W = [W_h; W_v]:
+//   dz = d_logp (onehot(a) - p) - d_entropy p o (log p + entropy),  dZ = [dz; d_values]
+//   dh = W^T dZ;  dW += dZ h^T;  de = dh[:H] o [e > 0];  dg = dh[H:]
+//   m_r . dg = dZ . hr_r with hr_r = W[:, H:] m_r, so ds_r = a_r (dZ . hr_r - dZ . (sum_r a_r hr_r))
+//   needs no H-vector; dm_r = a_r dg + ds_r w_a;  du_r = dm_r o [u_r > 0]
+//   dW_n += du_r f_r^T;  db_n += du_r;  dw_a += ds_r m_r;  db_a += ds_r;  dW_e += de obs^T;  db_e += de.
+// A block owns AG = 64 rows per tile.  Phase A, thread per row: the forward (first pass over the
+// rows), dZ, then a second pass over the rows recomputing (t_r, hr_r) to get a_r and ds_r, parked in
+// shared memory (8 B per valid row) — nothing of size H per neighbour row is stored anywhere.
+// Phase B, thread per HIDDEN UNIT j: loops over the tile's rows in order, recomputes e_j and u_rj from
+// obs and f_r (broadcast reads) and accumulates every gradient entry of unit j in registers
+// (dW_e[j], db_e[j], dW_n[j], db_n[j], dw_a[j], W[:, j], W[:, H + j]); the NZ + 1 bias sums ride on
+// threads 0..NZ-1 and H-1.  Each thread owns distinct entries, so there is no atomic: a block walks
+// tiles blockIdx, blockIdx + G, ... in order and writes ONE partial vector to the workspace;
+// policy_grad_reduce_kernel sums the G partials in a fixed order.  G = min(tiles, BWD_MAX_BLOCKS)
+// depends on n_rows only, so grad is bit-identical across calls, streams and B200s.
+constexpr int V2 = GSM_POLICY_VALUE_HEADS;
+constexpr int BWD_AG = 64;                 // rows per tile = threads per backward block (= H)
+constexpr int BWD_MAX_BLOCKS = 148 * 6;    // one wave at 6 blocks/SM (168 registers); a constant, NOT the device's SM count
+static_assert(BWD_AG == H, "phase B maps one thread to one hidden unit");
+
+template <int NA> struct PV {               // offsets into the parameter vector
+  static constexpr int EW = 0, EB = EW + H * GSM_OBS_DIM, NW = EB + H, NB = NW + H * GSM_NBR_FEAT_DIM,
+                       AW = NB + H, AB = AW + H, HW = AB + 1, HB = HW + NA * 2 * H, VW = HB + NA,
+                       VB = VW + V2 * 2 * H, N = VB + V2;
+  static __host__ __device__ constexpr int row(int a) { return a < NA ? HW + a * 2 * H : VW + (a - NA) * 2 * H; }
+  static __host__ __device__ constexpr int bias(int a) { return a < NA ? HB + a : VB + (a - NA); }
+};
+static_assert(PV<5>::N == GSM_POLICY_N_PARAMS(5) && PV<5>::N == 1864 && PV<9>::N == 2380, "vector size");
+
+struct EvalArgs {
+  const float* params; const float* obs; const float* nbr_feat; const int32_t* nbr_cnt;
+  const int32_t* actions; const int64_t* rows;
+  float* logp; float* entropy; float* values;                 // forward outputs
+  const float* d_logp; const float* d_entropy; const float* d_values;   // backward inputs
+  float* ws;                                                  // backward: [gridDim.x][N] partials
+  int64_t n_rows, n_tiles;
+  int K;
+};
+
+// e-branch of graph_actor_kernel: z[a] = b[a] + sum_j W[a][j] relu(W_e obs + b_e)_j, same chains
+template <int NA>
+__device__ __forceinline__ void ego_logits(const float* W, const float* o, float (&z)[NA + V2]) {
+  using P = PV<NA>;
+  const float o0 = o[0], o1 = o[1], o2 = o[2], o3 = o[3], o4 = o[4], o5 = o[5];
+#pragma unroll
+  for (int a = 0; a < NA + V2; a++) z[a] = W[P::bias(a)];
+#pragma unroll
+  for (int j = 0; j < H; j++) {
+    const float* we = W + P::EW + j * GSM_OBS_DIM;
+    float e = W[P::EB + j];
+    e = fmaf(we[0], o0, e); e = fmaf(we[1], o1, e); e = fmaf(we[2], o2, e);
+    e = fmaf(we[3], o3, e); e = fmaf(we[4], o4, e); e = fmaf(we[5], o5, e);
+    e = fmaxf(e, 0.f);
+#pragma unroll
+    for (int a = 0; a < NA + V2; a++) z[a] = fmaf(W[P::row(a) + j], e, z[a]);
+  }
+}
+
+// one valid neighbour row: returns the attention score t_r, hr[a] = W[a][H:] . m_r (phase 2 chains)
+template <int NA>
+__device__ __forceinline__ float nbr_row(const float* W, const float* f, float (&hr)[NA + V2]) {
+  using P = PV<NA>;
+  // an offset the compiler cannot see through: without it the ~1200 shared-memory weight loads are
+  // hoisted out of the caller's row loop as loop invariants and spilled to local memory
+  int off = 0;
+  asm volatile("" : "+r"(off));
+  W += off;
+  const float f0 = f[0], f1 = f[1], f2 = f[2], f3 = f[3], f4 = f[4], f5 = f[5];
+  float t = W[P::AB];
+#pragma unroll
+  for (int a = 0; a < NA + V2; a++) hr[a] = 0.f;
+#pragma unroll
+  for (int j = 0; j < H; j++) {
+    const float* wn = W + P::NW + j * GSM_NBR_FEAT_DIM;
+    float m = W[P::NB + j];
+    m = fmaf(wn[0], f0, m); m = fmaf(wn[1], f1, m); m = fmaf(wn[2], f2, m);
+    m = fmaf(wn[3], f3, m); m = fmaf(wn[4], f4, m); m = fmaf(wn[5], f5, m);
+    m = fmaxf(m, 0.f);
+    t = fmaf(W[P::AW + j], m, t);
+#pragma unroll
+    for (int a = 0; a < NA + V2; a++) hr[a] = fmaf(W[P::row(a) + H + j], m, hr[a]);
+  }
+  return t;
+}
+
+// The forward of one row in graph_actor_kernel's order.  Out: z = [logits; values]; mx, s: the
+// softmax max and sum over the valid rows; acc[a] * (1 / s) = sum_r a_r hr_r[a] (cnt > 0).
+template <int NA>
+__device__ __forceinline__ void row_forward(const float* W, const float* o, const float* f, int cnt,
+                                            float (&z)[NA + V2], float (&acc)[NA + V2], float& mx, float& s) {
+  ego_logits<NA>(W, o, z);
+  mx = -__int_as_float(0x7f800000); s = 0.f;
+#pragma unroll
+  for (int a = 0; a < NA + V2; a++) acc[a] = 0.f;
+  for (int r = 0; r < cnt; r++) {
+    float hr[NA + V2];
+    const float t = nbr_row<NA>(W, f + r * GSM_NBR_FEAT_DIM, hr);
+    const float nm = fmaxf(mx, t);
+    const float sc = expf(mx - nm), pw = expf(t - nm);     // first row: exp(-inf) = 0
+    s = fmaf(s, sc, pw);
+#pragma unroll
+    for (int a = 0; a < NA + V2; a++) acc[a] = fmaf(acc[a], sc, pw * hr[a]);
+    mx = nm;
+  }
+  if (cnt > 0) {
+    const float inv = 1.f / s;
+#pragma unroll
+    for (int a = 0; a < NA + V2; a++) z[a] = fmaf(acc[a], inv, z[a]);
+  }
+}
+
+// logp of action `act` exactly as graph_actor_kernel computes it (NaN for act outside [0, NA));
+// zm, se: max and sum of exp(z - zm) over the logits.
+template <int NA>
+__device__ __forceinline__ float row_logp(const float (&z)[NA + V2], int act, float& zm, float& se) {
+  zm = z[0];
+#pragma unroll
+  for (int a = 1; a < NA; a++) zm = fmaxf(zm, z[a]);
+  se = 0.f;
+#pragma unroll
+  for (int a = 0; a < NA; a++) se += expf(z[a] - zm);
+  float za = __int_as_float(0x7fc00000);
+#pragma unroll
+  for (int a = 0; a < NA; a++) if (act == a) za = z[a];
+  return za - zm - logf(se);
+}
+
+__device__ __forceinline__ int clamp_cnt(int c, int K) { return c < 0 ? 0 : (c > K ? K : c); }
+
+template <int NA>
+__global__ void __launch_bounds__(128) policy_eval_kernel(const __grid_constant__ EvalArgs p) {
+  constexpr int NP = PV<NA>::N;
+  __shared__ float s_w[NP];
+  for (int k = threadIdx.x; k < NP; k += blockDim.x) s_w[k] = p.params[k];
+  __syncthreads();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.n_rows) return;
+  const int64_t src = p.rows ? p.rows[i] : i;
+  const int cnt = clamp_cnt(p.nbr_cnt[src], p.K);
+  float z[NA + V2], acc[NA + V2], mx, s;
+  row_forward<NA>(s_w, p.obs + src * GSM_OBS_DIM, p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM, cnt, z, acc, mx, s);
+  if (p.values) {
+#pragma unroll
+    for (int v = 0; v < V2; v++) p.values[i * V2 + v] = z[NA + v];
+  }
+  float zm, se;
+  const float lp = row_logp<NA>(z, p.actions[src], zm, se);
+  if (p.logp) p.logp[i] = lp;
+  if (p.entropy) {                     // log(se) - sum_k p_k (z_k - zm) = logsumexp(z) - sum_k p_k z_k
+    const float inv = 1.f / se;
+    float pz = 0.f;
+#pragma unroll
+    for (int a = 0; a < NA; a++) pz = fmaf(expf(z[a] - zm) * inv, z[a] - zm, pz);
+    p.entropy[i] = logf(se) - pz;
+  }
+}
+
+template <int NA> struct BwdSmem {
+  float w[PV<NA>::N];
+  float obs[BWD_AG][GSM_OBS_DIM];
+  float dz[BWD_AG][NA + V2];
+  float dsum[BWD_AG];                  // sum_r ds_r of the row (db_a)
+  int cnt[BWD_AG];
+  long long src[BWD_AG];
+};
+
+template <int NA>
+__global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_constant__ EvalArgs p) {
+  constexpr int NZ = NA + V2, NP = PV<NA>::N;
+  using P = PV<NA>;
+  __shared__ BwdSmem<NA> sm;
+  extern __shared__ float s_rows[];    // [BWD_AG][K][2]: (a_r, ds_r) of the valid rows; a float2 array
+                                       // would round every kernel's static shared memory in this file up to 16 B
+  const int tid = threadIdx.x;
+  for (int k = tid; k < NP; k += BWD_AG) sm.w[k] = p.params[k];
+  const float* W = sm.w;
+  // phase-B accumulators of hidden unit j = tid, live across the tiles
+  float gwe[GSM_OBS_DIM], gwn[GSM_NBR_FEAT_DIM], ghe[NZ], ghg[NZ];
+  float gbe = 0.f, gbn = 0.f, gwa = 0.f, gsc = 0.f;   // gsc: bias sum of dZ[tid] (tid < NZ) or db_a (tid = H-1)
+#pragma unroll
+  for (int k = 0; k < GSM_OBS_DIM; k++) { gwe[k] = 0.f; gwn[k] = 0.f; }
+#pragma unroll
+  for (int a = 0; a < NZ; a++) { ghe[a] = 0.f; ghg[a] = 0.f; }
+  __syncthreads();
+
+  for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {   // block-uniform
+    const int64_t base = tile * BWD_AG;
+    const int nag = p.n_rows - base < BWD_AG ? (int)(p.n_rows - base) : BWD_AG;
+    // ---- phase A: thread = row ----
+    if (tid < nag) {
+      const int64_t i = base + tid;
+      const int64_t src = p.rows ? p.rows[i] : i;
+      const int cnt = clamp_cnt(p.nbr_cnt[src], p.K);
+      const float* o = p.obs + src * GSM_OBS_DIM;
+      const float* f = p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM;
+      float z[NZ], acc[NZ], mx, s;
+      row_forward<NA>(W, o, f, cnt, z, acc, mx, s);
+      float zm, se;
+      const int act = p.actions[src];
+      const float lp = row_logp<NA>(z, act, zm, se);
+      const float dlp = p.d_logp ? p.d_logp[i] : 0.f, dent = p.d_entropy ? p.d_entropy[i] : 0.f;
+      const float lse = zm + logf(se), inv_se = 1.f / se;
+      float pr[NA], ent = 0.f;
+#pragma unroll
+      for (int a = 0; a < NA; a++) { pr[a] = expf(z[a] - zm) * inv_se; ent = fmaf(pr[a], z[a] - zm, ent); }
+      ent = logf(se) - ent;
+      // an action outside [0, NA) has no one-hot: its NaN logp poisons the gradient it feeds
+      const float bad = (dlp != 0.f && lp != lp) ? __int_as_float(0x7fc00000) : 0.f;
+      float dz[NZ];
+#pragma unroll
+      for (int a = 0; a < NA; a++)
+        dz[a] = dlp * ((act == a ? 1.f : 0.f) - pr[a] + bad) - dent * pr[a] * ((z[a] - lse) + ent);
+#pragma unroll
+      for (int v = 0; v < V2; v++) dz[NA + v] = p.d_values ? p.d_values[i * V2 + v] : 0.f;
+      float dsum = 0.f;
+      if (cnt > 0) {
+        const float inv = 1.f / s;
+        float gdg = 0.f;                 // g . dg = dZ . sum_r a_r hr_r
+#pragma unroll
+        for (int a = 0; a < NZ; a++) gdg = fmaf(dz[a], acc[a] * inv, gdg);
+        float* pr_rows = s_rows + 2 * tid * p.K;
+        for (int r = 0; r < cnt; r++) {  // second pass: the same t_r, hr_r as the first
+          float hr[NZ];
+          const float t = nbr_row<NA>(W, f + r * GSM_NBR_FEAT_DIM, hr);
+          const float ar = expf(t - mx) * inv;
+          float q = 0.f;
+#pragma unroll
+          for (int a = 0; a < NZ; a++) q = fmaf(dz[a], hr[a], q);
+          const float ds = ar * (q - gdg);
+          pr_rows[2 * r] = ar; pr_rows[2 * r + 1] = ds;
+          dsum += ds;
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < GSM_OBS_DIM; k++) sm.obs[tid][k] = o[k];
+#pragma unroll
+      for (int a = 0; a < NZ; a++) sm.dz[tid][a] = dz[a];
+      sm.dsum[tid] = dsum;
+      sm.cnt[tid] = cnt;
+      sm.src[tid] = src;
+    }
+    __syncthreads();
+    // ---- phase B: thread = hidden unit j ----
+    {
+      const int j = tid;
+      float we[GSM_OBS_DIM], wn[GSM_NBR_FEAT_DIM], wh[NZ], wg[NZ];
+#pragma unroll
+      for (int k = 0; k < GSM_OBS_DIM; k++) { we[k] = W[P::EW + j * GSM_OBS_DIM + k]; wn[k] = W[P::NW + j * GSM_NBR_FEAT_DIM + k]; }
+#pragma unroll
+      for (int a = 0; a < NZ; a++) { wh[a] = W[P::row(a) + j]; wg[a] = W[P::row(a) + H + j]; }
+      const float be = W[P::EB + j], bn = W[P::NB + j], wa = W[P::AW + j];
+      for (int ag = 0; ag < nag; ag++) {
+        float dZ[NZ];
+#pragma unroll
+        for (int a = 0; a < NZ; a++) dZ[a] = sm.dz[ag][a];
+        float u = be;
+#pragma unroll
+        for (int k = 0; k < GSM_OBS_DIM; k++) u = fmaf(we[k], sm.obs[ag][k], u);
+        const float e = fmaxf(u, 0.f);
+        float dh = 0.f;
+#pragma unroll
+        for (int a = 0; a < NZ; a++) { dh = fmaf(wh[a], dZ[a], dh); ghe[a] = fmaf(dZ[a], e, ghe[a]); }
+        const float de = u > 0.f ? dh : 0.f;            // ReLU'(0) = 0, as in torch
+#pragma unroll
+        for (int k = 0; k < GSM_OBS_DIM; k++) gwe[k] = fmaf(de, sm.obs[ag][k], gwe[k]);
+        gbe += de;
+        const int c = sm.cnt[ag];                        // block-uniform: no divergence
+        if (c > 0) {
+          float dg = 0.f, g = 0.f;
+#pragma unroll
+          for (int a = 0; a < NZ; a++) dg = fmaf(wg[a], dZ[a], dg);
+          const float* f = p.nbr_feat + sm.src[ag] * p.K * GSM_NBR_FEAT_DIM;
+          const float* rr = s_rows + 2 * ag * p.K;
+          for (int r = 0; r < c; r++) {
+            float fr[GSM_NBR_FEAT_DIM];
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) fr[k] = __ldg(f + r * GSM_NBR_FEAT_DIM + k);
+            float um = bn;
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) um = fmaf(wn[k], fr[k], um);
+            const float m = fmaxf(um, 0.f);
+            const float ar = rr[2 * r], ds = rr[2 * r + 1];
+            g = fmaf(ar, m, g);
+            const float du = um > 0.f ? fmaf(ar, dg, ds * wa) : 0.f;
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) gwn[k] = fmaf(du, fr[k], gwn[k]);
+            gbn += du;
+            gwa = fmaf(ds, m, gwa);
+          }
+#pragma unroll
+          for (int a = 0; a < NZ; a++) ghg[a] = fmaf(dZ[a], g, ghg[a]);
+        }
+        if (j < NZ) gsc += sm.dz[ag][j];
+        else if (j == H - 1) gsc += sm.dsum[ag];
+      }
+    }
+    __syncthreads();                     // before the next tile overwrites the row state
+  }
+  // ---- this block's partial gradient, in vector order ----
+  float* out = p.ws + (int64_t)blockIdx.x * NP;
+  const int j = tid;
+#pragma unroll
+  for (int k = 0; k < GSM_OBS_DIM; k++) {
+    out[P::EW + j * GSM_OBS_DIM + k] = gwe[k];
+    out[P::NW + j * GSM_NBR_FEAT_DIM + k] = gwn[k];
+  }
+  out[P::EB + j] = gbe; out[P::NB + j] = gbn; out[P::AW + j] = gwa;
+#pragma unroll
+  for (int a = 0; a < NZ; a++) { out[P::row(a) + j] = ghe[a]; out[P::row(a) + H + j] = ghg[a]; }
+  if (j < NZ) out[j < NA ? P::HB + j : P::VB + (j - NA)] = gsc;
+  else if (j == H - 1) out[P::AB] = gsc;
+}
+
+// grad[k] = sum of the G partials in a fixed order: warp w sums partials w, w + 8, ... (lane = k),
+// then warp 0 adds the 8 warp sums in order.
+__global__ void __launch_bounds__(256) policy_grad_reduce_kernel(const float* __restrict__ ws, int G, int NP,
+                                                                 float* __restrict__ grad) {
+  __shared__ float s[8][32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int k = blockIdx.x * 32 + lane;
+  float acc = 0.f;
+  if (k < NP) {
+#pragma unroll 4
+    for (int g = w; g < G; g += 8) acc += ws[(int64_t)g * NP + k];
+  }
+  s[w][lane] = acc;
+  __syncthreads();
+  if (w == 0 && k < NP) {
+    float t = s[0][lane];
+#pragma unroll
+    for (int q = 1; q < 8; q++) t += s[q][lane];
+    grad[k] = t;
+  }
+}
+
+static int64_t bwd_blocks(int64_t n_rows) {
+  const int64_t tiles = (n_rows + BWD_AG - 1) / BWD_AG;
+  return tiles < BWD_MAX_BLOCKS ? tiles : BWD_MAX_BLOCKS;
+}
+
+static int n_params(int n_actions) { return n_actions == 5 ? PV<5>::N : PV<9>::N; }
+
+static int launch_evaluate(const EvalArgs& a, int n_actions, cudaStream_t st) {
+  const unsigned grid = (unsigned)((a.n_rows + 127) / 128);
+  if (n_actions == 5) policy_eval_kernel<5><<<grid, 128, 0, st>>>(a);
+  else policy_eval_kernel<9><<<grid, 128, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+template <int NA>
+static int launch_backward_na(EvalArgs a, float* grad, cudaStream_t st) {
+  const int64_t G = bwd_blocks(a.n_rows);
+  a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
+  const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
+  if (sizeof(BwdSmem<NA>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
+    const cudaError_t e = cudaFuncSetAttribute(policy_backward_kernel<NA>,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    if (e != cudaSuccess) return (int)e;
+  }
+  policy_backward_kernel<NA><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
+  policy_grad_reduce_kernel<<<(PV<NA>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA>::N, grad);
+  return (int)cudaGetLastError();
+}
+
 static int launch_actor(const PolicyParams& w, const PolicyIO& io, int n_actions, cudaStream_t st) {
   if (io.n_rows == 0) return 0;
   const int block = 128;            // = AG, the agents a block owns
@@ -364,9 +743,74 @@ int check_device(int device, const char* who) {
   }
   return GSM_OK;
 }
+int pfailf(int status, const char* who, const char* msg) {
+  snprintf(g_policy_err, sizeof(g_policy_err), "%s: %s", who, msg);
+  return status;
+}
+// The checks gsm_policy_evaluate and gsm_policy_backward share; none touches the device.
+int check_eval_io(const gsm_policy_eval_io* io, const char* who) {
+  if (!io) return pfailf(GSM_ERR_INVALID_ARG, who, "io is NULL");
+  if (io->struct_size != sizeof(gsm_policy_eval_io)) return pfailf(GSM_ERR_ABI, who, "io.struct_size mismatch");
+  if (io->n_actions != 5 && io->n_actions != 9)
+    return pfailf(GSM_ERR_UNSUPPORTED, who, "compiled learner instances exist for n_actions 5 and 9 only");
+  if (!io->params || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
+    return pfailf(GSM_ERR_INVALID_ARG, who, "params, obs, nbr_feat, nbr_cnt and actions are required");
+  if (io->n_rows < 0 || io->max_nbrs < 1) return pfailf(GSM_ERR_INVALID_ARG, who, "bad n_rows / max_nbrs");
+  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfailf(GSM_ERR_INVALID_ARG, who, "n_rows too large");
+  return GSM_OK;
+}
+gsm::EvalArgs eval_args(const gsm_policy_eval_io* io) {
+  gsm::EvalArgs a{};
+  a.params = io->params; a.obs = io->obs; a.nbr_feat = io->nbr_feat; a.nbr_cnt = io->nbr_cnt;
+  a.actions = io->actions; a.rows = io->rows;
+  a.n_rows = io->n_rows; a.K = io->max_nbrs;
+  return a;
+}
 }  // namespace
 
 extern "C" {
+
+int gsm_policy_evaluate(const gsm_policy_eval_io* io, int device, void* stream) {
+  if (const int st = check_eval_io(io, "gsm_policy_evaluate")) return st;
+  if (io->n_rows == 0) return GSM_OK;
+  if (const int ds = check_device(device, "gsm_policy_evaluate")) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_evaluate: cudaSetDevice failed");
+  gsm::EvalArgs a = eval_args(io);
+  a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
+  const int e = gsm::launch_evaluate(a, io->n_actions, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
+
+int64_t gsm_policy_backward_workspace(int64_t n_rows, int32_t n_actions) {
+  if (n_actions != 5 && n_actions != 9)
+    return pfailf(GSM_ERR_UNSUPPORTED, "gsm_policy_backward_workspace", "n_actions must be 5 or 9");
+  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_policy_backward_workspace", "n_rows < 0");
+  return gsm::bwd_blocks(n_rows) * gsm::n_params(n_actions) * (int64_t)sizeof(float);
+}
+
+int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const float* d_entropy,
+                        const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
+                        int device, void* stream) {
+  const char* who = "gsm_policy_backward";
+  if (const int st = check_eval_io(io, who)) return st;
+  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
+  const int64_t need = gsm_policy_backward_workspace(io->n_rows, io->n_actions);
+  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than gsm_policy_backward_workspace(n_rows, n_actions)");
+  if (io->n_rows == 0) return GSM_OK;
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_backward: cudaSetDevice failed");
+  gsm::EvalArgs a = eval_args(io);
+  a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
+  a.ws = (float*)workspace;
+  const int e = io->n_actions == 5 ? gsm::launch_backward_na<5>(a, grad, (cudaStream_t)stream)
+                                   : gsm::launch_backward_na<9>(a, grad, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
 
 const char* gsm_policy_last_error(void) { return g_policy_err; }
 

@@ -9,8 +9,11 @@ shared by all agents,
 
 `act` is ONE sm_100a kernel through the C ABI (`gsm_policy_act`): forward + sampling + log-prob,
 only the valid neighbour rows are read.  There is no fallback: `act` raises without the library
-or a device.  `logits_autograd` is the same function in plain torch ops for the LEARNER (it needs
-gradients, which the collect path does not); it is not used by `act` or by `collect_fused`.
+or a device.  `evaluate_actions` is the learner pass (SPEC.md §12): log-prob of given actions,
+entropy and both critics, differentiable through a forward kernel (`gsm_policy_evaluate`) and a
+backward kernel (`gsm_policy_backward`).  `logits_autograd` is the same function in plain torch ops
+(the reference formulation the kernels are tested against); it is not used by `act` or by
+`collect_fused`.
 """
 from __future__ import annotations
 
@@ -113,7 +116,44 @@ class GraphAttentionActor(torch.nn.Module):
             raise abi.GsmError(f"{lib.gsm_status_string(st).decode()}: {lib.gsm_policy_last_error().decode()}")
         return (actions, logp) + ((logits,) if want_logits else ()) + ((values,) if want_values else ())
 
-    # ---- learner path: same function, differentiable (not used by act / collect_fused) --------
+    # ---- learner pass: two kernels, differentiable ----------------------------------------------
+    def evaluate_actions(self, obs, graph, actions, rows=None):
+        """log pi(actions), entropy and the two critics, differentiable w.r.t. the parameters.
+
+        obs [..., 6], graph['nbr_feat'] [..., K, 6], graph['nbr_cnt'] [...] and actions [...]
+        (fp32 / int32 contiguous CUDA tensors on the parameters' device) are the source rows.  rows:
+        optional int64 1-D index into the flattened source rows (a shuffled minibatch read straight
+        out of the rollout buffer, no gather of nbr_feat).  Returns logp [n], entropy [n] and values
+        [n, 2] with n = the source shape, or [len(rows)].  logp and values are bit-identical to what
+        `act` / `collect_fused` wrote for the same rows and actions.  The range check on `rows`
+        synchronises and is skipped while a CUDA graph is being captured."""
+        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
+        params = torch.nn.utils.parameters_to_vector(self.parameters())
+        if not (obs.is_cuda and feat.is_cuda and cnt.is_cuda and actions.is_cuda):
+            raise abi.GsmError("CUDA tensors required: gs_marl_b200 has no CPU fallback")
+        dev = obs.device
+        if params.device != dev or any(t.device != dev for t in (feat, cnt, actions)):
+            raise abi.GsmError(f"the actor's parameters and all inputs must be on {dev}")
+        if (params.dtype != torch.float32 or obs.dtype != torch.float32 or feat.dtype != torch.float32
+                or cnt.dtype != torch.int32 or actions.dtype != torch.int32):
+            raise TypeError("the learner kernels are fp32: parameters/obs/nbr_feat float32, nbr_cnt/actions int32")
+        if not (obs.is_contiguous() and feat.is_contiguous() and cnt.is_contiguous() and actions.is_contiguous()):
+            raise ValueError("obs, nbr_feat, nbr_cnt and actions must be contiguous")
+        lead = tuple(cnt.shape)
+        if (obs.shape != lead + (abi.GSM_OBS_DIM,) or feat.shape[:-2] != lead
+                or feat.shape[-1] != abi.GSM_NBR_FEAT_DIM or tuple(actions.shape) != lead):
+            raise ValueError("obs / nbr_feat / nbr_cnt / actions shapes disagree")
+        if rows is not None:
+            if rows.dtype != torch.int64 or rows.dim() != 1 or rows.device != dev:
+                raise ValueError(f"rows must be a 1-D int64 tensor on {dev}")
+            rows = rows.contiguous()
+            if rows.numel() and not torch.cuda.is_current_stream_capturing():
+                lo, hi = torch.aminmax(rows)
+                if int(lo) < 0 or int(hi) >= cnt.numel():
+                    raise IndexError(f"rows out of range [0, {cnt.numel()})")
+        return _EvaluateActions.apply(params, obs, feat, cnt, actions, rows, self.n_actions)
+
+    # ---- the same function in plain torch (reference formulation; not used by the kernels) ----
     def logits_autograd(self, obs, graph):
         return self.head(self.embed_autograd(obs, graph))
 
@@ -130,3 +170,61 @@ class GraphAttentionActor(torch.nn.Module):
         a = torch.softmax(sc, -1).nan_to_num(0.0)            # rows with cnt == 0: all -inf -> 0
         agg = (a[..., None] * m).sum(-2)
         return torch.cat([e, agg], -1)
+
+
+def _eval_io(n_actions, params, obs, feat, cnt, actions, rows) -> abi.GsmPolicyEvalIO:
+    io = abi.GsmPolicyEvalIO()
+    io.struct_size, io.n_actions = C.sizeof(abi.GsmPolicyEvalIO), n_actions
+    io.params, io.obs, io.nbr_feat = params.data_ptr(), obs.data_ptr(), feat.data_ptr()
+    io.nbr_cnt, io.actions = cnt.data_ptr(), actions.data_ptr()
+    io.rows = rows.data_ptr() if rows is not None else None
+    io.n_rows = rows.numel() if rows is not None else cnt.numel()
+    io.max_nbrs = int(feat.shape[-2])
+    return io
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+class _EvaluateActions(torch.autograd.Function):
+    """forward: gsm_policy_evaluate; backward: gsm_policy_backward (grad w.r.t. the parameter vector)."""
+
+    @staticmethod
+    def forward(ctx, params, obs, feat, cnt, actions, rows, n_actions):
+        lib = abi.load_library()
+        params = params.contiguous()
+        dev = obs.device
+        shape = (rows.numel(),) if rows is not None else tuple(cnt.shape)
+        logp = torch.empty(shape, dtype=torch.float32, device=dev)
+        entropy = torch.empty(shape, dtype=torch.float32, device=dev)
+        values = torch.empty(shape + (abi.GSM_POLICY_VALUE_HEADS,), dtype=torch.float32, device=dev)
+        io = _eval_io(n_actions, params, obs, feat, cnt, actions, rows)
+        io.logp, io.entropy, io.values = logp.data_ptr(), entropy.data_ptr(), values.data_ptr()
+        _check(lib, lib.gsm_policy_evaluate(C.byref(io), dev.index or 0,
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        ctx.save_for_backward(params, obs, feat, cnt, actions, rows)
+        ctx.n_actions = n_actions
+        ctx.set_materialize_grads(False)          # an unused output arrives as None -> NULL (zero)
+        return logp, entropy, values
+
+    @staticmethod
+    def backward(ctx, d_logp, d_entropy, d_values):
+        lib = abi.load_library()
+        params, obs, feat, cnt, actions, rows = ctx.saved_tensors
+        dev = obs.device
+        io = _eval_io(ctx.n_actions, params, obs, feat, cnt, actions, rows)
+        if not io.n_rows:
+            return torch.zeros_like(params), None, None, None, None, None, None
+        grad = torch.empty_like(params)
+        ws = torch.empty(lib.gsm_policy_backward_workspace(io.n_rows, ctx.n_actions), dtype=torch.uint8, device=dev)
+        d = [g.contiguous() if g is not None else None for g in (d_logp, d_entropy, d_values)]
+        _check(lib, lib.gsm_policy_backward(C.byref(io), _ptr(d[0]), _ptr(d[1]), _ptr(d[2]), grad.data_ptr(),
+                                            ws.data_ptr(), ws.numel(), dev.index or 0,
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        return grad, None, None, None, None, None, None
+
+
+def _check(lib, st):
+    if st != 0:
+        raise abi.GsmError(f"{lib.gsm_status_string(st).decode()}: {lib.gsm_policy_last_error().decode()}")

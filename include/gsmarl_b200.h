@@ -300,6 +300,50 @@ typedef struct gsm_policy_io {   /* DEVICE pointers; a "row" is one agent of one
 int gsm_policy_act(const gsm_policy_weights* w, const gsm_policy_io* io, int device, void* stream);
 const char* gsm_policy_last_error(void);
 
+/* ---- learner pass (SPEC.md §12): evaluate_actions of the same actor, forward and backward ------
+ * Stands in for the lineage's evaluate_actions / get_values (SOURCES.txt:8, withheld).  The weights
+ * are a DEVICE float vector in torch.nn.utils.parameters_to_vector(GraphAttentionActor) order:
+ *   ego_w[64][6], ego_b[64], nbr_w[64][6], nbr_b[64], att_w[64], att_b, head_w[A][128], head_b[A],
+ *   value_w[2][128], value_b[2]   -> GSM_POLICY_N_PARAMS(A) floats (1864 for A = 5, 2380 for A = 9).
+ * No host copy and no host sync: a minibatch step can be captured in a CUDA graph.  Row i of the
+ * call reads source row src = rows ? rows[i] : i of obs / nbr_feat / nbr_cnt / actions and writes
+ * element i of every output.  Only the nbr_cnt[src] valid neighbour rows are read.  fp32 only. */
+#define GSM_POLICY_N_PARAMS(n_actions) (961 + 129 * (n_actions) + 2 * (2 * GSM_POLICY_HIDDEN + 1))
+
+typedef struct gsm_policy_eval_io {   /* DEVICE pointers */
+  uint32_t struct_size;      /* = sizeof(gsm_policy_eval_io); checked                          */
+  int32_t n_actions;         /* 5 or 9                                                         */
+  const float* params;       /* [GSM_POLICY_N_PARAMS(n_actions)]                               */
+  const float* obs;          /* [src_rows][GSM_OBS_DIM]                                        */
+  const float* nbr_feat;     /* [src_rows][max_nbrs][GSM_NBR_FEAT_DIM]                         */
+  const int32_t* nbr_cnt;    /* [src_rows]  valid rows (clamped to [0, max_nbrs])              */
+  const int32_t* actions;    /* [src_rows]  an action outside [0, n_actions) gives NaN logp / grad */
+  const int64_t* rows;       /* [n_rows] source row of row i (caller keeps it in range); NULL = i */
+  float* logp;               /* [n_rows] out, z_a - logsumexp(z); NULL = skip                  */
+  float* entropy;            /* [n_rows] out, logsumexp(z) - sum_k p_k z_k; NULL = skip        */
+  float* values;             /* [n_rows][GSM_POLICY_VALUE_HEADS] out; NULL = skip              */
+  int64_t n_rows;
+  int32_t max_nbrs;
+  int32_t reserved;          /* 0 */
+} gsm_policy_eval_io;
+
+/* logp / values bit-identical to what gsm_policy_act / gsm_collect wrote for the same rows and actions. */
+int gsm_policy_evaluate(const gsm_policy_eval_io* io, int device, void* stream);
+
+/* Workspace bytes gsm_policy_backward needs for n_rows rows (a function of n_rows and n_actions
+ * only); GSM_ERR_INVALID_ARG for n_rows < 0, GSM_ERR_UNSUPPORTED for n_actions not 5 or 9. */
+int64_t gsm_policy_backward_workspace(int64_t n_rows, int32_t n_actions);
+
+/* grad [GSM_POLICY_N_PARAMS] (overwritten) = d/dparams of
+ *   sum_i d_logp[i] logp[i] + d_entropy[i] entropy[i] + d_values[i] . values[i]
+ * over the rows of io (its output pointers are not used).  d_logp, d_entropy [n_rows] and d_values
+ * [n_rows][2] may each be NULL (= zero).  Deterministic: per-block partial sums into `workspace`
+ * (a partition of the rows that depends on n_rows only), combined in a fixed order; no atomics.
+ * n_rows == 0 leaves grad untouched. */
+int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const float* d_entropy,
+                        const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
+                        int device, void* stream);
+
 /* n_steps of {actor forward + sampling, env step} enqueued on `stream` with no host sync (2
  * kernels per step; capturable into a CUDA graph).  io->obs / nbr_* / adj / assign point at slot 0
  * of [n_steps+1][...] tensors whose slot 0 already holds the current observation (gsm_reset,
