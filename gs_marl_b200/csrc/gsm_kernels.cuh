@@ -132,15 +132,19 @@ template <> __device__ __forceinline__ double r_inf<double>() {
 __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                               uint32_t k0, uint32_t k1, uint32_t out[4]);
 __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo);
+__device__ __forceinline__ void spawn_draw_inline(uint64_t g, int ep, int e, uint64_t seed, double ext,
+                                                  double& x, double& y) {
+  uint32_t r[4];
+  philox4x32_10((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)ep, (uint32_t)e, (uint32_t)seed,
+                (uint32_t)(seed >> 32), r);
+  x = __dadd_rn(-ext, __dmul_rn(2.0 * ext, u53(r[0], r[1])));
+  y = __dadd_rn(-ext, __dmul_rn(2.0 * ext, u53(r[2], r[3])));
+}
 // Cold path (once per episode end): kept out of line so that the 10 unrolled Philox rounds do
 // not raise the register count of the step loops.
 static __device__ __noinline__ void spawn_draw_f64(uint64_t g, int ep, int e, uint64_t seed, double ext,
                                             double* x, double* y) {
-  uint32_t r[4];
-  philox4x32_10((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)ep, (uint32_t)e, (uint32_t)seed,
-                (uint32_t)(seed >> 32), r);
-  *x = __dadd_rn(-ext, __dmul_rn(2.0 * ext, u53(r[0], r[1])));
-  *y = __dadd_rn(-ext, __dmul_rn(2.0 * ext, u53(r[2], r[3])));
+  spawn_draw_inline(g, ep, e, seed, ext, *x, *y);
 }
 template <typename T>
 __device__ __forceinline__ void spawn_draw(uint64_t g, int ep, int e, uint64_t seed, double ext, T& x, T& y) {

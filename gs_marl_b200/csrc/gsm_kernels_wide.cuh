@@ -89,6 +89,29 @@ __device__ __forceinline__ void lds4(unsigned a, double& x, double& y, double& z
   asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(x), "=d"(y) : "r"(a) : "memory");
   asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(z), "=d"(w) : "r"(a + 16) : "memory");
 }
+// Predicated stores (`@q st.shared`): a lane-dependent or pass-dependent store costs no branch region.
+__device__ __forceinline__ void sts_if(bool on, unsigned a, unsigned v) {
+  asm volatile("{ .reg .pred q; setp.ne.u32 q, %2, 0; @q st.shared.u32 [%0], %1; }" :: "r"(a), "r"(v), "r"((unsigned)on) : "memory");
+}
+__device__ __forceinline__ void sts2_if(bool on, unsigned a, float x, float y) {
+  asm volatile("{ .reg .pred q; setp.ne.u32 q, %3, 0; @q st.shared.v2.f32 [%0], {%1, %2}; }" :: "r"(a), "f"(x), "f"(y), "r"((unsigned)on) : "memory");
+}
+__device__ __forceinline__ void sts2_if(bool on, unsigned a, double x, double y) {
+  asm volatile("{ .reg .pred q; setp.ne.u32 q, %3, 0; @q st.shared.v2.f64 [%0], {%1, %2}; }" :: "r"(a), "d"(x), "d"(y), "r"((unsigned)on) : "memory");
+}
+// A select the compiler keeps as one SEL: a chain of ?: on a lane index otherwise becomes a jump table (BRX).
+__device__ __forceinline__ unsigned selp(bool c, unsigned a, unsigned b) {
+  unsigned r;
+  asm("{ .reg .pred q; setp.ne.u32 q, %3, 0; selp.b32 %0, %1, %2, q; }" : "=r"(r) : "r"(a), "r"(b), "r"((unsigned)c));
+  return r;
+}
+// Arith<T>::div computed on every lane, for a result that is then selected: the compiler keeps a volatile asm
+// where it stands instead of sinking it into a branch region (fp32: the same div.approx.f32 that __fdividef
+// emits, so the same bits).
+__device__ __forceinline__ float div_eager(float a, float b) {
+  float r; asm volatile("div.approx.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r;
+}
+__device__ __forceinline__ double div_eager(double a, double b) { return a / b; }
 __device__ __forceinline__ float4 lds16(unsigned a) {
   float4 v; asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a) : "memory"); return v;
 }
@@ -145,6 +168,7 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
                 const __grid_constant__ WideSmem lay_rt) {
   constexpr int E = N + L, M = E - 1, GW = wide_pow2(M), EPW = 32 / GW;
   constexpr bool OBS = MODE == 1;
+  constexpr bool BF = MODE == 2;                       // branch-free chunk body (see the chunk loop)
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int RB = (int)sizeof(T);
   constexpr int RS4 = EPW * N * 4, RST = EPW * N * RB;      // bytes of a per-agent 4-byte / real block of the warp
@@ -167,7 +191,8 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
   const int env_w0 = keep((int)(((int64_t)blockIdx.x * (kWideThreads / 32) + warp) * EPW));
   bool active = env_w0 + grp < p.n_envs;
   if (OBS && p.mask != nullptr && active) active = p.mask[(int64_t)(env_w0 + grp) * p.mask_stride] != 0;
-  const int env = active ? env_w0 + grp : 0;            // idle groups shadow env 0, never store
+  // idle groups read only env 0's actions (an input), start from a dummy state and never store (below)
+  const int env = active ? env_w0 + grp : 0;
   const bool has = M == GW ? true : j < M;
   const bool own = j < N;                               // I own (integrate, publish) agent j
   const int ja = own ? j : 0;
@@ -196,17 +221,21 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
   const int goal_i = (int)(lfl >> 8) - 1;
 
   // ---- state: my own agent in registers, everything in the entity table ---------------------------
-  T mx, my, mvx, mvy;
-  {
+  // An idle group starts with every entity at rest at the origin and t = 0.  Its values then evolve (t counts up,
+  // coincident entities give NaN forces) but stay inside the group: `fin` and the episode-end minimum mask on
+  // `active`, the force butterfly runs within the group, and every store is predicated on `active` / act_bits.
+  T mx = 0, my = 0, mvx = 0, mvy = 0;
+  if (active) {
     const T* a = p.agent_state + ((int64_t)env * N + ja) * 4;
     mx = a[0]; my = a[1]; mvx = a[2]; mvy = a[3];
   }
   if (own) sts4(sa_ent + (unsigned)j * ES, mx, my, mvx, mvy);
   if (has && j + 1 >= N) {                               // lane j also holds landmark j + 1 - N
-    const T* l = p.lm_pos + ((int64_t)env * L + (j + 1 - N)) * 2;
-    sts4(sa_ent + (unsigned)(j + 1) * ES, l[0], l[1], (T)0, (T)0);
+    T lx = 0, ly = 0;
+    if (active) { const T* l = p.lm_pos + ((int64_t)env * L + (j + 1 - N)) * 2; lx = l[0]; ly = l[1]; }
+    sts4(sa_ent + (unsigned)(j + 1) * ES, lx, ly, (T)0, (T)0);
   }
-  int t_now = p.t[env];
+  int t_now = active ? p.t[env] : 0;
   const bool auto_reset = MODE == 2 && p.auto_reset != 0;
   const T accel_m = keep(wc.accel[ja]), mass_m = keep(wc.mass[ja]), massinv_m = keep(wc.mass_inv[ja]), maxsp_m = keep(wc.maxsp[ja]);
 
@@ -266,11 +295,24 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
   const unsigned o_idx = keep(lay.idx + (unsigned)(grp * N * K) * 4u);
   const unsigned o_sc = keep(lay.cnt + (unsigned)(j < 3 ? j : 0) * (unsigned)RS4 + (unsigned)(grp * N) * 4u);
   const unsigned o_obs = keep(lay.obs + (unsigned)grp * (unsigned)(N * GSM_OBS_DIM * RB));
+  // The hot loop runs up to step `stop` (warp-uniform): the launch's end or, with auto-reset, the first step
+  // after which an env of the warp ends its episode (at least one step: an env that starts at or past its
+  // episode's end is re-drawn after one).  It is counted once here and after every re-draw, so the loop has
+  // no per-step vote.  Idle groups never end an episode.
+  const auto segment_end = [&]() {
+    int s = n_steps;
+    if (MODE == 2 && auto_reset) {
+      const int left = __reduce_min_sync(FULL, active ? p.episode_length - t_now : INT_MAX);
+      s = step + max(1, min(left, n_steps - step));
+    }
+    return s;
+  };
+  int stop = segment_end();
   while (step < n_steps) {
-   // hot loop: runs until the launch ends or an env of the warp finishes its episode (MODE 2)
+   // hot loop: runs until `stop`
    for (;;) {
     if (!OBS && !pro) {
-      // ---- SPEC §2 + §4 for my own agent (lanes j >= N shadow agent 0 and publish nothing) -----------
+      // ---- SPEC §2 + §4 for my own agent (lanes j >= N integrate values that are never used or published) -
       T ux = actx_next, uy = acty_next;
       if (discrete) {
         const int a = act_next;
@@ -320,7 +362,21 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
       int cnt = __popc(bits);
       const int rank = __popc(bits & low_mask(j));
       const int pos = nb ? rank : cnt + (j - rank);
-      if (has && pos < K && st_on) {
+      // Two forms of the same stores and the same contact term, chosen per instance.  BF (auto-reset): every
+      // lane writes its pair's row (values or zeros, by selects) and the scalars with predicated stores, and
+      // computes the contact term and selects it — no branch regions.  Otherwise the branchy form: in the
+      // plain / observe instances the branch-free one costs a register and a spill (<float,3,6,0,8>: 71 -> 72
+      // registers, an 8 B stack) and runs 9 % slower as one launch (profiles/README.md, w7).
+      if (BF) {
+        // with K >= M every row lands inside the agent's K rows
+        const bool row_on = st_on && has && (KT >= M || pos < K);
+        sts_if(row_on, a_idx + (unsigned)pos * 4u + (unsigned)(i * K * 4), (unsigned)(nb ? e : -1));
+        const unsigned f = a_feat + (unsigned)pos * (unsigned)(GSM_NBR_FEAT_DIM * RB) + (unsigned)(i * K * GSM_NBR_FEAT_DIM * RB);
+        const T z = (T)0;
+        sts2_if(row_on, f, nb ? dx : z, nb ? dy : z);
+        sts2_if(row_on, f + 2 * RB, nb ? so.vx - si.vx : z, nb ? so.vy - si.vy : z);
+        sts2_if(row_on, f + 4 * RB, nb ? dist : z, nb ? type_o : z);
+      } else if (has && pos < K && st_on) {
         sts(a_idx + (unsigned)pos * 4u + (unsigned)(i * K * 4), nb ? e : -1);
         const unsigned f = a_feat + (unsigned)pos * (unsigned)(GSM_NBR_FEAT_DIM * RB) + (unsigned)(i * K * GSM_NBR_FEAT_DIM * RB);
         const T z = (T)0;
@@ -328,11 +384,14 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
         else { sts2(f, z, z); sts2(f + 2 * RB, z, z); sts2(f + 4 * RB, z, z); }
       }
       if (cnt > K) cnt = K;
-      if (st_on && j < 3) {                               // lanes 0, 1, 2 stage cnt, adj, cost of agent i
-        // entity-indexed adjacency: open a zero bit at the agent's own index i
-        const unsigned ebits = (bits & low_mask(i)) | ((bits & ~low_mask(i)) << 1);
+      // entity-indexed adjacency: open a zero bit at the agent's own index i
+      const unsigned ebits = (bits & low_mask(i)) | ((bits & ~low_mask(i)) << 1);
+      if (BF && RB == 4) {                                // lanes 0, 1, 2 stage cnt, adj, cost of agent i: three
+        const unsigned v = selp(j == 0, (unsigned)cnt, selp(j == 1, ebits, __float_as_uint((float)__popc(cbits))));
+        sts_if(st_on && j < 3, a_sc + (unsigned)(i * 4), v);   // equal 4-byte blocks, one store
+      } else if (st_on && j < 3) {
         const unsigned ao = (unsigned)(grp * N + i);
-        if (RB == 4) {                                    // three equal 4-byte blocks in a row: one store
+        if (RB == 4) {
           const unsigned v = j == 0 ? (unsigned)cnt : (j == 1 ? ebits : __float_as_uint((float)__popc(cbits)));
           if (!OBS || j < 2) sts(a_sc + (unsigned)(i * 4), v);
         } else {
@@ -342,8 +401,17 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
         }
       }
       if (j == N - 1 + i) { gxs = dx; gys = dy; gd = dist; }   // my landmark is this agent's goal
-      if (!OBS) {                                         // SPEC §3 for the next step, on the same geometry:
-        fcx[i] = 0; fcy[i] = 0;                           // the force uses p_i - p_e = -d, exactly
+      if (BF) {                                           // SPEC §3 for the next step, on the same geometry:
+        // the force uses p_i - p_e = -d, exactly
+        const T x = A::div_const(-(dist - dmin), p.km, p.km_inv);
+        const bool term = cpair && !(Prec<T>::kCut && x < (T)(-kFarCut));
+        const T pen = softplus1(x) * p.km;
+        const T qx = div_eager(p.cf * (-dx), dist), qy = div_eager(p.cf * (-dy), dist);
+        fcx[i] = term ? qx * pen : (T)0;
+        fcy[i] = term ? qy * pen : (T)0;
+        anyc = anyc || term;
+      } else if (!OBS) {
+        fcx[i] = 0; fcy[i] = 0;
         if (cpair) {
           const T x = A::div_const(-(dist - dmin), p.km, p.km_inv);
           if (!(Prec<T>::kCut && x < (T)(-kFarCut))) {
@@ -442,36 +510,39 @@ env_wide_kernel(const __grid_constant__ KParams<T> p, const int n_steps,
     sb += sb_delta;
     sb_delta = -sb_delta;
     step++;
-    if (step >= n_steps) break;
-    if (MODE == 2 && auto_reset && __any_sync(FULL, t_now >= p.episode_length)) break;
+    if (step >= stop) break;
    }
    if (OBS) break;
    // ---- episode end inside a fused rollout: re-draw (the terminal outputs stay in their slot).  Cold:
-   //      outside the hot loop so that its calls and spills stay out of it ------------------------------------
+   //      outside the hot loop, which it costs nothing ------------------------------------------------------
    if (MODE == 2 && auto_reset) {
-     const bool fin = t_now >= p.episode_length;
+     const bool fin = active && t_now >= p.episode_length;
      if (__any_sync(FULL, fin)) {
        __syncwarp();                                      // every lane has read the old table
+       int ep = 0;
        if (fin) {
          // the episode counter and the landmarks are not held in registers across the hot loop: both are
-         // read / written in global memory right here (once per episode)
+         // read / written in global memory right here (once per episode).  Lane j draws entities j, j + GW,
+         // ... (navigation-3: 9 entities on 8 lanes, two rounds), inline: no call, no stack frame
          const uint64_t genv = (uint64_t)(p.env_offset + env);
-         const int ep = p.episode[env];
-         spawn_draw<T>(genv, ep, ja, p.seed, p.ext[GSM_ENT_AGENT], mx, my);
-         mvx = 0; mvy = 0;
-         if (own) sts4(sa_ent + (unsigned)j * ES, mx, my, (T)0, (T)0);
-         if (has && j + 1 >= N) {
-           T lx, ly;
-           spawn_draw<T>(genv, ep, j + 1, p.seed, p.ext[wc.eflag[j + 1] >> 1], lx, ly);
-           sts4(sa_ent + (unsigned)(j + 1) * ES, lx, ly, (T)0, (T)0);
-           if (active) { T* l = p.lm_pos + ((int64_t)env * L + (j + 1 - N)) * 2; l[0] = lx; l[1] = ly; }
+         ep = p.episode[env];
+#pragma unroll 1
+         for (int e = j; e < E; e += GW) {
+           double dx, dy;
+           spawn_draw_inline(genv, ep, e, p.seed, p.ext[wc.eflag[e] >> 1], dx, dy);
+           const T x = (T)dx, y = (T)dy;
+           sts4(sa_ent + (unsigned)e * ES, x, y, (T)0, (T)0);
+           if (e < N) { mx = x; my = y; }                 // e = j: my own agent
+           else { T* l = p.lm_pos + ((int64_t)env * L + (e - N)) * 2; l[0] = x; l[1] = y; }
          }
+         mvx = 0; mvy = 0;
          t_now = 0;
        }
        __syncwarp();                                      // every lane of the env has read the old counter
-       if (fin && j == 0 && active) p.episode[env] += 1;
+       if (fin && j == 0) p.episode[env] = ep + 1;
        __syncwarp();
        pro = step < n_steps;                              // the new positions need their forces
+       stop = segment_end();
      }
    }
   }
