@@ -674,7 +674,10 @@ static int launch_backward_na(EvalArgs a, float* grad, cudaStream_t st) {
   if (sizeof(BwdSmem<NA>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
     const cudaError_t e = cudaFuncSetAttribute(policy_backward_kernel<NA>,
                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-    if (e != cudaSuccess) return (int)e;
+    if (e != cudaSuccess) {            // max_nbrs beyond the block's shared memory: report it here and clear
+      cudaGetLastError();              // it, or the next launch's cudaGetLastError() would report it again
+      return (int)e;
+    }
   }
   policy_backward_kernel<NA><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
   policy_grad_reduce_kernel<<<(PV<NA>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA>::N, grad);

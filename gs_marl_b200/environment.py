@@ -118,6 +118,8 @@ class MultiAgentGraphConstrainEnv:
         m, stride = None, 1
         if mask is not None:
             mt = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            if tuple(mt.shape) != (self.n_envs,):       # the reset kernel reads one byte per env
+                raise ValueError(f"mask must have shape ({self.n_envs},), got {tuple(mt.shape)}")
             m = C.c_void_p(mt.data_ptr())
         with torch.cuda.device(self.device):
             self._check(self.lib.gsm_reset(self._h, self._seed, m, stride, C.byref(self._io),
@@ -152,6 +154,13 @@ class MultiAgentGraphConstrainEnv:
             raise ValueError(f"actions must have shape (T,)+{tuple(shape)}")
         if out is None:
             out = {k: self._alloc(k, (T,)) for k in self.OUTPUTS}
+        for k in self.OUTPUTS:                            # the kernel writes T full slots of each
+            dt, shape = self._shapes[k]
+            o = out[k]
+            if tuple(o.shape) != (T,) + tuple(shape) or o.dtype != _TORCH_DT[dt] or o.device != self.device \
+                    or not o.is_contiguous():
+                raise ValueError(f"out[{k!r}] must be a contiguous {_TORCH_DT[dt]} tensor of shape "
+                                 f"{(T,) + tuple(shape)} on {self.device}")
         io = self._make_io(out, a)
         ar = self.auto_reset if auto_reset is None else bool(auto_reset)
         with torch.cuda.device(self.device):
@@ -178,6 +187,13 @@ class MultiAgentGraphConstrainEnv:
         def prep(x, dt):
             return None if x is None else torch.as_tensor(x).to(device=self.device, dtype=dt).contiguous()
         a, l, t = prep(agent_state, r), prep(landmark_pos, r), prep(step_count, torch.int32)
+        w = self.world
+        # the copies read n_envs rows of each: a smaller array would be read past its end
+        for name, x, shape in (("agent_state", a, (self.n_envs, w.n_agents, 4)),
+                               ("landmark_pos", l, (self.n_envs, w.n_landmarks, 2)),
+                               ("step_count", t, (self.n_envs,))):
+            if x is not None and tuple(x.shape) != shape:
+                raise ValueError(f"{name} must have shape {shape}, got {tuple(x.shape)}")
         p = [C.c_void_p(x.data_ptr()) if x is not None and x.numel() else None for x in (a, l, t)]
         with torch.cuda.device(self.device):
             self._check(self.lib.gsm_set_state(self._h, p[0], p[1], p[2], self._stream()))
