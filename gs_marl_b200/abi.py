@@ -16,6 +16,8 @@ GSM_MAX_LSA_N = 32
 GSM_POLICY_HIDDEN = 64
 GSM_POLICY_MAX_ACTIONS = 9
 GSM_POLICY_VALUE_HEADS = 2
+GSM_POLICY_GAUSS_DIM = 2
+GSM_POLICY_GAUSS_N_PARAMS = 1479
 
 GSM_F32, GSM_F64 = 0, 1
 GSM_SCN_NAVIGATION, GSM_SCN_POLYGON, GSM_SCN_LINE = 0, 1, 2
@@ -95,6 +97,39 @@ class GsmPolicyEvalIO(C.Structure):
     ]
 
 
+class GsmPolicyGaussWeights(C.Structure):
+    """gsm_policy_gauss_weights: the Gaussian actor, row-major [out][in], host memory."""
+    _H, _D = GSM_POLICY_HIDDEN, GSM_POLICY_GAUSS_DIM
+    _fields_ = [
+        ("struct_size", C.c_uint32),
+        ("ego_w", C.c_float * GSM_OBS_DIM * _H), ("ego_b", C.c_float * _H),
+        ("nbr_w", C.c_float * GSM_NBR_FEAT_DIM * _H), ("nbr_b", C.c_float * _H),
+        ("att_w", C.c_float * _H), ("att_b", C.c_float),
+        ("mean_w", C.c_float * (2 * _H) * _D), ("mean_b", C.c_float * _D), ("log_std", C.c_float * _D),
+        ("value_w", C.c_float * (2 * _H) * GSM_POLICY_VALUE_HEADS), ("value_b", C.c_float * GSM_POLICY_VALUE_HEADS),
+    ]
+
+
+class GsmPolicyGaussIO(C.Structure):
+    _fields_ = [
+        ("obs", C.c_void_p), ("nbr_feat", C.c_void_p), ("nbr_cnt", C.c_void_p),
+        ("actions", C.c_void_p), ("logp", C.c_void_p), ("mean", C.c_void_p),
+        ("values", C.c_void_p), ("n_rows", C.c_int64), ("row_offset", C.c_uint64), ("seed", C.c_uint64), ("step", C.c_uint64),
+        ("max_nbrs", C.c_int32), ("greedy", C.c_int32),
+    ]
+
+
+class GsmPolicyGaussEvalIO(C.Structure):
+    """gsm_policy_gauss_eval_io: DEVICE pointers; `params` is the parameters_to_vector(GaussianGraphActor) vector."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("action_dim", C.c_int32),
+        ("params", C.c_void_p), ("obs", C.c_void_p), ("nbr_feat", C.c_void_p), ("nbr_cnt", C.c_void_p),
+        ("actions", C.c_void_p), ("rows", C.c_void_p),
+        ("logp", C.c_void_p), ("entropy", C.c_void_p), ("values", C.c_void_p),
+        ("n_rows", C.c_int64), ("max_nbrs", C.c_int32), ("reserved", C.c_int32),
+    ]
+
+
 def policy_n_params(n_actions: int) -> int:
     """GSM_POLICY_N_PARAMS: length of the learner's parameter vector."""
     return 961 + 129 * n_actions + 2 * (2 * GSM_POLICY_HIDDEN + 1)
@@ -141,6 +176,14 @@ SYMBOLS = {
                           C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gsm_collect": (C.c_int, [_H, C.POINTER(GsmPolicyWeights), C.c_int32, _IO, C.c_void_p, C.c_void_p,
                               C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
+    "gsm_policy_act_gauss": (C.c_int, [C.POINTER(GsmPolicyGaussWeights), C.POINTER(GsmPolicyGaussIO), C.c_int,
+                                       C.c_void_p]),
+    "gsm_policy_evaluate_gauss": (C.c_int, [C.POINTER(GsmPolicyGaussEvalIO), C.c_int, C.c_void_p]),
+    "gsm_policy_backward_workspace_gauss": (C.c_int64, [C.c_int64]),
+    "gsm_policy_backward_gauss": (C.c_int, [C.POINTER(GsmPolicyGaussEvalIO), C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gsm_collect_gauss": (C.c_int, [_H, C.POINTER(GsmPolicyGaussWeights), C.c_int32, _IO, C.c_void_p, C.c_void_p,
+                                    C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
 }
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libgsmarl_b200.so")

@@ -767,20 +767,15 @@ int gsm_get_state_host(gsm_env* h, void* agent_state, void* landmark_pos, int32_
   return GSM_OK;
 }
 
-int gsm_collect(gsm_env* h, const gsm_policy_weights* w, int32_t n_steps, const gsm_step_io* io,
-                float* logp, float* values, uint64_t seed, uint64_t first_step, int32_t greedy,
-                void* stream) {
-  if (!h || !io || !w || n_steps < 1) return GSM_ERR_INVALID_ARG;
-  if (!is_f32(h) || h->hp.action_mode != GSM_ACT_DISCRETE)
-    return fail(h, GSM_ERR_UNSUPPORTED, "gsm_collect needs a GSM_F32 handle with discrete actions");
-  if (w->n_actions != h->hp.n_actions)
-    return fail(h, GSM_ERR_INVALID_ARG, "gsm_collect: weights.n_actions != cfg.n_discrete_actions");
-  if (!io->actions || !io->obs || !io->nbr_feat || !io->nbr_cnt)
-    return fail(h, GSM_ERR_INVALID_ARG, "gsm_collect needs io.actions, io.obs, io.nbr_feat and io.nbr_cnt");
-  if (h->auto_reset && !io->done) return fail(h, GSM_ERR_INVALID_ARG, "auto-reset collect needs io.done");
+}  // extern "C"
+
+namespace {
+// The collect loop both heads share: step t's actor reads observation slot t and writes actions slot
+// t (`act(t, obs, nbr_feat, nbr_cnt, actions)` enqueues it); gsm_step writes step outputs into slot t
+// and observation outputs into slot t + 1; auto-reset re-draws finished envs into slot t + 1.
+template <class Act>
+int collect_loop(gsm_env* h, int32_t n_steps, const gsm_step_io* io, void* stream, Act&& act) {
   DeviceGuard guard(h->device);
-  const int64_t rows = h->hp.n_envs * h->hp.N;
-  const int64_t slot_rows = (h->slot_envs ? h->slot_envs : h->hp.n_envs) * h->hp.N;
   for (int t = 0; t < n_steps; t++) {
     gsm_step_io cur;     // step outputs: slot t; observation outputs: slot t + 1
     for (int k = 0; k < IO_COUNT; k++) {
@@ -789,19 +784,10 @@ int gsm_collect(gsm_env* h, const gsm_policy_weights* w, int32_t n_steps, const 
                             k == IO_ADJ || k == IO_ASSIGN;
       io_set(cur, k, b ? b + (size_t)(t + (obs_like ? 1 : 0)) * slot_bytes(h, k) : nullptr);
     }
-    gsm_policy_io pio;
-    pio.obs = (const float*)((const unsigned char*)io->obs + (size_t)t * slot_bytes(h, IO_OBS));
-    pio.nbr_feat = (const float*)((const unsigned char*)io->nbr_feat + (size_t)t * slot_bytes(h, IO_NBR_FEAT));
-    pio.nbr_cnt = (const int32_t*)((const unsigned char*)io->nbr_cnt + (size_t)t * slot_bytes(h, IO_NBR_CNT));
-    pio.actions = (int32_t*)const_cast<void*>(cur.actions);
-    pio.logp = logp ? logp + (size_t)t * slot_rows : nullptr;
-    pio.logits = nullptr;
-    pio.values = values ? values + (size_t)t * slot_rows * GSM_POLICY_VALUE_HEADS : nullptr;
-    pio.n_rows = rows;
-    pio.row_offset = (uint64_t)h->hp.env_offset * (uint64_t)h->hp.N;
-    pio.seed = seed; pio.step = first_step + (uint64_t)t;
-    pio.max_nbrs = h->hp.K; pio.greedy = greedy;
-    int st = gsm_policy_act(w, &pio, h->device, stream);
+    const float* obs = (const float*)((const unsigned char*)io->obs + (size_t)t * slot_bytes(h, IO_OBS));
+    const float* feat = (const float*)((const unsigned char*)io->nbr_feat + (size_t)t * slot_bytes(h, IO_NBR_FEAT));
+    const int32_t* cnt = (const int32_t*)((const unsigned char*)io->nbr_cnt + (size_t)t * slot_bytes(h, IO_NBR_CNT));
+    int st = act(t, obs, feat, cnt, const_cast<void*>(cur.actions));
     if (st) return fail(h, st, gsm_policy_last_error());
     h->launches += 1;
     st = do_step(h, cur, (cudaStream_t)stream);
@@ -812,6 +798,69 @@ int gsm_collect(gsm_env* h, const gsm_policy_weights* w, int32_t n_steps, const 
     }
   }
   return GSM_OK;
+}
+
+// The checks both collects share after the handle's kind; GSM_OK or the status to return.
+int check_collect_io(gsm_env* h, const gsm_step_io* io, const char* who) {
+  if (!io->actions || !io->obs || !io->nbr_feat || !io->nbr_cnt)
+    return fail(h, GSM_ERR_INVALID_ARG, std::string(who) + " needs io.actions, io.obs, io.nbr_feat and io.nbr_cnt");
+  if (h->auto_reset && !io->done) return fail(h, GSM_ERR_INVALID_ARG, "auto-reset collect needs io.done");
+  return GSM_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int gsm_collect(gsm_env* h, const gsm_policy_weights* w, int32_t n_steps, const gsm_step_io* io,
+                float* logp, float* values, uint64_t seed, uint64_t first_step, int32_t greedy,
+                void* stream) {
+  if (!h || !io || !w || n_steps < 1) return GSM_ERR_INVALID_ARG;
+  if (!is_f32(h) || h->hp.action_mode != GSM_ACT_DISCRETE)
+    return fail(h, GSM_ERR_UNSUPPORTED, "gsm_collect needs a GSM_F32 handle with discrete actions");
+  if (w->n_actions != h->hp.n_actions)
+    return fail(h, GSM_ERR_INVALID_ARG, "gsm_collect: weights.n_actions != cfg.n_discrete_actions");
+  if (const int st = check_collect_io(h, io, "gsm_collect")) return st;
+  const int64_t rows = h->hp.n_envs * h->hp.N;
+  const int64_t slot_rows = (h->slot_envs ? h->slot_envs : h->hp.n_envs) * h->hp.N;
+  return collect_loop(h, n_steps, io, stream, [&](int t, const float* obs, const float* feat, const int32_t* cnt,
+                                                  void* actions) {
+    gsm_policy_io pio;
+    pio.obs = obs; pio.nbr_feat = feat; pio.nbr_cnt = cnt;
+    pio.actions = (int32_t*)actions;
+    pio.logp = logp ? logp + (size_t)t * slot_rows : nullptr;
+    pio.logits = nullptr;
+    pio.values = values ? values + (size_t)t * slot_rows * GSM_POLICY_VALUE_HEADS : nullptr;
+    pio.n_rows = rows;
+    pio.row_offset = (uint64_t)h->hp.env_offset * (uint64_t)h->hp.N;
+    pio.seed = seed; pio.step = first_step + (uint64_t)t;
+    pio.max_nbrs = h->hp.K; pio.greedy = greedy;
+    return gsm_policy_act(w, &pio, h->device, stream);
+  });
+}
+
+int gsm_collect_gauss(gsm_env* h, const gsm_policy_gauss_weights* w, int32_t n_steps, const gsm_step_io* io,
+                      float* logp, float* values, uint64_t seed, uint64_t first_step, int32_t greedy,
+                      void* stream) {
+  if (!h || !io || !w || n_steps < 1) return GSM_ERR_INVALID_ARG;
+  if (!is_f32(h) || h->hp.action_mode != GSM_ACT_CONTINUOUS)
+    return fail(h, GSM_ERR_UNSUPPORTED, "gsm_collect_gauss needs a GSM_F32 handle with continuous actions");
+  if (const int st = check_collect_io(h, io, "gsm_collect_gauss")) return st;
+  const int64_t rows = h->hp.n_envs * h->hp.N;
+  const int64_t slot_rows = (h->slot_envs ? h->slot_envs : h->hp.n_envs) * h->hp.N;
+  return collect_loop(h, n_steps, io, stream, [&](int t, const float* obs, const float* feat, const int32_t* cnt,
+                                                  void* actions) {
+    gsm_policy_gauss_io pio;
+    pio.obs = obs; pio.nbr_feat = feat; pio.nbr_cnt = cnt;
+    pio.actions = (float*)actions;
+    pio.logp = logp ? logp + (size_t)t * slot_rows : nullptr;
+    pio.mean = nullptr;
+    pio.values = values ? values + (size_t)t * slot_rows * GSM_POLICY_VALUE_HEADS : nullptr;
+    pio.n_rows = rows;
+    pio.row_offset = (uint64_t)h->hp.env_offset * (uint64_t)h->hp.N;
+    pio.seed = seed; pio.step = first_step + (uint64_t)t;
+    pio.max_nbrs = h->hp.K; pio.greedy = greedy;
+    return gsm_policy_act_gauss(w, &pio, h->device, stream);
+  });
 }
 
 int64_t gsm_kernel_launches(const gsm_env* h) { return h ? h->launches : 0; }

@@ -10,6 +10,8 @@
 //   a_r = softmax_r(w_a . m_r + b_a)                        masked to the cnt valid rows
 //   z   = W_h [e ; sum_r a_r m_r] + b_h                     [n_actions] logits
 //   action = argmax_k (z_k + Gumbel_k),  Gumbel from Philox4x32-10 keyed like the env resets.
+// For continuous-action worlds the same embedding feeds a diagonal Gaussian head (SPEC.md §10b / §12b,
+// HeadKind below): action = W_mu h + b_mu + exp(log_std) eps, eps by Box-Muller on the same Philox stream.
 //
 // Design for sm_100a (details in front of graph_actor_kernel below): a block owns 128 agents; the
 // ego branch runs as packed FFMA2 over agent pairs, the block's VALID neighbour rows are flattened
@@ -29,6 +31,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <type_traits>
 
 #include "../../include/gsmarl_b200.h"
 
@@ -48,12 +51,42 @@ struct PolicyParams {                 // kernel-parameter image of gsm_policy_we
   float att_b;
 };
 
-struct PolicyIO {
+// Head kinds (SPEC.md §10 / §10b).  The embedding h = [e; sum_r a_r m_r] and everything that computes
+// it are shared; the kind selects the weights' image, the action type and the epilogue.
+//   HEAD_CAT:   NA logits, categorical sample (Gumbel-max), int32 action.
+//   HEAD_GAUSS: NA = GSM_POLICY_GAUSS_DIM means, diagonal Gaussian with a state-independent log_std,
+//               float action [2] = mean + exp(log_std) eps (Box-Muller), no clamping.
+enum HeadKind { HEAD_CAT = 0, HEAD_GAUSS = 1 };
+constexpr int GD = GSM_POLICY_GAUSS_DIM;
+
+struct GaussParams {                  // kernel-parameter image of gsm_policy_gauss_weights
+  float ego_w[H][GSM_OBS_DIM];
+  float ego_b[H];
+  float nbr_w[H][GSM_NBR_FEAT_DIM];
+  float nbr_b[H];
+  float att_w[H];
+  // rows 0..GD-1: the means; rows GD, GD+1: the two critics
+  float head_w[GD + GSM_POLICY_VALUE_HEADS][2 * H];
+  float head_b[GD + GSM_POLICY_VALUE_HEADS];
+  float att_b;
+  float log_std[GD];
+};
+
+template <int KIND> struct Head;
+template <> struct Head<HEAD_CAT> { using Params = PolicyParams; using Act = int32_t; };
+template <> struct Head<HEAD_GAUSS> { using Params = GaussParams; using Act = float; };
+
+template <int KIND> struct ActorIO {
   const float* obs; const float* nbr_feat; const int32_t* nbr_cnt;
-  int32_t* actions; float* logp; float* logits; float* values;
+  typename Head<KIND>::Act* actions;   // [n_rows] (categorical) or [n_rows][GD] (Gaussian)
+  float* logp;
+  float* dist;                         // [n_rows][NA]: the logits or the means; NULL = skip
+  float* values;
   int64_t n_rows; uint64_t row_offset, seed, step;
   int K, greedy;
 };
+using PolicyIO = ActorIO<HEAD_CAT>;
+using GaussIO = ActorIO<HEAD_GAUSS>;
 
 __device__ __forceinline__ void philox_p(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                          uint32_t k0, uint32_t k1, uint32_t out[4]) {
@@ -66,6 +99,33 @@ __device__ __forceinline__ void philox_p(uint32_t c0, uint32_t c1, uint32_t c2, 
     k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
   }
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
+
+// the categorical sampler's map of a Philox word to (0, 1), below
+__device__ __forceinline__ float unit_open(uint32_t x) {
+  return (float)(x >> 9) * 1.1920928955078125e-7f + 5.9604644775390625e-8f;
+}
+
+// SPEC.md §10b: log N(a; mu, exp(log_std)^2) summed over the two dimensions, with
+// delta_d = (a_d - mu_d) exp(-log_std_d) returned for the backward.  The actor and the learner call
+// this ONE function on the STORED action, and every rounding is explicit (no contraction that could
+// differ between the call sites), so what collect wrote and what evaluate returns are bit-identical.
+// A non-finite action gives NaN: a - a is 0 for every finite a and NaN otherwise.
+__device__ __forceinline__ float gauss_logp(float a0, float a1, float mu0, float mu1, float ls0, float ls1,
+                                            float& d0, float& d1) {
+  constexpr float LOG_2PI = 1.8378770664093453f;
+  d0 = __fmul_rn(__fsub_rn(a0, mu0), expf(-ls0));
+  d1 = __fmul_rn(__fsub_rn(a1, mu1), expf(-ls1));
+  const float t0 = __fsub_rn(__fmul_rn(-0.5f, __fmul_rn(d0, d0)), ls0);
+  const float t1 = __fsub_rn(__fmul_rn(-0.5f, __fmul_rn(d1, d1)), ls1);
+  const float fin = __fadd_rn(__fsub_rn(a0, a0), __fsub_rn(a1, a1));
+  return __fadd_rn(__fsub_rn(__fadd_rn(t0, t1), LOG_2PI), fin);
+}
+
+// entropy of the diagonal Gaussian: sum_d log_std_d + 1/2 (1 + log 2 pi)
+__device__ __forceinline__ float gauss_entropy(float ls0, float ls1) {
+  constexpr float HALF_LOG_2PIE = 1.4189385332046727f;
+  return __fadd_rn(__fadd_rn(ls0, HALF_LOG_2PIE), __fadd_rn(ls1, HALF_LOG_2PIE));
 }
 
 // NV = 0: actor only; NV = GSM_POLICY_VALUE_HEADS: the critics ride along as NV more rows of the head
@@ -90,9 +150,11 @@ __device__ __forceinline__ void philox_p(uint32_t c0, uint32_t c1, uint32_t c2, 
 // re-assembles every (row 0, row 1) operand pair with two MOVs per FFMA2.
 __device__ __forceinline__ float2 bc(float w) { return make_float2(w, w); }
 
-template <int NA, int NV>
+//
+// KIND (HeadKind) changes only the epilogue after the z rows are complete: NA logits or NA = GD means.
+template <int NA, int NV, int KIND>
 __global__ void __launch_bounds__(128)
-graph_actor_kernel(const __grid_constant__ PolicyParams w, const __grid_constant__ PolicyIO io) {
+graph_actor_kernel(const __grid_constant__ typename Head<KIND>::Params w, const __grid_constant__ ActorIO<KIND> io) {
   constexpr int NZ = NA + NV, AG = 128, RS = NZ + 1, CH = RS <= 10 ? 1024 : 512;   // static smem <= 48 KB
   __shared__ int s_pre[AG + 1];
   __shared__ int s_wtot[4];
@@ -228,9 +290,33 @@ graph_actor_kernel(const __grid_constant__ PolicyParams w, const __grid_constant
     for (int v = 0; v < NV; v++) io.values[i * NV + v] = z[NA + v];
   }
 
-  if (io.logits) {
+  if (io.dist) {
 #pragma unroll
-    for (int a = 0; a < NA; a++) io.logits[i * NA + a] = z[a];
+    for (int a = 0; a < NA; a++) io.dist[i * NA + a] = z[a];
+  }
+
+  if constexpr (KIND == HEAD_GAUSS) {
+    static_assert(NA == GD, "the Gaussian head has GD means");
+    // sample: Box-Muller on words 0, 1 of one Philox block, counter (row lo, row hi, step, 0x80000000)
+    float a0 = z[0], a1 = z[1];
+    if (!io.greedy) {
+      const uint64_t g = io.row_offset + (uint64_t)i;
+      uint32_t r[4];
+      philox_p((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)io.step, 0x80000000u,
+               (uint32_t)io.seed, (uint32_t)(io.seed >> 32), r);
+      const float rho = sqrtf(-2.f * logf(unit_open(r[0])));
+      float sn, cs;
+      sincospif(2.f * unit_open(r[1]), &sn, &cs);      // 2 u is exact
+      a0 = fmaf(expf(w.log_std[0]), rho * cs, z[0]);
+      a1 = fmaf(expf(w.log_std[1]), rho * sn, z[1]);
+    }
+    io.actions[i * GD] = a0;
+    io.actions[i * GD + 1] = a1;
+    if (io.logp) {
+      float d0, d1;
+      io.logp[i] = gauss_logp(a0, a1, z[0], z[1], w.log_std[0], w.log_std[1], d0, d1);
+    }
+    return;                             // (the categorical epilogue below is unreachable here)
   }
 
   // sample: Gumbel-max, one Philox block per 4 actions; counter (row lo, row hi, step, block)
@@ -337,18 +423,22 @@ constexpr int BWD_AG = 64;                 // rows per tile = threads per backwa
 constexpr int BWD_MAX_BLOCKS = 148 * 6;    // one wave at 6 blocks/SM (168 registers); a constant, NOT the device's SM count
 static_assert(BWD_AG == H, "phase B maps one thread to one hidden unit");
 
-template <int NA> struct PV {               // offsets into the parameter vector
+template <int NA, int KIND> struct PV {     // offsets into the parameter vector
+  // the Gaussian's log_std [NA] sits between the head and the critics (parameters_to_vector order)
   static constexpr int EW = 0, EB = EW + H * GSM_OBS_DIM, NW = EB + H, NB = NW + H * GSM_NBR_FEAT_DIM,
-                       AW = NB + H, AB = AW + H, HW = AB + 1, HB = HW + NA * 2 * H, VW = HB + NA,
-                       VB = VW + V2 * 2 * H, N = VB + V2;
+                       AW = NB + H, AB = AW + H, HW = AB + 1, HB = HW + NA * 2 * H, LS = HB + NA,
+                       VW = LS + (KIND == HEAD_GAUSS ? NA : 0), VB = VW + V2 * 2 * H, N = VB + V2;
   static __host__ __device__ constexpr int row(int a) { return a < NA ? HW + a * 2 * H : VW + (a - NA) * 2 * H; }
   static __host__ __device__ constexpr int bias(int a) { return a < NA ? HB + a : VB + (a - NA); }
 };
-static_assert(PV<5>::N == GSM_POLICY_N_PARAMS(5) && PV<5>::N == 1864 && PV<9>::N == 2380, "vector size");
+static_assert(PV<5, HEAD_CAT>::N == GSM_POLICY_N_PARAMS(5) && PV<5, HEAD_CAT>::N == 1864 &&
+              PV<9, HEAD_CAT>::N == 2380, "vector size");
+static_assert(PV<GD, HEAD_GAUSS>::N == GSM_POLICY_GAUSS_N_PARAMS && GSM_POLICY_GAUSS_N_PARAMS == 1479, "vector size");
 
-struct EvalArgs {
+template <int KIND> struct EvalArgs {
   const float* params; const float* obs; const float* nbr_feat; const int32_t* nbr_cnt;
-  const int32_t* actions; const int64_t* rows;
+  const typename Head<KIND>::Act* actions;   // [src_rows] or [src_rows][GD]
+  const int64_t* rows;
   float* logp; float* entropy; float* values;                 // forward outputs
   const float* d_logp; const float* d_entropy; const float* d_values;   // backward inputs
   float* ws;                                                  // backward: [gridDim.x][N] partials
@@ -357,9 +447,9 @@ struct EvalArgs {
 };
 
 // e-branch of graph_actor_kernel: z[a] = b[a] + sum_j W[a][j] relu(W_e obs + b_e)_j, same chains
-template <int NA>
+template <int NA, int KIND>
 __device__ __forceinline__ void ego_logits(const float* W, const float* o, float (&z)[NA + V2]) {
-  using P = PV<NA>;
+  using P = PV<NA, KIND>;
   const float o0 = o[0], o1 = o[1], o2 = o[2], o3 = o[3], o4 = o[4], o5 = o[5];
 #pragma unroll
   for (int a = 0; a < NA + V2; a++) z[a] = W[P::bias(a)];
@@ -376,9 +466,9 @@ __device__ __forceinline__ void ego_logits(const float* W, const float* o, float
 }
 
 // one valid neighbour row: returns the attention score t_r, hr[a] = W[a][H:] . m_r (phase 2 chains)
-template <int NA>
+template <int NA, int KIND>
 __device__ __forceinline__ float nbr_row(const float* W, const float* f, float (&hr)[NA + V2]) {
-  using P = PV<NA>;
+  using P = PV<NA, KIND>;
   // an offset the compiler cannot see through: without it the ~1200 shared-memory weight loads are
   // hoisted out of the caller's row loop as loop invariants and spilled to local memory
   int off = 0;
@@ -404,16 +494,16 @@ __device__ __forceinline__ float nbr_row(const float* W, const float* f, float (
 
 // The forward of one row in graph_actor_kernel's order.  Out: z = [logits; values]; mx, s: the
 // softmax max and sum over the valid rows; acc[a] * (1 / s) = sum_r a_r hr_r[a] (cnt > 0).
-template <int NA>
+template <int NA, int KIND>
 __device__ __forceinline__ void row_forward(const float* W, const float* o, const float* f, int cnt,
                                             float (&z)[NA + V2], float (&acc)[NA + V2], float& mx, float& s) {
-  ego_logits<NA>(W, o, z);
+  ego_logits<NA, KIND>(W, o, z);
   mx = -__int_as_float(0x7f800000); s = 0.f;
 #pragma unroll
   for (int a = 0; a < NA + V2; a++) acc[a] = 0.f;
   for (int r = 0; r < cnt; r++) {
     float hr[NA + V2];
-    const float t = nbr_row<NA>(W, f + r * GSM_NBR_FEAT_DIM, hr);
+    const float t = nbr_row<NA, KIND>(W, f + r * GSM_NBR_FEAT_DIM, hr);
     const float nm = fmaxf(mx, t);
     const float sc = expf(mx - nm), pw = expf(t - nm);     // first row: exp(-inf) = 0
     s = fmaf(s, sc, pw);
@@ -446,9 +536,10 @@ __device__ __forceinline__ float row_logp(const float (&z)[NA + V2], int act, fl
 
 __device__ __forceinline__ int clamp_cnt(int c, int K) { return c < 0 ? 0 : (c > K ? K : c); }
 
-template <int NA>
-__global__ void __launch_bounds__(128) policy_eval_kernel(const __grid_constant__ EvalArgs p) {
-  constexpr int NP = PV<NA>::N;
+template <int NA, int KIND>
+__global__ void __launch_bounds__(128) policy_eval_kernel(const __grid_constant__ EvalArgs<KIND> p) {
+  using P = PV<NA, KIND>;
+  constexpr int NP = P::N;
   __shared__ float s_w[NP];
   for (int k = threadIdx.x; k < NP; k += blockDim.x) s_w[k] = p.params[k];
   __syncthreads();
@@ -457,37 +548,52 @@ __global__ void __launch_bounds__(128) policy_eval_kernel(const __grid_constant_
   const int64_t src = p.rows ? p.rows[i] : i;
   const int cnt = clamp_cnt(p.nbr_cnt[src], p.K);
   float z[NA + V2], acc[NA + V2], mx, s;
-  row_forward<NA>(s_w, p.obs + src * GSM_OBS_DIM, p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM, cnt, z, acc, mx, s);
+  row_forward<NA, KIND>(s_w, p.obs + src * GSM_OBS_DIM, p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM, cnt, z, acc, mx, s);
   if (p.values) {
 #pragma unroll
     for (int v = 0; v < V2; v++) p.values[i * V2 + v] = z[NA + v];
   }
-  float zm, se;
-  const float lp = row_logp<NA>(z, p.actions[src], zm, se);
-  if (p.logp) p.logp[i] = lp;
-  if (p.entropy) {                     // log(se) - sum_k p_k (z_k - zm) = logsumexp(z) - sum_k p_k z_k
-    const float inv = 1.f / se;
-    float pz = 0.f;
+  if constexpr (KIND == HEAD_GAUSS) {
+    const float ls0 = s_w[P::LS], ls1 = s_w[P::LS + 1];
+    float d0, d1;
+    const float lp = gauss_logp(p.actions[src * GD], p.actions[src * GD + 1], z[0], z[1], ls0, ls1, d0, d1);
+    if (p.logp) p.logp[i] = lp;
+    if (p.entropy) p.entropy[i] = gauss_entropy(ls0, ls1);
+  } else {
+    float zm, se;
+    const float lp = row_logp<NA>(z, p.actions[src], zm, se);
+    if (p.logp) p.logp[i] = lp;
+    if (p.entropy) {                     // log(se) - sum_k p_k (z_k - zm) = logsumexp(z) - sum_k p_k z_k
+      const float inv = 1.f / se;
+      float pz = 0.f;
 #pragma unroll
-    for (int a = 0; a < NA; a++) pz = fmaf(expf(z[a] - zm) * inv, z[a] - zm, pz);
-    p.entropy[i] = logf(se) - pz;
+      for (int a = 0; a < NA; a++) pz = fmaf(expf(z[a] - zm) * inv, z[a] - zm, pz);
+      p.entropy[i] = logf(se) - pz;
+    }
   }
 }
 
-template <int NA> struct BwdSmem {
-  float w[PV<NA>::N];
+template <int NA, int KIND> struct BwdSmem {
+  float w[PV<NA, KIND>::N];
   float obs[BWD_AG][GSM_OBS_DIM];
   float dz[BWD_AG][NA + V2];
   float dsum[BWD_AG];                  // sum_r ds_r of the row (db_a)
   int cnt[BWD_AG];
   long long src[BWD_AG];
 };
+// the Gaussian adds each row's two dlog_std terms (summed by threads NZ, NZ + 1 in phase B); the
+// categorical layout stays as it is
+template <int NA> struct BwdSmemGauss : BwdSmem<NA, HEAD_GAUSS> {
+  float dls[BWD_AG][GD];
+};
+template <int NA, int KIND>
+using BwdSmemOf = std::conditional_t<KIND == HEAD_GAUSS, BwdSmemGauss<NA>, BwdSmem<NA, KIND>>;
 
-template <int NA>
-__global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_constant__ EvalArgs p) {
-  constexpr int NZ = NA + V2, NP = PV<NA>::N;
-  using P = PV<NA>;
-  __shared__ BwdSmem<NA> sm;
+template <int NA, int KIND>
+__global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_constant__ EvalArgs<KIND> p) {
+  using P = PV<NA, KIND>;
+  constexpr int NZ = NA + V2, NP = P::N;
+  __shared__ BwdSmemOf<NA, KIND> sm;
   extern __shared__ float s_rows[];    // [BWD_AG][K][2]: (a_r, ds_r) of the valid rows; a float2 array
                                        // would round every kernel's static shared memory in this file up to 16 B
   const int tid = threadIdx.x;
@@ -513,9 +619,15 @@ __global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_co
       const float* o = p.obs + src * GSM_OBS_DIM;
       const float* f = p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM;
       float z[NZ], acc[NZ], mx, s;
-      row_forward<NA>(W, o, f, cnt, z, acc, mx, s);
+      row_forward<NA, KIND>(W, o, f, cnt, z, acc, mx, s);
+      // The categorical dz stays at this scope for BOTH kinds, on purpose: guarded by
+      // `if constexpr (KIND == HEAD_CAT)` (or nested in an if-constexpr / else) it changes the register
+      // allocation and SASS of the categorical instances, which must stay as they were.  For the
+      // Gaussian it is dead code: act is the constant 0, every dz[a < NA] it writes is rewritten by the
+      // Gaussian block below and nothing else reads its values, so the compiler removes it (same
+      // registers as the nested form).  Only dlp and dent are shared with the Gaussian block.
       float zm, se;
-      const int act = p.actions[src];
+      const int act = KIND == HEAD_CAT ? (int)p.actions[src] : 0;
       const float lp = row_logp<NA>(z, act, zm, se);
       const float dlp = p.d_logp ? p.d_logp[i] : 0.f, dent = p.d_entropy ? p.d_entropy[i] : 0.f;
       const float lse = zm + logf(se), inv_se = 1.f / se;
@@ -529,6 +641,20 @@ __global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_co
 #pragma unroll
       for (int a = 0; a < NA; a++)
         dz[a] = dlp * ((act == a ? 1.f : 0.f) - pr[a] + bad) - dent * pr[a] * ((z[a] - lse) + ent);
+      if constexpr (KIND == HEAD_GAUSS) {
+        // SPEC.md §12b: dmu_d = d_logp delta_d exp(-log_std_d);
+        // dlog_std_d = d_logp (delta_d^2 - 1) + d_entropy.  A non-finite action (NaN logp) gives a NaN
+        // gradient exactly where d_logp != 0; where d_logp == 0 the action does not enter it.
+        const float ls0 = W[P::LS], ls1 = W[P::LS + 1];
+        float d0, d1;
+        const float glp = gauss_logp(p.actions[src * GD], p.actions[src * GD + 1], z[0], z[1], ls0, ls1, d0, d1);
+        const bool use = dlp != 0.f;
+        const float gbad = (use && glp != glp) ? __int_as_float(0x7fc00000) : 0.f;
+        dz[0] = use ? dlp * d0 * expf(-ls0) + gbad : 0.f;
+        dz[1] = use ? dlp * d1 * expf(-ls1) + gbad : 0.f;
+        sm.dls[tid][0] = (use ? dlp * fmaf(d0, d0, -1.f) + gbad : 0.f) + dent;
+        sm.dls[tid][1] = (use ? dlp * fmaf(d1, d1, -1.f) + gbad : 0.f) + dent;
+      }
 #pragma unroll
       for (int v = 0; v < V2; v++) dz[NA + v] = p.d_values ? p.d_values[i * V2 + v] : 0.f;
       float dsum = 0.f;
@@ -540,7 +666,7 @@ __global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_co
         float* pr_rows = s_rows + 2 * tid * p.K;
         for (int r = 0; r < cnt; r++) {  // second pass: the same t_r, hr_r as the first
           float hr[NZ];
-          const float t = nbr_row<NA>(W, f + r * GSM_NBR_FEAT_DIM, hr);
+          const float t = nbr_row<NA, KIND>(W, f + r * GSM_NBR_FEAT_DIM, hr);
           const float ar = expf(t - mx) * inv;
           float q = 0.f;
 #pragma unroll
@@ -611,6 +737,7 @@ __global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_co
         }
         if (j < NZ) gsc += sm.dz[ag][j];
         else if (j == H - 1) gsc += sm.dsum[ag];
+        else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) gsc += sm.dls[ag][j - NZ]; }
       }
     }
     __syncthreads();                     // before the next tile overwrites the row state
@@ -628,6 +755,7 @@ __global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_co
   for (int a = 0; a < NZ; a++) { out[P::row(a) + j] = ghe[a]; out[P::row(a) + H + j] = ghg[a]; }
   if (j < NZ) out[j < NA ? P::HB + j : P::VB + (j - NA)] = gsc;
   else if (j == H - 1) out[P::AB] = gsc;
+  else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) out[P::LS + (j - NZ)] = gsc; }
 }
 
 // grad[k] = sum of the G partials in a fixed order: warp w sums partials w, w + 8, ... (lane = k),
@@ -657,30 +785,35 @@ static int64_t bwd_blocks(int64_t n_rows) {
   return tiles < BWD_MAX_BLOCKS ? tiles : BWD_MAX_BLOCKS;
 }
 
-static int n_params(int n_actions) { return n_actions == 5 ? PV<5>::N : PV<9>::N; }
+static int n_params(int n_actions) { return n_actions == 5 ? PV<5, HEAD_CAT>::N : PV<9, HEAD_CAT>::N; }
 
-static int launch_evaluate(const EvalArgs& a, int n_actions, cudaStream_t st) {
+static int launch_evaluate(const EvalArgs<HEAD_CAT>& a, int n_actions, cudaStream_t st) {
   const unsigned grid = (unsigned)((a.n_rows + 127) / 128);
-  if (n_actions == 5) policy_eval_kernel<5><<<grid, 128, 0, st>>>(a);
-  else policy_eval_kernel<9><<<grid, 128, 0, st>>>(a);
+  if (n_actions == 5) policy_eval_kernel<5, HEAD_CAT><<<grid, 128, 0, st>>>(a);
+  else policy_eval_kernel<9, HEAD_CAT><<<grid, 128, 0, st>>>(a);
   return (int)cudaGetLastError();
 }
 
-template <int NA>
-static int launch_backward_na(EvalArgs a, float* grad, cudaStream_t st) {
+static int launch_evaluate_gauss(const EvalArgs<HEAD_GAUSS>& a, cudaStream_t st) {
+  policy_eval_kernel<GD, HEAD_GAUSS><<<(unsigned)((a.n_rows + 127) / 128), 128, 0, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+template <int NA, int KIND>
+static int launch_backward_na(EvalArgs<KIND> a, float* grad, cudaStream_t st) {
   const int64_t G = bwd_blocks(a.n_rows);
   a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
   const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
-  if (sizeof(BwdSmem<NA>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
-    const cudaError_t e = cudaFuncSetAttribute(policy_backward_kernel<NA>,
+  if (sizeof(BwdSmemOf<NA, KIND>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
+    const cudaError_t e = cudaFuncSetAttribute(policy_backward_kernel<NA, KIND>,
                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) {            // max_nbrs beyond the block's shared memory: report it here and clear
       cudaGetLastError();              // it, or the next launch's cudaGetLastError() would report it again
       return (int)e;
     }
   }
-  policy_backward_kernel<NA><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
-  policy_grad_reduce_kernel<<<(PV<NA>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA>::N, grad);
+  policy_backward_kernel<NA, KIND><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
+  policy_grad_reduce_kernel<<<(PV<NA, KIND>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA, KIND>::N, grad);
   return (int)cudaGetLastError();
 }
 
@@ -690,11 +823,19 @@ static int launch_actor(const PolicyParams& w, const PolicyIO& io, int n_actions
   const int64_t grid = (io.n_rows + block - 1) / block;
   constexpr int V = GSM_POLICY_VALUE_HEADS;
   const unsigned gd = (unsigned)grid;
-  if (n_actions == 5 && !io.values) graph_actor_kernel<5, 0><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 5) graph_actor_kernel<5, V><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 9 && !io.values) graph_actor_kernel<9, 0><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 9) graph_actor_kernel<9, V><<<gd, block, 0, st>>>(w, io);
+  if (n_actions == 5 && !io.values) graph_actor_kernel<5, 0, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
+  else if (n_actions == 5) graph_actor_kernel<5, V, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
+  else if (n_actions == 9 && !io.values) graph_actor_kernel<9, 0, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
+  else if (n_actions == 9) graph_actor_kernel<9, V, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
   else return -1;
+  return (int)cudaGetLastError();
+}
+
+static int launch_actor_gauss(const GaussParams& w, const GaussIO& io, cudaStream_t st) {
+  if (io.n_rows == 0) return 0;
+  const unsigned gd = (unsigned)((io.n_rows + 127) / 128);
+  if (!io.values) graph_actor_kernel<GD, 0, HEAD_GAUSS><<<gd, 128, 0, st>>>(w, io);
+  else graph_actor_kernel<GD, GSM_POLICY_VALUE_HEADS, HEAD_GAUSS><<<gd, 128, 0, st>>>(w, io);
   return (int)cudaGetLastError();
 }
 
@@ -750,24 +891,45 @@ int pfailf(int status, const char* who, const char* msg) {
   snprintf(g_policy_err, sizeof(g_policy_err), "%s: %s", who, msg);
   return status;
 }
-// The checks gsm_policy_evaluate and gsm_policy_backward share; none touches the device.
-int check_eval_io(const gsm_policy_eval_io* io, const char* who) {
+// The checks the evaluate and backward entry points of both heads share; none touches the device.
+template <class IO> int check_eval_io_t(const IO* io, const char* who) {
   if (!io) return pfailf(GSM_ERR_INVALID_ARG, who, "io is NULL");
-  if (io->struct_size != sizeof(gsm_policy_eval_io)) return pfailf(GSM_ERR_ABI, who, "io.struct_size mismatch");
-  if (io->n_actions != 5 && io->n_actions != 9)
-    return pfailf(GSM_ERR_UNSUPPORTED, who, "compiled learner instances exist for n_actions 5 and 9 only");
+  if (io->struct_size != sizeof(IO)) return pfailf(GSM_ERR_ABI, who, "io.struct_size mismatch");
+  if constexpr (std::is_same_v<IO, gsm_policy_eval_io>) {
+    if (io->n_actions != 5 && io->n_actions != 9)
+      return pfailf(GSM_ERR_UNSUPPORTED, who, "compiled learner instances exist for n_actions 5 and 9 only");
+  } else {
+    if (io->action_dim != GSM_POLICY_GAUSS_DIM)
+      return pfailf(GSM_ERR_UNSUPPORTED, who, "the Gaussian learner instance has action_dim 2 only");
+  }
   if (!io->params || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
     return pfailf(GSM_ERR_INVALID_ARG, who, "params, obs, nbr_feat, nbr_cnt and actions are required");
   if (io->n_rows < 0 || io->max_nbrs < 1) return pfailf(GSM_ERR_INVALID_ARG, who, "bad n_rows / max_nbrs");
   if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfailf(GSM_ERR_INVALID_ARG, who, "n_rows too large");
   return GSM_OK;
 }
-gsm::EvalArgs eval_args(const gsm_policy_eval_io* io) {
-  gsm::EvalArgs a{};
+int check_eval_io(const gsm_policy_eval_io* io, const char* who) { return check_eval_io_t(io, who); }
+template <int KIND, class IO> gsm::EvalArgs<KIND> eval_args(const IO* io) {
+  gsm::EvalArgs<KIND> a{};
   a.params = io->params; a.obs = io->obs; a.nbr_feat = io->nbr_feat; a.nbr_cnt = io->nbr_cnt;
   a.actions = io->actions; a.rows = io->rows;
   a.n_rows = io->n_rows; a.K = io->max_nbrs;
   return a;
+}
+int pack_gauss(const gsm_policy_gauss_weights* w, gsm::GaussParams* p) {
+  if (!w) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_gauss: weights is NULL");
+  if (w->struct_size != sizeof(gsm_policy_gauss_weights))
+    return pfail(GSM_ERR_ABI, "gsm_policy_gauss: weights.struct_size mismatch");
+  static_assert(sizeof(p->ego_w) == sizeof(w->ego_w) && sizeof(p->log_std) == sizeof(w->log_std), "layout");
+  std::memcpy(p->ego_w, w->ego_w, sizeof(p->ego_w));   std::memcpy(p->ego_b, w->ego_b, sizeof(p->ego_b));
+  std::memcpy(p->nbr_w, w->nbr_w, sizeof(p->nbr_w));   std::memcpy(p->nbr_b, w->nbr_b, sizeof(p->nbr_b));
+  std::memcpy(p->att_w, w->att_w, sizeof(p->att_w));   p->att_b = w->att_b;
+  std::memcpy(p->head_w, w->mean_w, sizeof(w->mean_w));                        // means, then the critics
+  std::memcpy(p->head_w[GSM_POLICY_GAUSS_DIM], w->value_w, sizeof(w->value_w));
+  std::memcpy(p->head_b, w->mean_b, sizeof(w->mean_b));
+  std::memcpy(&p->head_b[GSM_POLICY_GAUSS_DIM], w->value_b, sizeof(w->value_b));
+  std::memcpy(p->log_std, w->log_std, sizeof(p->log_std));
+  return GSM_OK;
 }
 }  // namespace
 
@@ -779,7 +941,7 @@ int gsm_policy_evaluate(const gsm_policy_eval_io* io, int device, void* stream) 
   if (const int ds = check_device(device, "gsm_policy_evaluate")) return ds;
   DevGuard guard(device);
   if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_evaluate: cudaSetDevice failed");
-  gsm::EvalArgs a = eval_args(io);
+  gsm::EvalArgs<gsm::HEAD_CAT> a = eval_args<gsm::HEAD_CAT>(io);
   a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
   const int e = gsm::launch_evaluate(a, io->n_actions, (cudaStream_t)stream);
   if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
@@ -806,11 +968,11 @@ int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const
   if (const int ds = check_device(device, who)) return ds;
   DevGuard guard(device);
   if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_backward: cudaSetDevice failed");
-  gsm::EvalArgs a = eval_args(io);
+  gsm::EvalArgs<gsm::HEAD_CAT> a = eval_args<gsm::HEAD_CAT>(io);
   a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
   a.ws = (float*)workspace;
-  const int e = io->n_actions == 5 ? gsm::launch_backward_na<5>(a, grad, (cudaStream_t)stream)
-                                   : gsm::launch_backward_na<9>(a, grad, (cudaStream_t)stream);
+  const int e = io->n_actions == 5 ? gsm::launch_backward_na<5, gsm::HEAD_CAT>(a, grad, (cudaStream_t)stream)
+                                   : gsm::launch_backward_na<9, gsm::HEAD_CAT>(a, grad, (cudaStream_t)stream);
   if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
   return GSM_OK;
 }
@@ -830,10 +992,72 @@ int gsm_policy_act(const gsm_policy_weights* w, const gsm_policy_io* io, int dev
   if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_act: cudaSetDevice failed");
   gsm::PolicyIO k;
   k.obs = io->obs; k.nbr_feat = io->nbr_feat; k.nbr_cnt = io->nbr_cnt;
-  k.actions = io->actions; k.logp = io->logp; k.logits = io->logits; k.values = io->values;
+  k.actions = io->actions; k.logp = io->logp; k.dist = io->logits; k.values = io->values;
   k.n_rows = io->n_rows; k.row_offset = io->row_offset; k.seed = io->seed; k.step = io->step;
   k.K = io->max_nbrs; k.greedy = io->greedy;
   const int e = gsm::launch_actor(p, k, w->n_actions, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
+
+int gsm_policy_act_gauss(const gsm_policy_gauss_weights* w, const gsm_policy_gauss_io* io, int device,
+                         void* stream) {
+  gsm::GaussParams p;
+  int st = pack_gauss(w, &p);
+  if (st) return st;
+  if (!io || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
+    return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: obs, nbr_feat, nbr_cnt and actions are required");
+  if (io->n_rows < 0 || io->max_nbrs < 1) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: bad n_rows / max_nbrs");
+  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: n_rows too large");
+  if (const int ds = check_device(device, "gsm_policy_act_gauss")) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_act_gauss: cudaSetDevice failed");
+  gsm::GaussIO k;
+  k.obs = io->obs; k.nbr_feat = io->nbr_feat; k.nbr_cnt = io->nbr_cnt;
+  k.actions = io->actions; k.logp = io->logp; k.dist = io->mean; k.values = io->values;
+  k.n_rows = io->n_rows; k.row_offset = io->row_offset; k.seed = io->seed; k.step = io->step;
+  k.K = io->max_nbrs; k.greedy = io->greedy;
+  const int e = gsm::launch_actor_gauss(p, k, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
+
+int gsm_policy_evaluate_gauss(const gsm_policy_gauss_eval_io* io, int device, void* stream) {
+  const char* who = "gsm_policy_evaluate_gauss";
+  if (const int st = check_eval_io_t(io, who)) return st;
+  if (io->n_rows == 0) return GSM_OK;
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_evaluate_gauss: cudaSetDevice failed");
+  gsm::EvalArgs<gsm::HEAD_GAUSS> a = eval_args<gsm::HEAD_GAUSS>(io);
+  a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
+  const int e = gsm::launch_evaluate_gauss(a, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
+
+int64_t gsm_policy_backward_workspace_gauss(int64_t n_rows) {
+  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_policy_backward_workspace_gauss", "n_rows < 0");
+  return gsm::bwd_blocks(n_rows) * GSM_POLICY_GAUSS_N_PARAMS * (int64_t)sizeof(float);
+}
+
+int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d_logp, const float* d_entropy,
+                              const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
+                              int device, void* stream) {
+  const char* who = "gsm_policy_backward_gauss";
+  if (const int st = check_eval_io_t(io, who)) return st;
+  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
+  const int64_t need = gsm_policy_backward_workspace_gauss(io->n_rows);
+  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than gsm_policy_backward_workspace_gauss(n_rows)");
+  if (io->n_rows == 0) return GSM_OK;
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_backward_gauss: cudaSetDevice failed");
+  gsm::EvalArgs<gsm::HEAD_GAUSS> a = eval_args<gsm::HEAD_GAUSS>(io);
+  a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
+  a.ws = (float*)workspace;
+  const int e = gsm::launch_backward_na<gsm::GD, gsm::HEAD_GAUSS>(a, grad, (cudaStream_t)stream);
   if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
   return GSM_OK;
 }

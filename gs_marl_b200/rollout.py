@@ -143,20 +143,26 @@ def collect_fused(env: MultiAgentGraphConstrainEnv, actor, buf: GraphRolloutBuff
     """The same rollout with the actor forward + sampling as this library's kernel
     (`gsm_collect`: per step one actor launch and one env-step launch, enqueued from C with no
     Python or host sync in between; actions, log-probs and — with_values — the two critics'
-    predictions land in the buffer slots).  `actor` is a
-    `policy.GraphAttentionActor`.  With a `StreamShardedEnv` every sub-shard runs its own
+    predictions land in the buffer slots).  `actor` is a `policy.GraphAttentionActor` for a
+    discrete-action world or a `policy.GaussianGraphActor` (`gsm_collect_gauss`) for a continuous one.  With a `StreamShardedEnv` every sub-shard runs its own
     actor -> env-step chain on its own stream into its env slice of the buffer, so one shard's actor
     kernel (fp32-issue-bound) overlaps another's env step (HBM-bound).  graph=True captures the 2·T launches into a CUDA graph and
     returns it WITHOUT having advanced the env (replay runs the rollout from the env's current
     state and whatever slot 0 holds, with the Philox step counters and the weights baked in at
     capture: re-capture after an optimizer step)."""
+    mode, kind = env.world.action_mode, getattr(actor, "action_mode", None)
+    if kind is not None and kind != mode:       # other actors: the C side reports a mismatch (GSM_ERR_UNSUPPORTED)
+        raise ValueError(f"{type(actor).__name__} samples {kind} actions; the env's action_mode is "
+                         f"{mode!r} (use {'GaussianGraphActor' if mode == 'continuous' else 'GraphAttentionActor'})")
     w = actor.packed()
+    collect_fn = "gsm_collect_gauss" if isinstance(w, abi.GsmPolicyGaussWeights) else "gsm_collect"
     logp, values = buf.data["logp"], buf.data["values"]
     for sh in buf._shards:          # reset-on-done inside the loop follows the env's flag
         sh._check(sh.lib.gsm_set_auto_reset(sh._h, int(bool(env.auto_reset))))
 
+
     def enqueue():
-        buf._on_shards(lambda sh, j, st: sh._check(sh.lib.gsm_collect(
+        buf._on_shards(lambda sh, j, st: sh._check(getattr(sh.lib, collect_fn)(
             sh._h, C.byref(w), buf.T, C.byref(buf._io_all[j]),
             C.c_void_p(logp[0, buf._bounds[j][0]:].data_ptr()),
             C.c_void_p(values[0, buf._bounds[j][0]:].data_ptr()) if with_values else None, int(seed), int(first_step),

@@ -344,6 +344,80 @@ int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const
                         const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                         int device, void* stream);
 
+/* ---- Gaussian actor for GSM_ACT_CONTINUOUS worlds (SPEC.md §10b / §12b) ----------------------
+ * The same embedding h = [e ; sum_r a_r m_r] as above, with a diagonal Gaussian head:
+ *   mean = mean_w h + mean_b [2];  sigma = exp(log_std), log_std [2] a free parameter (not a function
+ *   of the state);  action = mean + sigma * eps, eps by Box-Muller from words 0 and 1 of
+ *   Philox4x32-10(key = seed, counter = (row lo, row hi, step, 0x80000000)) — or action = mean when
+ *   greedy != 0.  Actions are not clipped or squashed.
+ *   logp = sum_d (-1/2 delta_d^2 - log_std_d) - log(2 pi), delta_d = (a_d - mean_d) exp(-log_std_d)
+ *   (NaN for a non-finite action);  entropy = sum_d (log_std_d + 1/2 (1 + log 2 pi)).
+ * The learner's parameter vector is parameters_to_vector(GaussianGraphActor) order:
+ *   ego_w[64][6], ego_b[64], nbr_w[64][6], nbr_b[64], att_w[64], att_b, mean_w[2][128], mean_b[2],
+ *   log_std[2], value_w[2][128], value_b[2]   -> GSM_POLICY_GAUSS_N_PARAMS floats. */
+#define GSM_POLICY_GAUSS_DIM 2
+#define GSM_POLICY_GAUSS_N_PARAMS 1479
+
+typedef struct gsm_policy_gauss_weights {   /* HOST memory, row-major [out][in] */
+  uint32_t struct_size;          /* = sizeof(gsm_policy_gauss_weights); checked */
+  float ego_w[GSM_POLICY_HIDDEN][GSM_OBS_DIM];
+  float ego_b[GSM_POLICY_HIDDEN];
+  float nbr_w[GSM_POLICY_HIDDEN][GSM_NBR_FEAT_DIM];
+  float nbr_b[GSM_POLICY_HIDDEN];
+  float att_w[GSM_POLICY_HIDDEN];
+  float att_b;
+  float mean_w[GSM_POLICY_GAUSS_DIM][2 * GSM_POLICY_HIDDEN];
+  float mean_b[GSM_POLICY_GAUSS_DIM];
+  float log_std[GSM_POLICY_GAUSS_DIM];
+  float value_w[GSM_POLICY_VALUE_HEADS][2 * GSM_POLICY_HIDDEN];
+  float value_b[GSM_POLICY_VALUE_HEADS];
+} gsm_policy_gauss_weights;
+
+typedef struct gsm_policy_gauss_io {   /* gsm_policy_io with float actions and the mean; DEVICE pointers */
+  const float* obs;        /* [n_rows][GSM_OBS_DIM]                     */
+  const float* nbr_feat;   /* [n_rows][max_nbrs][GSM_NBR_FEAT_DIM]      */
+  const int32_t* nbr_cnt;  /* [n_rows]  valid rows (clamped to [0, max_nbrs]) */
+  float* actions;          /* [n_rows][GSM_POLICY_GAUSS_DIM] out        */
+  float* logp;             /* [n_rows]  out, log pi(action); NULL = skip */
+  float* mean;             /* [n_rows][GSM_POLICY_GAUSS_DIM] out; NULL = skip */
+  float* values;           /* [n_rows][GSM_POLICY_VALUE_HEADS] out; NULL = skip (actor-only kernel) */
+  int64_t n_rows;
+  uint64_t row_offset;     /* global index of row 0 (env_offset * N): sharding-invariant draws */
+  uint64_t seed, step;
+  int32_t max_nbrs;
+  int32_t greedy;
+} gsm_policy_gauss_io;
+
+int gsm_policy_act_gauss(const gsm_policy_gauss_weights* w, const gsm_policy_gauss_io* io, int device,
+                         void* stream);
+
+typedef struct gsm_policy_gauss_eval_io {   /* gsm_policy_eval_io with float actions; DEVICE pointers */
+  uint32_t struct_size;      /* = sizeof(gsm_policy_gauss_eval_io); checked                    */
+  int32_t action_dim;        /* GSM_POLICY_GAUSS_DIM                                           */
+  const float* params;       /* [GSM_POLICY_GAUSS_N_PARAMS]                                    */
+  const float* obs;          /* [src_rows][GSM_OBS_DIM]                                        */
+  const float* nbr_feat;     /* [src_rows][max_nbrs][GSM_NBR_FEAT_DIM]                         */
+  const int32_t* nbr_cnt;    /* [src_rows]  valid rows (clamped to [0, max_nbrs])              */
+  const float* actions;      /* [src_rows][GSM_POLICY_GAUSS_DIM]                               */
+  const int64_t* rows;       /* [n_rows] source row of row i (caller keeps it in range); NULL = i */
+  float* logp;               /* [n_rows] out; NULL = skip                                      */
+  float* entropy;            /* [n_rows] out; NULL = skip                                      */
+  float* values;             /* [n_rows][GSM_POLICY_VALUE_HEADS] out; NULL = skip              */
+  int64_t n_rows;
+  int32_t max_nbrs;
+  int32_t reserved;          /* 0 */
+} gsm_policy_gauss_eval_io;
+
+/* As gsm_policy_evaluate / gsm_policy_backward_workspace / gsm_policy_backward, for the Gaussian
+ * head: logp / values bit-identical to what gsm_policy_act_gauss / gsm_collect_gauss wrote; grad
+ * [GSM_POLICY_GAUSS_N_PARAMS]; the same determinism rule.  A non-finite action gives NaN logp, and a
+ * NaN gradient only where its d_logp != 0. */
+int gsm_policy_evaluate_gauss(const gsm_policy_gauss_eval_io* io, int device, void* stream);
+int64_t gsm_policy_backward_workspace_gauss(int64_t n_rows);
+int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d_logp, const float* d_entropy,
+                              const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
+                              int device, void* stream);
+
 /* n_steps of {actor forward + sampling, env step} enqueued on `stream` with no host sync (2
  * kernels per step; capturable into a CUDA graph).  io->obs / nbr_* / adj / assign point at slot 0
  * of [n_steps+1][...] tensors whose slot 0 already holds the current observation (gsm_reset,
@@ -361,6 +435,12 @@ int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const
 int gsm_collect(gsm_env* h, const gsm_policy_weights* w, int32_t n_steps, const gsm_step_io* io,
                 float* logp, float* values, uint64_t seed, uint64_t first_step, int32_t greedy,
                 void* stream);
+
+/* gsm_collect with the Gaussian actor: io->actions is float [n_steps][n_envs][N][2].  Needs a
+ * GSM_F32, GSM_ACT_CONTINUOUS handle; everything else as gsm_collect. */
+int gsm_collect_gauss(gsm_env* h, const gsm_policy_gauss_weights* w, int32_t n_steps, const gsm_step_io* io,
+                      float* logp, float* values, uint64_t seed, uint64_t first_step, int32_t greedy,
+                      void* stream);
 
 /* buffer.compute_returns + compute_cost_returns (utils/graph_separated_buffer.py, SOURCES.txt:33;
  * withheld: the on-policy lineage's GAE recursion, declared in SPEC.md §11) for both critics in one
