@@ -1,8 +1,11 @@
-"""The wide navigation kernel (env_wide_kernel: navigation with 3, 4 or 5 agents) and its in-kernel auto-reset,
-against a float64 numpy restatement of SPEC.md §2-4 and §6-8 written in this file.
+"""The navigation kernels with in-kernel auto-reset against the float64 numpy restatement of SPEC.md §2-8 in
+tests/_env_reference.py:
+  * the wide kernel (env_wide_kernel: navigation with 3, 4 or 5 agents), fp64 and fp32;
+  * the lane kernel (env_lane_kernel: one lane per agent, N >= 6), fp32, with and without CARRY (the contact force
+    of step s + 1 summed in the graph phase of step s; on for N >= 48), at the sizes bench.py runs it.
 
 The reference shares no code with the kernels or with the C oracle: Philox4x32-10, the spawn draw, the contact
-force, the integration, the graph, reward, cost, done and the auto-reset rule are all restated here, vectorised
+force, the integration, the graph, reward, cost, done and the auto-reset rule are all restated there, vectorised
 over envs.  The CPU tests pin it to the C oracle (oracle/gsm_oracle.py), so a fault in the reference cannot hide
 a fault in the kernel; the GPU tests compare the kernel with it over multi-step rollouts.
 
@@ -16,177 +19,15 @@ import numpy as np
 import pytest
 import torch
 
-from tests._util import make_cfg, near_threshold_rows, random_actions
+from tests._env_reference import (F32_TOL, RefNav, assert_step, check_fused_f32, env_sample, philox4x32_10,
+                                  ref_fused_rollout, spawn_draw, squeezed_start)
+from tests._util import make_cfg, random_actions
 
 # fp64 kernels round every SPEC operation once (-fmad=false); they differ from this reference only in libm's
 # last ulp and in the order in which pair forces are summed, which the stiff contacts amplify over 25 steps
 # to well below 1e-9 (SPEC §9).
 F64_TOL = dict(rtol=1e-9, atol=1e-9)
-# fp32 production bar (SPEC §9): 1e-4 relative; atol 2e-5 covers values that cross zero (positions, deltas)
-# with ~2 ulp of the unit-scale state
-F32_TOL = dict(rtol=1e-4, atol=2e-5)
 BENCH_ENVS = 16384                     # bench.py ENVS_PER_GPU: navigation-3, one launch of T = 25
-
-
-# ---- float64 reference ------------------------------------------------------------------------
-_M32 = np.uint64(0xFFFFFFFF)
-
-
-def philox4x32_10(c0, c1, c2, c3, k0, k1):
-    """Philox4x32-10 on uint64 arrays holding 32-bit words -> (r0, r1, r2, r3)."""
-    c0, c1, c2, c3, k0, k1 = (np.asarray(x, np.uint64) & _M32 for x in (c0, c1, c2, c3, k0, k1))
-    for _ in range(10):
-        p0 = np.uint64(0xD2511F53) * c0
-        p1 = np.uint64(0xCD9E8D57) * c2
-        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & _M32, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & _M32
-        k0 = (k0 + np.uint64(0x9E3779B9)) & _M32
-        k1 = (k1 + np.uint64(0xBB67AE85)) & _M32
-    return c0, c1, c2, c3
-
-
-def spawn_draw(cfg, genv, ep, seed):
-    """SPEC §8: positions [n, E, 2] (fp64) of every entity of global envs `genv` in episodes `ep`."""
-    E = cfg.n_entities
-    g = np.asarray(genv, np.uint64)[:, None]
-    e = np.arange(E, dtype=np.uint64)[None, :]
-    r0, r1, r2, r3 = philox4x32_10(g & _M32, g >> np.uint64(32), np.asarray(ep, np.int64)[:, None].astype(np.uint64),
-                                   e, np.uint64(seed) & _M32, np.uint64(seed) >> np.uint64(32))
-    u = lambda hi, lo: ((hi >> np.uint64(5)).astype(np.float64) * 67108864.0 + (lo >> np.uint64(6)).astype(np.float64)) / 2.0 ** 53
-    ext = np.asarray(cfg.spawn_extent, np.float64)[np.asarray(cfg.type)][None, :]
-    return np.stack([-ext + (2.0 * ext) * u(r0, r1), -ext + (2.0 * ext) * u(r2, r3)], -1)
-
-
-class RefNav:
-    """Batched navigation world in float64: state, one step, observation, the SPEC §8 re-draw.  `real` is the
-    precision of the state the kernel holds: a re-drawn position is rounded to it, as the kernel stores it."""
-
-    def __init__(self, cfg, agent_state, landmark_pos, t, episode, seed, env_offset=0):
-        assert cfg.scenario == "navigation"
-        self.cfg, self.seed, self.env_offset = cfg, int(seed), int(env_offset)
-        self.real = np.float32 if cfg.dtype == "f32" else np.float64
-        self.ag = np.array(agent_state, np.float64)            # [B, N, 4]: x, y, vx, vy
-        self.lm = np.array(landmark_pos, np.float64)            # [B, L, 2]
-        self.t = np.array(t, np.int64)
-        self.ep = np.array(episode, np.int64)
-        c = cfg
-        self.size = np.asarray(c.size, np.float64)
-        self.collide = np.asarray(c.collide, bool)
-        self.type = np.asarray(c.type, np.int64)
-        self.u = np.asarray(c.discrete_u, np.float64)
-
-    @property
-    def B(self):
-        return self.ag.shape[0]
-
-    def redraw(self, mask):
-        """SPEC §8 for the envs in `mask` [B]: spawn draw of (env, ep), v = 0, t = 0, then ep += 1."""
-        idx = np.flatnonzero(mask)
-        if idx.size == 0:
-            return
-        N = self.cfg.n_agents
-        p = spawn_draw(self.cfg, self.env_offset + idx, self.ep[idx], self.seed).astype(self.real).astype(np.float64)
-        self.ag[idx, :, :2] = p[:, :N]
-        self.ag[idx, :, 2:] = 0.0
-        self.lm[idx] = p[:, N:]
-        self.t[idx] = 0
-        self.ep[idx] += 1
-
-    def _geometry(self):
-        N = self.cfg.n_agents
-        pos = np.concatenate([self.ag[..., :2], self.lm], 1)                      # [B, E, 2]
-        d = pos[:, None, :, :] - pos[:, :N, None, :]                              # [B, N, E, 2]: p_e - p_i
-        dist = np.sqrt(d[..., 0] * d[..., 0] + d[..., 1] * d[..., 1])
-        return pos, d, dist
-
-    def step(self, actions):
-        """SPEC §2-4, then the outputs of the new state (§6-7)."""
-        c, N = self.cfg, self.cfg.n_agents
-        a = np.asarray(actions)
-        if c.action_mode == "discrete":
-            ok = (a >= 0) & (a < len(self.u))
-            ctrl = np.where(ok[..., None], self.u[np.clip(a, 0, len(self.u) - 1)], 0.0)
-        else:
-            ctrl = a.astype(np.float64)
-        F = np.asarray(c.accel, np.float64)[None, :, None] * ctrl                    # [B, N, 2]
-        _, d, dist = self._geometry()
-        pair = self.collide[:N, None] & self.collide[None, :]
-        pair[np.arange(N), np.arange(N)] = False
-        x = -(dist - (self.size[:N, None] + self.size[None, :])[None]) / c.contact_margin
-        pen = np.logaddexp(0.0, x) * c.contact_margin
-        with np.errstate(invalid="ignore", divide="ignore"):
-            f = np.where(pair[None, ..., None], c.contact_force * (-d) / dist[..., None] * pen[..., None], 0.0)
-        F = F + f.sum(2)
-        v = self.ag[..., 2:] * (1.0 - c.damping) + (F / np.asarray(c.mass, np.float64)[None, :, None]) * c.dt
-        ms = np.asarray(c.max_speed, np.float64)[None, :]
-        sp = np.sqrt(v[..., 0] * v[..., 0] + v[..., 1] * v[..., 1])
-        clamp = (ms > 0) & (sp > ms)
-        v = np.where(clamp[..., None], v / np.where(clamp, sp, 1.0)[..., None] * ms[..., None], v)
-        self.ag[..., 2:] = v
-        self.ag[..., :2] = self.ag[..., :2] + v * c.dt
-        self.t += 1
-        return self.observe()
-
-    def observe(self):
-        c, N, K, E = self.cfg, self.cfg.n_agents, self.cfg.max_nbrs, self.cfg.n_entities
-        B = self.B
-        pos, d, dist = self._geometry()
-        vel = np.concatenate([self.ag[..., 2:], np.zeros_like(self.lm)], 1)       # [B, E, 2]
-        ar = np.arange(N)
-        nb = dist < c.sensing_radius
-        if c.own_goal_always:
-            nb[:, ar, N + ar] = True
-        nb[:, ar, ar] = False
-        rank = np.cumsum(nb, 2) - 1
-        keep = nb & (rank < K)
-        bi, ii, ee = np.nonzero(keep)
-        kk = rank[bi, ii, ee]
-        out = {"nbr_idx": np.full((B, N, K), -1, np.int32), "nbr_feat": np.zeros((B, N, K, 6))}
-        out["nbr_idx"][bi, ii, kk] = ee
-        dv = vel[:, None, :, :] - vel[:, :N, None, :]
-        out["nbr_feat"][bi, ii, kk] = np.stack([d[..., 0], d[..., 1], dv[..., 0], dv[..., 1], dist,
-                                                np.broadcast_to(self.type[None, None, :].astype(np.float64), dist.shape)],
-                                               -1)[bi, ii, ee]
-        out["nbr_cnt"] = np.minimum(nb.sum(2), K).astype(np.int32)
-        out["adj"] = (nb.astype(np.uint64) << np.arange(E, dtype=np.uint64)).sum(2).astype(np.uint32)[..., None]   # E <= 32: one word
-        g = d[:, ar, N + ar]                                                        # goal i = landmark i
-        gd = dist[:, ar, N + ar]
-        out["obs"] = np.concatenate([self.ag[..., 2:], self.ag[..., :2], g], -1)
-        r = (0.0 - c.w_dist * gd) + np.where(gd < c.goal_tol, c.w_goal, 0.0)
-        if c.share_reward:
-            s = r[:, 0].copy()
-            for i in range(1, N):
-                s = s + r[:, i]
-            r = np.repeat((s / N)[:, None], N, 1)
-        out["reward"] = r
-        counted = (self.type == 0) | ((self.type == 2) & bool(c.cost_obstacles))
-        counted = np.broadcast_to(counted[None, :], (N, E)).copy()
-        counted[ar, ar] = False
-        hit = dist < (self.size[:N, None] + self.size[None, :])[None]
-        out["cost"] = (hit & counted[None]).sum(2).astype(np.float64)
-        out["done"] = np.repeat((self.t >= c.episode_length)[:, None], N, 1)
-        out["assign"] = np.broadcast_to(ar[None, :], (B, N)).astype(np.int32)
-        return out
-
-
-def ref_fused_rollout(ref, acts, auto_reset=True):
-    """The fused-rollout convention: outputs of every slot (terminal rows stay), then the re-draw of the envs that
-    finished.  Returns (per-slot outputs, per-slot bool [B] of the envs re-drawn after that slot)."""
-    outs, redrawn = [], []
-    for s in range(len(acts)):
-        outs.append(ref.step(acts[s]))
-        fin = ref.t >= ref.cfg.episode_length if auto_reset else np.zeros(ref.B, bool)
-        ref.redraw(fin)
-        redrawn.append(fin)
-    return outs, redrawn
-
-
-def squeezed_start(cfg, B, seed, t0, scale=0.45):
-    """A SPEC §8 draw pulled towards the origin (contacts from the first step on), at step counters t0."""
-    p = spawn_draw(cfg, np.arange(B), np.zeros(B, np.int64), seed) * scale
-    p = p.astype(np.float32 if cfg.dtype == "f32" else np.float64).astype(np.float64)
-    N = cfg.n_agents
-    ag = np.concatenate([p[:, :N], np.zeros_like(p[:, :N])], -1)
-    return ag, p[:, N:], np.asarray(t0, np.int64)
 
 
 # ---- CPU: the reference against the C oracle -------------------------------------------------
@@ -215,7 +56,13 @@ def test_philox_and_spawn_draw_equal_the_oracle():
 
 
 @pytest.mark.parametrize("N,kw", [(3, {}), (4, {"share_reward": True}), (5, {"max_nbrs": 6}),
-                                  (3, {"max_nbrs": 3, "own_goal_always": False, "cost_obstacles": False})])
+                                  (3, {"max_nbrs": 3, "own_goal_always": False, "cost_obstacles": False}),
+                                  # the lane kernel's teams: 6, 12, 24; 33 with 66 entities (3 adjacency words,
+                                  # K > 32); 48 with 144 entities (5 words) and K truncation at 32
+                                  (6, {}), (12, {}), (24, {}), (33, {"n_obstacles": 0, "max_nbrs": 65}),
+                                  (48, {"max_nbrs": 32}),
+                                  (12, {"share_reward": True, "own_goal_always": False, "cost_obstacles": False,
+                                        "action_mode": "continuous"})])
 def test_reference_rollout_equals_the_oracle(N, kw):
     """25 fp64 steps with staggered episode ends and re-draws: the reference against the C oracle."""
     from oracle import gsm_oracle as O
@@ -256,34 +103,42 @@ def _env(cfg, B, **kw):
     return MultiAgentGraphConstrainEnv(cfg, B, **kw)
 
 
-def _np(bufs):
+def _np(bufs, idx=None):
+    """Host copies of [T, B, ...] outputs, only the envs `idx` (gathered on the device) if given."""
     out = {}
     for k, v in bufs.items():
+        if idx is not None:
+            v = v.index_select(1, torch.as_tensor(idx, device=v.device))
         a = v.detach().cpu().numpy()
         out[k] = a.view(np.uint32) if k == "adj" else a
     return out
 
 
-INT_KEYS = ("nbr_idx", "nbr_cnt", "adj", "done", "assign", "cost")
-REAL_KEYS = ("obs", "nbr_feat", "reward")
+def _state(env, idx=None):
+    """(agent_state, landmark_pos, t, episode) as numpy, only the envs `idx` if given."""
+    xs = list(env.get_state()) + [env.get_episode()]
+    if idx is not None:
+        xs = [x.index_select(0, torch.as_tensor(idx, device=x.device)) for x in xs]
+    return [x.cpu().numpy() for x in xs]
 
 
-def _assert_step(got, want, ok, tol, ctx):
-    """Integer outputs (and the cost count) exact on the rows `ok` [B, N], reals within `tol` there."""
-    for k in INT_KEYS:
-        g, w = np.asarray(got[k])[ok], np.asarray(want[k])[ok].astype(np.asarray(got[k]).dtype)
-        bad = np.argwhere(g != w)
-        assert bad.size == 0, f"{ctx} {k}: {len(bad)} rows differ"
-    for k in REAL_KEYS:
-        np.testing.assert_allclose(got[k][ok], want[k][ok], **tol, err_msg=f"{ctx} {k}")
-
-
-def _staggered_env(cfg, B, seed, t0):
+def _staggered_env(cfg, B, seed, t0, idx=None):
+    """An env at a squeezed SPEC §8 draw with step counters t0, and the reference of its envs `idx` (all)."""
     env = _env(cfg, B, seed=seed)
     ag, lm, t = squeezed_start(cfg, B, seed + 1, t0)
     env.reset()
     env.set_state(ag, lm, t)
-    return env, RefNav(cfg, ag, lm, t, env.get_episode().cpu().numpy(), seed)
+    idx = np.arange(B) if idx is None else np.asarray(idx)
+    return env, RefNav(cfg, ag[idx], lm[idx], t[idx], env.get_episode().cpu().numpy()[idx], seed, genv=idx)
+
+
+def _lane_envs_per_cta(N):
+    return 1 if N > 32 else 32 // N * 4            # gsm_kernels_lane.cuh lane_geom
+
+
+def _setenv(monkeypatch, env_vars):
+    for k, v in env_vars.items():
+        monkeypatch.setenv(k, v)
 
 
 @gpu
@@ -302,7 +157,7 @@ def test_fused_auto_reset_rollout_f64_vs_reference(N, kw, B):
     want, redrawn = ref_fused_rollout(ref, acts)
     ok = np.ones((B, N), bool)
     for s in range(T):
-        _assert_step({k: got[k][s] for k in got}, want[s], ok, F64_TOL, f"N={N} B={B} t={s}")
+        assert_step({k: got[k][s] for k in got}, want[s], ok, F64_TOL, f"N={N} B={B} t={s}")
     ag, lm, t = (x.cpu().numpy() for x in env.get_state())
     np.testing.assert_allclose(ag, ref.ag, **F64_TOL)
     assert (lm == ref.lm).all() and (t == ref.t).all()
@@ -311,13 +166,27 @@ def test_fused_auto_reset_rollout_f64_vs_reference(N, kw, B):
     env.close()
 
 
+# lane-kernel instances: (N, kw, env vars) -> what the case reaches
+LANE_12 = (12, {}, {})                                                 # 2 envs per warp
+LANE_48 = (48, {"max_nbrs": 32}, {})                                   # CARRY, env spans 2 warps
+LANE_12_CARRY = (12, {}, {"GSM_LANE_CARRY_MIN_N": "6"})                # CARRY, envs of a warp end on different steps
+
+
 @gpu
-@pytest.mark.parametrize("N", [3, 4, 5])
-def test_only_finished_envs_are_redrawn_f64(N):
+@pytest.mark.parametrize("dtype,N,kw,env_vars", [
+    pytest.param("f64", 3, {}, {}, id="f64-3"), pytest.param("f64", 4, {}, {}, id="f64-4"),
+    pytest.param("f64", 5, {}, {}, id="f64-5"), pytest.param("f64", *LANE_12, id="f64-lane12"),
+    pytest.param("f32", 3, {}, {}, id="f32-3"), pytest.param("f32", 4, {}, {}, id="f32-4"),
+    pytest.param("f32", 5, {}, {}, id="f32-5"), pytest.param("f32", *LANE_12, id="f32-lane12"),
+    pytest.param("f32", 24, {"max_nbrs": 32}, {}, id="f32-lane24"), pytest.param("f32", *LANE_48, id="f32-lane48-carry"),
+    pytest.param("f32", *LANE_12_CARRY, id="f32-lane12-carry")])
+def test_only_finished_envs_are_redrawn(dtype, N, kw, env_vars, monkeypatch):
     """Half of the envs finish on step 2 of a 5-step launch, the other half never: the finished ones restart
-    from the SPEC §8 draw of their episode (bit for bit: the draw is integer + exact fp64 arithmetic), the others
-    are untouched — every output and the final state equal the same launch without auto-reset."""
-    cfg = make_cfg("navigation", N, "f64", episode_length=10)
+    from the SPEC §8 draw of their episode (bit for bit: the draw is integer + exact fp64 arithmetic, rounded to
+    the state's precision), the others are untouched — every output and the final state equal the same launch
+    without auto-reset.  fp64 runs free against the reference, fp32 slot by slot (check_fused_f32)."""
+    _setenv(monkeypatch, env_vars)
+    cfg = make_cfg("navigation", N, dtype, episode_length=10, **kw)
     B, T, seed = 203, 5, 21
     fin_env = np.arange(B) % 2 == 0
     t0 = np.where(fin_env, 8, 0)                                     # 8 + 2 = 10: done on step index 1
@@ -326,19 +195,24 @@ def test_only_finished_envs_are_redrawn_f64(N):
     ep0 = env.get_episode().clone()
     acts = random_actions(cfg, np.random.default_rng(N), (T, B))
     ar = _np(env.rollout(acts, auto_reset=True))
-    ar_state = [x.cpu().numpy() for x in env.get_state()] + [env.get_episode().cpu().numpy()]
+    ar_state = _state(env)
     env.set_state(ag0, lm0, tt0)
     env.set_episode(ep0)
     plain = _np(env.rollout(acts, auto_reset=False))
-    plain_state = [x.cpu().numpy() for x in env.get_state()] + [env.get_episode().cpu().numpy()]
+    plain_state = _state(env)
     env.close()
 
-    want, redrawn = ref_fused_rollout(ref, acts)
-    assert (redrawn[1] == fin_env).all() and not any(r.any() for i, r in enumerate(redrawn) if i != 1)
-    for s in range(T):
-        _assert_step({k: ar[k][s] for k in ar}, want[s], np.ones((B, N), bool), F64_TOL, f"N={N} t={s}")
+    if dtype == "f64":
+        want, redrawn = ref_fused_rollout(ref, acts)
+        for s in range(T):
+            assert_step({k: ar[k][s] for k in ar}, want[s], np.ones((B, N), bool), F64_TOL, f"N={N} t={s}")
+        redrawn = [r.sum() for r in redrawn]
+    else:
+        checked, rows, redrawn = check_fused_f32(ref, ar, acts, f"N={N}")
+        assert checked > 0.5 * rows, (checked, rows)
+    assert redrawn[1] == fin_env.sum() and sum(redrawn) == redrawn[1]
     # the re-draw itself: finished envs end the launch at t = 3 from positions drawn in episode ep0 + 0
-    draw = spawn_draw(cfg, np.arange(B), ep0.cpu().numpy(), seed)
+    draw = spawn_draw(cfg, np.arange(B), ep0.cpu().numpy(), seed).astype(cfg.np_real)
     assert (ar_state[1][fin_env] == draw[fin_env, N:]).all(), "landmarks of a finished env are not its re-draw"
     assert (ar_state[1][~fin_env] == lm0.cpu().numpy()[~fin_env]).all(), "an unfinished env's landmarks moved"
     assert (ar_state[2] == np.where(fin_env, T - 2, t0 + T)).all()
@@ -378,18 +252,25 @@ def test_step_api_auto_reset_returns_the_reset_observation(N):
         first = ref.observe()
         for k in ("obs", "nbr_idx", "nbr_feat", "nbr_cnt", "adj"):
             want[k] = np.where(fin.reshape((B,) + (1,) * (want[k].ndim - 1)), first[k], want[k])
-        _assert_step(got, want, np.ones((B, N), bool), F64_TOL, f"N={N} step {s}")
+        assert_step(got, want, np.ones((B, N), bool), F64_TOL, f"N={N} step {s}")
         assert (got["done"].all(1) == fin).all()
     env.close()
 
 
 @gpu
-@pytest.mark.parametrize("T", [25, 7])
-def test_auto_reset_instance_equals_plain_instance_when_nothing_finishes(T):
-    """The benchmark's instance (<float, 3, 6, auto-reset, K = 8>) against the plain one at the bench size: with
-    no episode ending inside the launch, the two must give the same bits in every output and the final state."""
-    cfg = make_cfg("navigation", 3, "f32", episode_length=1000)
-    B = BENCH_ENVS
+@pytest.mark.parametrize("N,B,kw,env_vars,T", [
+    pytest.param(3, BENCH_ENVS, {}, {}, 25, id="25"), pytest.param(3, BENCH_ENVS, {}, {}, 7, id="7"),
+    pytest.param(6, 1001, {}, {}, 25, id="lane6-1001"), pytest.param(12, 8192, {}, {}, 25, id="lane12-8192"),
+    pytest.param(24, 4096, {"max_nbrs": 32}, {}, 25, id="lane24-4096"),
+    pytest.param(48, 4096, {"max_nbrs": 32}, {}, 25, id="lane48-4096-carry"),
+    pytest.param(96, 4096, {"max_nbrs": 32}, {}, 25, id="lane96-4096-carry"),
+    pytest.param(*LANE_12_CARRY[:1], 1003, *LANE_12_CARRY[1:], 25, id="lane12-1003-carry")])
+def test_auto_reset_instance_equals_plain_instance_when_nothing_finishes(N, B, kw, env_vars, T, monkeypatch):
+    """The benchmark's instances (wide <float, 3, 6, auto-reset, K = 8>; lane <float, auto-reset, CARRY>) against
+    the plain ones at the bench sizes: with no episode ending inside the launch, the two must give the same bits
+    in every output and the final state."""
+    _setenv(monkeypatch, env_vars)
+    cfg = make_cfg("navigation", N, "f32", episode_length=1000, **kw)
     env = _env(cfg, B, seed=4)
     env.reset()
     rng = np.random.default_rng(T)
@@ -401,44 +282,70 @@ def test_auto_reset_instance_equals_plain_instance_when_nothing_finishes(T):
         env.set_state(*s0)
         out = env.rollout(acts, auto_reset=ar)
         res.append([v.clone() for k, v in sorted(out.items()) if k != "actions"] + [x.clone() for x in env.get_state()])
+        del out
     env.close()
     assert not bool(res[0][sorted(env.OUTPUTS).index("done")].any())
-    for a, b in zip(*res):
-        assert torch.equal(a, b)
+    for k, a, b in zip(sorted(env.OUTPUTS) + ["agent_state", "landmark_pos", "t"], *res):
+        assert torch.equal(a, b), k
+
+
+# fp32 cases: (N, B, kw, env vars, envs the reference follows (0: all)) -> what the case reaches
+F32_CASES = [
+    pytest.param(3, BENCH_ENVS, {}, {}, 0, id="3-16384"), pytest.param(3, 1, {}, {}, 0, id="3-1"),
+    pytest.param(4, 1001, {}, {}, 0, id="4-1001"), pytest.param(5, 999, {}, {}, 0, id="5-999"),
+    # lane kernel, plain: 5 envs per warp with 2 idle lanes and a ragged last CTA; 2 envs per warp at configs[4]'s
+    # share and ragged (the 16 + 8-byte row stores); one env per warp (configs[2]); an env over 2 warps with 31
+    # idle lanes, 3 adjacency words, K = 65 > 32
+    pytest.param(6, 1001, {}, {}, 0, id="lane6-1001"),
+    pytest.param(12, 8192, {}, {}, 512, id="lane12-8192"), pytest.param(12, 1003, {}, {}, 0, id="lane12-1003"),
+    pytest.param(24, 4096, {"max_nbrs": 32}, {}, 256, id="lane24-4096"),
+    pytest.param(33, 67, {"n_obstacles": 0, "max_nbrs": 65}, {}, 0, id="lane33-67"),
+    # CARRY + auto-reset (configs[2]): multi-warp envs, 5 / 9 adjacency words, K truncation at 32
+    pytest.param(48, 4096, {"max_nbrs": 32}, {}, 256, id="lane48-4096-carry"),
+    pytest.param(96, 4096, {"max_nbrs": 32}, {}, 256, id="lane96-4096-carry"),
+    # CARRY with several envs per warp that finish on different steps
+    pytest.param(*LANE_12_CARRY[:1], 1003, *LANE_12_CARRY[1:], 0, id="lane12-1003-carry"),
+    pytest.param(24, 1024, {"max_nbrs": 32}, {"GSM_LANE_CARRY_MIN_N": "6"}, 256, id="lane24-1024-carry"),
+    # CARRY instance with carry_ok false (contact reach beyond the sensing radius: sweep every step)
+    pytest.param(48, 512, {"max_nbrs": 32, "sensing_radius": 0.33}, {}, 128, id="lane48-carry-sweep"),
+    # col_in_nb false: the candidate test also takes the contact distance
+    pytest.param(24, 1024, {"max_nbrs": 32, "sensing_radius": 0.3}, {}, 256, id="lane24-contact-candidates"),
+    # a re-draw after every step: the carried force is never valid
+    pytest.param(48, 512, {"max_nbrs": 32, "episode_length": 1}, {}, 128, id="lane48-carry-ep1"),
+    # the switches
+    pytest.param(12, 1003, {"share_reward": True, "action_mode": "continuous", "cost_obstacles": False,
+                            "own_goal_always": False}, {}, 0, id="lane12-switches"),
+]
 
 
 @gpu
-@pytest.mark.parametrize("N,B", [(3, BENCH_ENVS), (3, 1), (4, 1001), (5, 999)])
-def test_fused_auto_reset_rollout_f32_vs_reference(N, B):
+@pytest.mark.parametrize("N,B,kw,env_vars,n_ref", F32_CASES)
+def test_fused_auto_reset_rollout_f32_vs_reference(N, B, kw, env_vars, n_ref, monkeypatch):
     """fp32 production instances over one 25-step fused launch with staggered episode ends (the benchmark's
-    shape for N = 3).  fp32 and fp64 trajectories part at the stiff contacts, so each slot is checked against ONE
-    reference step from the kernel's own state of the slot before: the agent state is exactly obs[..., :4] of
-    that slot, the landmarks only change in a re-draw, which the reference makes itself (fp64 draw rounded to
-    fp32, as the kernel stores it).  Integer outputs must match except on rows with a predicate within 1e-4 of
-    its threshold (SPEC §9) or a goal distance within 1e-4 of goal_tol (the reward's step); after a re-draw the positions are the draw's exact fp32 values."""
-    cfg = make_cfg("navigation", N, "f32", episode_length=25)
+    shapes: navigation-3 x 16384 on the wide kernel, navigation-12 / 24 / 48 / 96 on the lane kernel), slot by
+    slot against the reference (check_fused_f32: one reference step from the kernel's own state of the slot
+    before).  At the large sizes the kernel runs the whole batch and the reference follows a seeded sample of
+    n_ref envs that includes the last CTA's envs and envs that finish in every slot.  Then the final state, step
+    and episode counters of those envs."""
+    _setenv(monkeypatch, env_vars)
+    kw = dict(kw)
+    cfg = make_cfg("navigation", N, "f32", episode_length=kw.pop("episode_length", 25), **kw)
     T, seed = 25, 31
-    t0 = np.arange(B) % 25
-    env, ref = _staggered_env(cfg, B, seed, t0)
+    t0 = np.arange(B) % cfg.episode_length
+    idx = env_sample(B, n_ref, t0, _lane_envs_per_cta(N) if N >= 6 else 16, seed=N)
+    env, ref = _staggered_env(cfg, B, seed, t0, idx)
     acts = random_actions(cfg, np.random.default_rng(N), (T, B))
-    got = _np(env.rollout(acts, auto_reset=True))
-    final = [x.cpu().numpy() for x in env.get_state()] + [env.get_episode().cpu().numpy()]
+    got = _np(env.rollout(acts, auto_reset=True), idx)
+    final = _state(env, idx)
     env.close()
-    checked = ends = 0
-    for s in range(T):
-        want = ref.step(acts[s])
-        gd = np.hypot(want["obs"][..., 4], want["obs"][..., 5])
-        ok = ~near_threshold_rows(cfg, ref.ag, ref.lm, 1e-4) & (np.abs(gd - cfg.goal_tol) > 1e-4)
-        _assert_step({k: got[k][s] for k in got}, want, ok, F32_TOL, f"N={N} B={B} t={s}")
-        checked += int(ok.sum())
-        fin = ref.t >= cfg.episode_length
-        ends += int(fin.sum())
-        ref.redraw(fin)
-        # continue from the kernel's own state (exact fp32 values) where the env did not restart
-        keep = ~fin
-        ref.ag[keep, :, 2:] = got["obs"][s][keep][..., 0:2]
-        ref.ag[keep, :, :2] = got["obs"][s][keep][..., 2:4]
-    assert checked > 0.5 * T * B * N and ends >= B * (T - 1) // 25
+    checked, rows, ends = check_fused_f32(ref, got, acts[:, idx], f"N={N} B={B}")
+    print(f"[f32 auto-reset] N={N} B={B} {kw} {env_vars}: reference follows {idx.size} envs "
+          f"({idx.size / B:.3f} of the batch), rows checked {checked / rows:.4f}, re-draws {int(ends.sum())}")
+    assert checked > 0.5 * rows, (checked, rows)
+    if idx.size >= cfg.episode_length:
+        assert (ends > 0).all(), f"slots without a re-drawn env: {np.flatnonzero(ends == 0)}"
+    else:
+        assert ends.sum() >= idx.size * (T - 1) // cfg.episode_length
     # final state: restarted-and-stepped envs within fp32 rounding, the counters exactly
     np.testing.assert_allclose(final[0], ref.ag, **F32_TOL)
     assert (final[1] == ref.lm).all() and (final[2] == ref.t).all() and (final[3] == ref.ep).all()
