@@ -130,6 +130,23 @@ class GsmPolicyGaussEvalIO(C.Structure):
     ]
 
 
+GSM_EPISODE_STAT_FIELDS = 16
+
+
+class GsmEpisodeIO(C.Structure):
+    """gsm_episode_io: DEVICE pointers over the buffer's reward / cost / done slots (SPEC.md §13)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("dtype", C.c_int32),
+        ("reward", C.c_void_p), ("cost", C.c_void_p), ("done", C.c_void_p),
+        ("carry_return", C.c_void_p), ("carry_cost", C.c_void_p), ("carry_length", C.c_void_p),
+        ("totals", C.c_void_p), ("episodes", C.c_void_p),
+        ("last_return", C.c_void_p), ("last_cost", C.c_void_p), ("last_length", C.c_void_p),
+        ("team_last_return", C.c_void_p), ("team_last_cost", C.c_void_p),
+        ("n_rows", C.c_int64), ("slot_rows", C.c_int64), ("n_steps", C.c_int32), ("agents_per_env", C.c_int32),
+        ("agent_cost_limit", C.c_double), ("team_cost_limit", C.c_double),
+    ]
+
+
 def policy_n_params(n_actions: int) -> int:
     """GSM_POLICY_N_PARAMS: length of the learner's parameter vector."""
     return 961 + 129 * n_actions + 2 * (2 * GSM_POLICY_HIDDEN + 1)
@@ -184,6 +201,8 @@ SYMBOLS = {
                                             C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gsm_collect_gauss": (C.c_int, [_H, C.POINTER(GsmPolicyGaussWeights), C.c_int32, _IO, C.c_void_p, C.c_void_p,
                                     C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
+    "gsm_episode_stats_workspace": (C.c_int64, [C.c_int64, C.c_int32]),
+    "gsm_episode_stats": (C.c_int, [C.POINTER(GsmEpisodeIO), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
 }
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "libgsmarl_b200.so")

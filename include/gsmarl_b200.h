@@ -454,6 +454,55 @@ int gsm_gae(const float* reward, const float* cost, const float* values, const u
             int32_t n_steps, int64_t n_rows, int64_t slot_rows, float gamma, float lam,
             float* returns, float* advantages, int device, void* stream);
 
+/* ---- episode statistics (SPEC.md §13): the runner's per-episode logging over the buffer slots --------
+ * Episode return, cost and length per agent row and per team, across calls: rollouts shorter or longer
+ * than an episode and staggered episode ends are handled by a per-row fp64 carry.  Slot t with done = 1
+ * is the last step of an episode (the gsm_gae rule).  Per row, for t = 0 .. T-1:
+ *   R += (double)reward[t];  C += (double)cost[t];  n += 1;  if done[t]: agent episode (R, C, n), carry = 0.
+ * An env's team episode ends where its agent 0's done is set: team return = (sum_j R_j) / N, team cost =
+ * sum_j C_j (j ascending, fp64), team length = n of agent 0.  Safe: cost == 0; over the limit: cost >
+ * agent_cost_limit (agent episodes) or > team_cost_limit (team episodes).
+ * totals [GSM_EPISODE_STAT_FIELDS] (overwritten every call; additive across calls and ranks):
+ *   agent episodes  0 count, 1 sum return, 2 sum return^2, 3 sum cost, 4 sum cost^2, 5 sum length,
+ *                   6 safe count, 7 over-limit count;  team episodes  8 .. 15, the same fields.
+ * Deterministic: per-block partials in `workspace` (a partition of the rows that depends on n_rows and
+ * agents_per_env only), combined in a fixed order; no atomics.  Two launches, no host sync. */
+#define GSM_EPISODE_STAT_FIELDS 16
+
+typedef struct gsm_episode_io {   /* DEVICE pointers; row = one agent of one env, rows [g*N, (g+1)*N) = env g */
+  uint32_t struct_size;          /* = sizeof(gsm_episode_io); checked                                 */
+  int32_t dtype;                 /* gsm_dtype of reward / cost                                        */
+  const void* reward;            /* real [n_steps][slot_rows]                                         */
+  const void* cost;              /* real [n_steps][slot_rows]                                         */
+  const uint8_t* done;           /* u8   [n_steps][slot_rows]                                         */
+  double* carry_return;          /* [n_rows] in/out: the partial episode of each row                  */
+  double* carry_cost;            /* [n_rows] in/out                                                   */
+  int32_t* carry_length;         /* [n_rows] in/out                                                   */
+  double* totals;                /* [GSM_EPISODE_STAT_FIELDS] out                                     */
+  int32_t* episodes;             /* [n_rows / N] out: team episodes each env completed in this call   */
+  double* last_return;           /* [n_rows] the last agent episode completed in this call; rows that */
+  double* last_cost;             /* [n_rows]   completed none are left untouched; NULL = skip         */
+  int32_t* last_length;          /* [n_rows]                                                          */
+  double* team_last_return;      /* [n_rows / N] the same rule per env; NULL = skip                   */
+  double* team_last_cost;        /* [n_rows / N]                                                      */
+  int64_t n_rows;                /* a multiple of agents_per_env; 0 = no-op                           */
+  int64_t slot_rows;             /* slot stride in rows, >= n_rows                                    */
+  int32_t n_steps;               /* T >= 1                                                            */
+  int32_t agents_per_env;        /* N, 1 .. 1024                                                      */
+  double agent_cost_limit;
+  double team_cost_limit;
+} gsm_episode_io;
+
+/* Workspace bytes gsm_episode_stats needs (a function of n_rows and agents_per_env only);
+ * GSM_ERR_INVALID_ARG for n_rows < 0, agents_per_env outside [1, 1024] or n_rows % agents_per_env != 0. */
+int64_t gsm_episode_stats_workspace(int64_t n_rows, int32_t agents_per_env);
+
+/* GSM_ERR_ABI for a bad struct_size; GSM_ERR_INVALID_ARG for a missing reward / cost / done / carry /
+ * totals / episodes pointer, n_steps < 1, a bad agents_per_env or n_rows (as above), slot_rows < n_rows,
+ * an unknown dtype or a workspace smaller than gsm_episode_stats_workspace. */
+int gsm_episode_stats(const gsm_episode_io* io, void* workspace, size_t workspace_bytes, int device,
+                      void* stream);
+
 #ifdef __cplusplus
 }
 #endif
