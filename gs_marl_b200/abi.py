@@ -147,6 +147,19 @@ class GsmEpisodeIO(C.Structure):
     ]
 
 
+GSM_PPO_STAT_FIELDS = 8
+
+
+class GsmPpoLossIO(C.Structure):
+    """gsm_ppo_loss_io: DEVICE pointers over the buffer's loss inputs and the loss coefficients (SPEC.md §14)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("reserved", C.c_int32),
+        ("old_logp", C.c_void_p), ("old_values", C.c_void_p), ("returns", C.c_void_p), ("advantages", C.c_void_p),
+        ("adv_moments", C.c_void_p), ("lagrange", C.c_void_p), ("stats", C.c_void_p),
+        ("clip", C.c_float), ("value_clip", C.c_float), ("value_coef", C.c_float), ("entropy_coef", C.c_float),
+    ]
+
+
 def policy_n_params(n_actions: int) -> int:
     """GSM_POLICY_N_PARAMS: length of the learner's parameter vector."""
     return 961 + 129 * n_actions + 2 * (2 * GSM_POLICY_HIDDEN + 1)
@@ -201,6 +214,14 @@ SYMBOLS = {
                                             C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gsm_collect_gauss": (C.c_int, [_H, C.POINTER(GsmPolicyGaussWeights), C.c_int32, _IO, C.c_void_p, C.c_void_p,
                                     C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
+    "gsm_ppo_backward_workspace": (C.c_int64, [C.c_int64, C.c_int32]),
+    "gsm_ppo_backward_workspace_gauss": (C.c_int64, [C.c_int64]),
+    "gsm_ppo_backward": (C.c_int, [C.POINTER(GsmPolicyEvalIO), C.POINTER(GsmPpoLossIO), C.c_void_p, C.c_void_p,
+                                   C.c_size_t, C.c_int, C.c_void_p]),
+    "gsm_ppo_backward_gauss": (C.c_int, [C.POINTER(GsmPolicyGaussEvalIO), C.POINTER(GsmPpoLossIO), C.c_void_p,
+                                         C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gsm_adam_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
+                                C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_int, C.c_void_p]),
     "gsm_episode_stats_workspace": (C.c_int64, [C.c_int64, C.c_int32]),
     "gsm_episode_stats": (C.c_int, [C.POINTER(GsmEpisodeIO), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
 }

@@ -589,174 +589,65 @@ template <int NA> struct BwdSmemGauss : BwdSmem<NA, HEAD_GAUSS> {
 template <int NA, int KIND>
 using BwdSmemOf = std::conditional_t<KIND == HEAD_GAUSS, BwdSmemGauss<NA>, BwdSmem<NA, KIND>>;
 
-template <int NA, int KIND>
-__global__ void __launch_bounds__(BWD_AG) policy_backward_kernel(const __grid_constant__ EvalArgs<KIND> p) {
-  using P = PV<NA, KIND>;
-  constexpr int NZ = NA + V2, NP = P::N;
-  __shared__ BwdSmemOf<NA, KIND> sm;
-  extern __shared__ float s_rows[];    // [BWD_AG][K][2]: (a_r, ds_r) of the valid rows; a float2 array
-                                       // would round every kernel's static shared memory in this file up to 16 B
-  const int tid = threadIdx.x;
-  for (int k = tid; k < NP; k += BWD_AG) sm.w[k] = p.params[k];
-  const float* W = sm.w;
-  // phase-B accumulators of hidden unit j = tid, live across the tiles
-  float gwe[GSM_OBS_DIM], gwn[GSM_NBR_FEAT_DIM], ghe[NZ], ghg[NZ];
-  float gbe = 0.f, gbn = 0.f, gwa = 0.f, gsc = 0.f;   // gsc: bias sum of dZ[tid] (tid < NZ) or db_a (tid = H-1)
-#pragma unroll
-  for (int k = 0; k < GSM_OBS_DIM; k++) { gwe[k] = 0.f; gwn[k] = 0.f; }
-#pragma unroll
-  for (int a = 0; a < NZ; a++) { ghe[a] = 0.f; ghg[a] = 0.f; }
-  __syncthreads();
+// ---- fused PPO loss (SPEC.md §14): the loss seeds computed in phase A from the row's own logp, entropy
+// and values, per-row statistics parked in shared memory and summed per block in row order ----------
+constexpr int PPO_ROW_STATS = 7;      // L_pi, L_V reward, L_V cost, entropy, rho, clipped, approx KL
+constexpr int PPO_WS_STATS = 8;       // workspace floats per block behind its gradient partial
 
-  for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {   // block-uniform
-    const int64_t base = tile * BWD_AG;
-    const int nag = p.n_rows - base < BWD_AG ? (int)(p.n_rows - base) : BWD_AG;
-    // ---- phase A: thread = row ----
-    if (tid < nag) {
-      const int64_t i = base + tid;
-      const int64_t src = p.rows ? p.rows[i] : i;
-      const int cnt = clamp_cnt(p.nbr_cnt[src], p.K);
-      const float* o = p.obs + src * GSM_OBS_DIM;
-      const float* f = p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM;
-      float z[NZ], acc[NZ], mx, s;
-      row_forward<NA, KIND>(W, o, f, cnt, z, acc, mx, s);
-      // The categorical dz stays at this scope for BOTH kinds, on purpose: guarded by
-      // `if constexpr (KIND == HEAD_CAT)` (or nested in an if-constexpr / else) it changes the register
-      // allocation and SASS of the categorical instances, which must stay as they were.  For the
-      // Gaussian it is dead code: act is the constant 0, every dz[a < NA] it writes is rewritten by the
-      // Gaussian block below and nothing else reads its values, so the compiler removes it (same
-      // registers as the nested form).  Only dlp and dent are shared with the Gaussian block.
-      float zm, se;
-      const int act = KIND == HEAD_CAT ? (int)p.actions[src] : 0;
-      const float lp = row_logp<NA>(z, act, zm, se);
-      const float dlp = p.d_logp ? p.d_logp[i] : 0.f, dent = p.d_entropy ? p.d_entropy[i] : 0.f;
-      const float lse = zm + logf(se), inv_se = 1.f / se;
-      float pr[NA], ent = 0.f;
+template <int KIND> struct PpoArgs : EvalArgs<KIND> {
+  const float* old_logp; const float* old_values; const float* returns; const float* adv;   // source rows
+  const float* adv_moments; const float* lagrange;                                          // device scalars
+  float clip, value_clip, value_coef, entropy_coef, inv_n;
+};
+template <class Base> struct PpoSmem : Base {
+  float st[BWD_AG][PPO_ROW_STATS];     // the tile's per-row statistics
+  float stacc[PPO_ROW_STATS];          // the block's sums over its tiles (thread k owns entry k)
+};
+
+// SPEC.md §14 for one row: the seeds d_logp, d_entropy, d_values of the §12 chain and the row's statistics.
+// A comparison with a NaN operand is false, so a NaN log-prob (an action outside the head's range)
+// reaches d_logp and poisons the gradient, as in gsm_policy_backward.
+template <int KIND>
+__device__ __forceinline__ void ppo_seeds(const PpoArgs<KIND>& p, int64_t src, float lp, float ent, const float* v,
+                                          float& dlp, float& dent, float (&dv)[V2], float* st) {
+  const float* mom = p.adv_moments;
+  const float a0 = (p.adv[src * V2] - mom[0]) / (mom[1] + 1e-5f);
+  const float a1 = (p.adv[src * V2 + 1] - mom[2]) / (mom[3] + 1e-5f);
+  const float A = a0 - p.lagrange[0] * a1;
+  const float olp = p.old_logp[src];
+  const float rho = expf(lp - olp);
+  const float s1 = rho * A, s2 = fminf(fmaxf(rho, 1.f - p.clip), 1.f + p.clip) * A;
+  dlp = s2 < s1 ? 0.f : -s1 * p.inv_n;
+  st[0] = -(s2 < s1 ? s2 : s1);
 #pragma unroll
-      for (int a = 0; a < NA; a++) { pr[a] = expf(z[a] - zm) * inv_se; ent = fmaf(pr[a], z[a] - zm, ent); }
-      ent = logf(se) - ent;
-      // an action outside [0, NA) has no one-hot: its NaN logp poisons the gradient it feeds
-      const float bad = (dlp != 0.f && lp != lp) ? __int_as_float(0x7fc00000) : 0.f;
-      float dz[NZ];
-#pragma unroll
-      for (int a = 0; a < NA; a++)
-        dz[a] = dlp * ((act == a ? 1.f : 0.f) - pr[a] + bad) - dent * pr[a] * ((z[a] - lse) + ent);
-      if constexpr (KIND == HEAD_GAUSS) {
-        // SPEC.md §12b: dmu_d = d_logp delta_d exp(-log_std_d);
-        // dlog_std_d = d_logp (delta_d^2 - 1) + d_entropy.  A non-finite action (NaN logp) gives a NaN
-        // gradient exactly where d_logp != 0; where d_logp == 0 the action does not enter it.
-        const float ls0 = W[P::LS], ls1 = W[P::LS + 1];
-        float d0, d1;
-        const float glp = gauss_logp(p.actions[src * GD], p.actions[src * GD + 1], z[0], z[1], ls0, ls1, d0, d1);
-        const bool use = dlp != 0.f;
-        const float gbad = (use && glp != glp) ? __int_as_float(0x7fc00000) : 0.f;
-        dz[0] = use ? dlp * d0 * expf(-ls0) + gbad : 0.f;
-        dz[1] = use ? dlp * d1 * expf(-ls1) + gbad : 0.f;
-        sm.dls[tid][0] = (use ? dlp * fmaf(d0, d0, -1.f) + gbad : 0.f) + dent;
-        sm.dls[tid][1] = (use ? dlp * fmaf(d1, d1, -1.f) + gbad : 0.f) + dent;
-      }
-#pragma unroll
-      for (int v = 0; v < V2; v++) dz[NA + v] = p.d_values ? p.d_values[i * V2 + v] : 0.f;
-      float dsum = 0.f;
-      if (cnt > 0) {
-        const float inv = 1.f / s;
-        float gdg = 0.f;                 // g . dg = dZ . sum_r a_r hr_r
-#pragma unroll
-        for (int a = 0; a < NZ; a++) gdg = fmaf(dz[a], acc[a] * inv, gdg);
-        float* pr_rows = s_rows + 2 * tid * p.K;
-        for (int r = 0; r < cnt; r++) {  // second pass: the same t_r, hr_r as the first
-          float hr[NZ];
-          const float t = nbr_row<NA, KIND>(W, f + r * GSM_NBR_FEAT_DIM, hr);
-          const float ar = expf(t - mx) * inv;
-          float q = 0.f;
-#pragma unroll
-          for (int a = 0; a < NZ; a++) q = fmaf(dz[a], hr[a], q);
-          const float ds = ar * (q - gdg);
-          pr_rows[2 * r] = ar; pr_rows[2 * r + 1] = ds;
-          dsum += ds;
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < GSM_OBS_DIM; k++) sm.obs[tid][k] = o[k];
-#pragma unroll
-      for (int a = 0; a < NZ; a++) sm.dz[tid][a] = dz[a];
-      sm.dsum[tid] = dsum;
-      sm.cnt[tid] = cnt;
-      sm.src[tid] = src;
-    }
-    __syncthreads();
-    // ---- phase B: thread = hidden unit j ----
-    {
-      const int j = tid;
-      float we[GSM_OBS_DIM], wn[GSM_NBR_FEAT_DIM], wh[NZ], wg[NZ];
-#pragma unroll
-      for (int k = 0; k < GSM_OBS_DIM; k++) { we[k] = W[P::EW + j * GSM_OBS_DIM + k]; wn[k] = W[P::NW + j * GSM_NBR_FEAT_DIM + k]; }
-#pragma unroll
-      for (int a = 0; a < NZ; a++) { wh[a] = W[P::row(a) + j]; wg[a] = W[P::row(a) + H + j]; }
-      const float be = W[P::EB + j], bn = W[P::NB + j], wa = W[P::AW + j];
-      for (int ag = 0; ag < nag; ag++) {
-        float dZ[NZ];
-#pragma unroll
-        for (int a = 0; a < NZ; a++) dZ[a] = sm.dz[ag][a];
-        float u = be;
-#pragma unroll
-        for (int k = 0; k < GSM_OBS_DIM; k++) u = fmaf(we[k], sm.obs[ag][k], u);
-        const float e = fmaxf(u, 0.f);
-        float dh = 0.f;
-#pragma unroll
-        for (int a = 0; a < NZ; a++) { dh = fmaf(wh[a], dZ[a], dh); ghe[a] = fmaf(dZ[a], e, ghe[a]); }
-        const float de = u > 0.f ? dh : 0.f;            // ReLU'(0) = 0, as in torch
-#pragma unroll
-        for (int k = 0; k < GSM_OBS_DIM; k++) gwe[k] = fmaf(de, sm.obs[ag][k], gwe[k]);
-        gbe += de;
-        const int c = sm.cnt[ag];                        // block-uniform: no divergence
-        if (c > 0) {
-          float dg = 0.f, g = 0.f;
-#pragma unroll
-          for (int a = 0; a < NZ; a++) dg = fmaf(wg[a], dZ[a], dg);
-          const float* f = p.nbr_feat + sm.src[ag] * p.K * GSM_NBR_FEAT_DIM;
-          const float* rr = s_rows + 2 * ag * p.K;
-          for (int r = 0; r < c; r++) {
-            float fr[GSM_NBR_FEAT_DIM];
-#pragma unroll
-            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) fr[k] = __ldg(f + r * GSM_NBR_FEAT_DIM + k);
-            float um = bn;
-#pragma unroll
-            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) um = fmaf(wn[k], fr[k], um);
-            const float m = fmaxf(um, 0.f);
-            const float ar = rr[2 * r], ds = rr[2 * r + 1];
-            g = fmaf(ar, m, g);
-            const float du = um > 0.f ? fmaf(ar, dg, ds * wa) : 0.f;
-#pragma unroll
-            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) gwn[k] = fmaf(du, fr[k], gwn[k]);
-            gbn += du;
-            gwa = fmaf(ds, m, gwa);
-          }
-#pragma unroll
-          for (int a = 0; a < NZ; a++) ghg[a] = fmaf(dZ[a], g, ghg[a]);
-        }
-        if (j < NZ) gsc += sm.dz[ag][j];
-        else if (j == H - 1) gsc += sm.dsum[ag];
-        else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) gsc += sm.dls[ag][j - NZ]; }
-      }
-    }
-    __syncthreads();                     // before the next tile overwrites the row state
+  for (int h = 0; h < V2; h++) {
+    const float ov = p.old_values[src * V2 + h], R = p.returns[src * V2 + h];
+    const float dov = v[h] - ov;
+    const float vc = ov + fminf(fmaxf(dov, -p.value_clip), p.value_clip);
+    const float e1 = v[h] - R, e2 = vc - R, q1 = e1 * e1, q2 = e2 * e2;
+    // the clipped branch carries the gradient where the clip is not active (vc = v up to rounding)
+    const bool inside = fabsf(dov) <= p.value_clip;
+    dv[h] = q1 < q2 ? (inside ? p.value_coef * e2 * p.inv_n : 0.f) : p.value_coef * e1 * p.inv_n;
+    st[1 + h] = 0.5f * (q1 < q2 ? q2 : q1);
   }
-  // ---- this block's partial gradient, in vector order ----
-  float* out = p.ws + (int64_t)blockIdx.x * NP;
-  const int j = tid;
-#pragma unroll
-  for (int k = 0; k < GSM_OBS_DIM; k++) {
-    out[P::EW + j * GSM_OBS_DIM + k] = gwe[k];
-    out[P::NW + j * GSM_NBR_FEAT_DIM + k] = gwn[k];
-  }
-  out[P::EB + j] = gbe; out[P::NB + j] = gbn; out[P::AW + j] = gwa;
-#pragma unroll
-  for (int a = 0; a < NZ; a++) { out[P::row(a) + j] = ghe[a]; out[P::row(a) + H + j] = ghg[a]; }
-  if (j < NZ) out[j < NA ? P::HB + j : P::VB + (j - NA)] = gsc;
-  else if (j == H - 1) out[P::AB] = gsc;
-  else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) out[P::LS + (j - NZ)] = gsc; }
+  dent = -p.entropy_coef * p.inv_n;
+  st[3] = ent; st[4] = rho; st[5] = fabsf(rho - 1.f) > p.clip ? 1.f : 0.f; st[6] = olp - lp;
 }
+
+#define GSM_BWD_KERNEL policy_backward_kernel
+#define GSM_BWD_ARGS EvalArgs
+#define GSM_BWD_LOSS false
+#include "gsm_policy_backward.inl"
+#undef GSM_BWD_KERNEL
+#undef GSM_BWD_ARGS
+#undef GSM_BWD_LOSS
+#define GSM_BWD_KERNEL ppo_backward_kernel
+#define GSM_BWD_ARGS PpoArgs
+#define GSM_BWD_LOSS true
+#include "gsm_policy_backward.inl"
+#undef GSM_BWD_KERNEL
+#undef GSM_BWD_ARGS
+#undef GSM_BWD_LOSS
 
 // grad[k] = sum of the G partials in a fixed order: warp w sums partials w, w + 8, ... (lane = k),
 // then warp 0 adds the 8 warp sums in order.
@@ -778,6 +669,91 @@ __global__ void __launch_bounds__(256) policy_grad_reduce_kernel(const float* __
     for (int q = 1; q < 8; q++) t += s[q][lane];
     grad[k] = t;
   }
+}
+
+// ppo_backward_kernel's partials: blocks 0 .. ceil(NP / 32) - 1 reduce the gradient exactly as
+// policy_grad_reduce_kernel does (partials of stride NP + PPO_WS_STATS); the last block reduces the
+// statistics in the same order, then lanes 0..6 write their means over the n rows and lane 0 adds
+// L = L_pi + c_v (L_V reward + L_V cost) - c_e entropy.  Counts (the clip fraction) are exact in fp32
+// below 2^24 rows.
+__global__ void __launch_bounds__(256) ppo_reduce_kernel(const float* __restrict__ ws, int G, int NP,
+                                                         float* __restrict__ grad, float* __restrict__ stats,
+                                                         float n, float value_coef, float entropy_coef) {
+  __shared__ float s[8][32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int ngrad = (NP + 31) / 32;
+  const bool is_stats = (int)blockIdx.x == ngrad;
+  const int k = is_stats ? NP + lane : blockIdx.x * 32 + lane;
+  const bool live = is_stats ? lane < PPO_ROW_STATS : k < NP;
+  const int64_t stride = NP + PPO_WS_STATS;
+  float acc = 0.f;
+  if (live) {
+#pragma unroll 4
+    for (int g = w; g < G; g += 8) acc += ws[(int64_t)g * stride + k];
+  }
+  s[w][lane] = acc;
+  __syncthreads();
+  if (w != 0) return;
+  float t = s[0][lane];
+#pragma unroll
+  for (int q = 1; q < 8; q++) t += s[q][lane];
+  if (!is_stats) {
+    if (live) grad[k] = t;
+    return;
+  }
+  const float mean = t / n;
+  const float lpi = __shfl_sync(~0u, mean, 0), lv0 = __shfl_sync(~0u, mean, 1), lv1 = __shfl_sync(~0u, mean, 2),
+              ent = __shfl_sync(~0u, mean, 3);
+  if (live) stats[lane] = mean;
+  if (lane == 0) stats[PPO_ROW_STATS] = lpi + value_coef * (lv0 + lv1) - entropy_coef * ent;
+}
+
+// ---- Adam step (SPEC.md §14): torch.nn.utils.clip_grad_norm_ then torch.optim.Adam (no weight decay,
+// no amsgrad) over the whole parameter vector in ONE block: the norm as a fixed-order fp64 sum (thread
+// partials in index order, a shuffle tree, the warp sums in order), the clip, the update.  A non-finite
+// norm skips the step (p, m, v and the step counter unchanged); the norm is written either way.
+struct AdamArgs {
+  float* params; const float* grad; float* m; float* v; int32_t* step; float* grad_norm;
+  int64_t n;
+  float lr, beta1, beta2, eps, max_norm;
+};
+constexpr int ADAM_THREADS = 1024;
+
+__global__ void __launch_bounds__(ADAM_THREADS) adam_step_kernel(const __grid_constant__ AdamArgs a) {
+  __shared__ double s_part[ADAM_THREADS / 32];
+  __shared__ float s_norm;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  double ss = 0.0;
+  for (int64_t k = tid; k < a.n; k += ADAM_THREADS) { const double g = a.grad[k]; ss = fma(g, g, ss); }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) ss += __shfl_xor_sync(~0u, ss, d);
+  if (lane == 0) s_part[warp] = ss;
+  __syncthreads();
+  if (tid == 0) {
+    double t = 0.0;
+    for (int q = 0; q < ADAM_THREADS / 32; q++) t += s_part[q];
+    const float norm = (float)sqrt(t);
+    s_norm = norm;
+    *a.grad_norm = norm;
+  }
+  __syncthreads();
+  const float norm = s_norm;
+  if (!isfinite(norm)) return;                       // block-uniform
+  const float coef = fminf(a.max_norm / (norm + 1e-6f), 1.f);
+  const int32_t t = *a.step + 1;
+  const double bc1 = 1.0 - pow((double)a.beta1, (double)t), bc2 = 1.0 - pow((double)a.beta2, (double)t);
+  const float step_size = (float)((double)a.lr / bc1), bc2_sqrt = (float)sqrt(bc2);
+  const float b1 = a.beta1, b2 = a.beta2;
+  for (int64_t k = tid; k < a.n; k += ADAM_THREADS) {
+    const float g = a.grad[k] * coef;
+    const float m = b1 * a.m[k] + (1.f - b1) * g;
+    const float v = b2 * a.v[k] + (1.f - b2) * (g * g);
+    a.m[k] = m;
+    a.v[k] = v;
+    a.params[k] -= step_size * (m / (sqrtf(v) / bc2_sqrt + a.eps));
+  }
+  __syncthreads();                                   // every thread has read *step
+  if (tid == 0) *a.step = t;
 }
 
 static int64_t bwd_blocks(int64_t n_rows) {
@@ -814,6 +790,24 @@ static int launch_backward_na(EvalArgs<KIND> a, float* grad, cudaStream_t st) {
   }
   policy_backward_kernel<NA, KIND><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
   policy_grad_reduce_kernel<<<(PV<NA, KIND>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA, KIND>::N, grad);
+  return (int)cudaGetLastError();
+}
+
+template <int NA, int KIND>
+static int launch_ppo_na(PpoArgs<KIND> a, float* grad, float* stats, cudaStream_t st) {
+  const int64_t G = bwd_blocks(a.n_rows);
+  a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
+  a.inv_n = 1.f / (float)a.n_rows;
+  const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
+  if (sizeof(PpoSmem<BwdSmemOf<NA, KIND>>) + dyn > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(ppo_backward_kernel<NA, KIND>,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+  }
+  ppo_backward_kernel<NA, KIND><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
+  constexpr int NP = PV<NA, KIND>::N;
+  ppo_reduce_kernel<<<(NP + 31) / 32 + 1, 256, 0, st>>>(a.ws, (int)G, NP, grad, stats, (float)a.n_rows,
+                                                         a.value_coef, a.entropy_coef);
   return (int)cudaGetLastError();
 }
 
@@ -929,6 +923,44 @@ int pack_gauss(const gsm_policy_gauss_weights* w, gsm::GaussParams* p) {
   std::memcpy(p->head_b, w->mean_b, sizeof(w->mean_b));
   std::memcpy(&p->head_b[GSM_POLICY_GAUSS_DIM], w->value_b, sizeof(w->value_b));
   std::memcpy(p->log_std, w->log_std, sizeof(p->log_std));
+  return GSM_OK;
+}
+int check_loss_io(const gsm_ppo_loss_io* l, const char* who) {
+  if (!l) return pfailf(GSM_ERR_INVALID_ARG, who, "loss is NULL");
+  if (l->struct_size != sizeof(gsm_ppo_loss_io)) return pfailf(GSM_ERR_ABI, who, "loss.struct_size mismatch");
+  if (!l->old_logp || !l->old_values || !l->returns || !l->advantages || !l->adv_moments || !l->lagrange || !l->stats)
+    return pfailf(GSM_ERR_INVALID_ARG, who,
+                  "old_logp, old_values, returns, advantages, adv_moments, lagrange and stats are required");
+  if (!(l->clip > 0.f) || !(l->value_clip > 0.f)) return pfailf(GSM_ERR_INVALID_ARG, who, "clip and value_clip must be > 0");
+  if (!(l->value_coef >= 0.f) || !(l->entropy_coef >= 0.f))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "value_coef and entropy_coef must be >= 0");
+  return GSM_OK;
+}
+template <int KIND> void set_loss(gsm::PpoArgs<KIND>& a, const gsm_ppo_loss_io* l) {
+  a.old_logp = l->old_logp; a.old_values = l->old_values; a.returns = l->returns; a.adv = l->advantages;
+  a.adv_moments = l->adv_moments; a.lagrange = l->lagrange;
+  a.clip = l->clip; a.value_clip = l->value_clip; a.value_coef = l->value_coef; a.entropy_coef = l->entropy_coef;
+}
+// the argument checks and the launch of both heads; need: the workspace bytes for io->n_rows
+template <int KIND, class IO, class Launch>
+int ppo_backward_t(const IO* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace, size_t workspace_bytes,
+                   int device, void* stream, const char* who, int64_t (*need_fn)(const IO*), Launch launch) {
+  if (const int st = check_eval_io_t(io, who)) return st;
+  if (const int st = check_loss_io(loss, who)) return st;
+  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
+  const int64_t need = need_fn(io);
+  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than the ppo backward workspace for n_rows");
+  if (io->n_rows == 0) return GSM_OK;
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
+  gsm::PpoArgs<KIND> a{};
+  static_cast<gsm::EvalArgs<KIND>&>(a) = eval_args<KIND>(io);
+  set_loss(a, loss);
+  a.ws = (float*)workspace;
+  const int e = launch(a, grad, loss->stats, (cudaStream_t)stream);
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
   return GSM_OK;
 }
 }  // namespace
@@ -1059,6 +1091,60 @@ int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d
   a.ws = (float*)workspace;
   const int e = gsm::launch_backward_na<gsm::GD, gsm::HEAD_GAUSS>(a, grad, (cudaStream_t)stream);
   if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
+}
+
+int64_t gsm_ppo_backward_workspace(int64_t n_rows, int32_t n_actions) {
+  if (n_actions != 5 && n_actions != 9)
+    return pfailf(GSM_ERR_UNSUPPORTED, "gsm_ppo_backward_workspace", "n_actions must be 5 or 9");
+  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_ppo_backward_workspace", "n_rows < 0");
+  return gsm::bwd_blocks(n_rows) * (gsm::n_params(n_actions) + gsm::PPO_WS_STATS) * (int64_t)sizeof(float);
+}
+
+int64_t gsm_ppo_backward_workspace_gauss(int64_t n_rows) {
+  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_ppo_backward_workspace_gauss", "n_rows < 0");
+  return gsm::bwd_blocks(n_rows) * (GSM_POLICY_GAUSS_N_PARAMS + gsm::PPO_WS_STATS) * (int64_t)sizeof(float);
+}
+
+int gsm_ppo_backward(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace,
+                     size_t workspace_bytes, int device, void* stream) {
+  return ppo_backward_t<gsm::HEAD_CAT>(
+      io, loss, grad, workspace, workspace_bytes, device, stream, "gsm_ppo_backward",
+      +[](const gsm_policy_eval_io* q) { return gsm_ppo_backward_workspace(q->n_rows, q->n_actions); },
+      [&](const gsm::PpoArgs<gsm::HEAD_CAT>& a, float* g, float* st, cudaStream_t s) {
+        return io->n_actions == 5 ? gsm::launch_ppo_na<5, gsm::HEAD_CAT>(a, g, st, s)
+                                  : gsm::launch_ppo_na<9, gsm::HEAD_CAT>(a, g, st, s);
+      });
+}
+
+int gsm_ppo_backward_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss, float* grad,
+                           void* workspace, size_t workspace_bytes, int device, void* stream) {
+  return ppo_backward_t<gsm::HEAD_GAUSS>(
+      io, loss, grad, workspace, workspace_bytes, device, stream, "gsm_ppo_backward_gauss",
+      +[](const gsm_policy_gauss_eval_io* q) { return gsm_ppo_backward_workspace_gauss(q->n_rows); },
+      [](const gsm::PpoArgs<gsm::HEAD_GAUSS>& a, float* g, float* st, cudaStream_t s) {
+        return gsm::launch_ppo_na<gsm::GD, gsm::HEAD_GAUSS>(a, g, st, s);
+      });
+}
+
+int gsm_adam_step(float* params, const float* grad, float* m, float* v, int32_t* step, int64_t n, float lr,
+                  float beta1, float beta2, float eps, float max_grad_norm, float* grad_norm, int device,
+                  void* stream) {
+  const char* who = "gsm_adam_step";
+  if (!params || !grad || !m || !v || !step || !grad_norm)
+    return pfailf(GSM_ERR_INVALID_ARG, who, "params, grad, m, v, step and grad_norm are required");
+  if (n < 1) return pfailf(GSM_ERR_INVALID_ARG, who, "n < 1");
+  if (!(beta1 >= 0.f && beta1 < 1.f) || !(beta2 >= 0.f && beta2 < 1.f))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "beta1 and beta2 must lie in [0, 1)");
+  if (!(lr >= 0.f) || !(eps >= 0.f) || !(max_grad_norm > 0.f))
+    return pfailf(GSM_ERR_INVALID_ARG, who, "lr and eps must be >= 0 and max_grad_norm > 0");
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
+  const gsm::AdamArgs a{params, grad, m, v, step, grad_norm, n, lr, beta1, beta2, eps, max_grad_norm};
+  gsm::adam_step_kernel<<<1, gsm::ADAM_THREADS, 0, (cudaStream_t)stream>>>(a);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return pfail(GSM_ERR_CUDA, cudaGetErrorString(e));
   return GSM_OK;
 }
 

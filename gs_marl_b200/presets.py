@@ -38,3 +38,20 @@ def unverified_sensing_radius(n_agents: int) -> float:
 def unverified_spawn_extent(n_agents: int) -> float:
     """World half-extent grows with sqrt(N/3) (demo GIFs zoom out with N; SURVEY App. C)."""
     return math.sqrt(max(n_agents, 3) / 3.0)
+
+# PPO-Lagrangian hyper-parameters typical of the MAPPO / MAPPO-L lineage (the reference's learner and
+# its config are withheld); `learner.LagrangianPPO` takes every one as a required keyword.
+UNVERIFIED_PPO_LAG = dict(
+    clip=0.2,
+    value_clip=0.2,
+    value_coef=1.0,
+    entropy_coef=0.01,
+    lr=5e-4,
+    betas=(0.9, 0.999),
+    eps=1e-5,
+    max_grad_norm=10.0,
+    ppo_epoch=5,
+    num_mini_batch=1,
+    lagrangian_lr=1e-2,
+    cost_limit=0.0,
+)

@@ -418,6 +418,64 @@ int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d
                               const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                               int device, void* stream);
 
+/* ---- PPO-Lagrangian update (SPEC.md §14): the loss fused into the learner backward, one Adam step ----
+ * Declared stand-in for the lineage's MAPPO-Lagrangian learner (withheld).  One minibatch of n rows; row
+ * i reads source row src = rows ? rows[i] : i of the buffer's obs / nbr_feat / nbr_cnt / actions (the
+ * eval io, whose output pointers are ignored) and of old_logp / old_values / returns / advantages:
+ *   Ahat_h = (A_h - mu_h) / (sigma_h + 1e-5);  Abar = Ahat_0 - lambda Ahat_1;  rho = exp(logp - old_logp)
+ *   L_pi = -(1/n) sum min(rho Abar, clip(rho, 1 - clip, 1 + clip) Abar)
+ *   vc_h = old_v_h + clip(v_h - old_v_h, -value_clip, value_clip)
+ *   L_V  = (1/n) sum_h sum max(1/2 (v_h - R_h)^2, 1/2 (vc_h - R_h)^2)
+ *   L    = L_pi + value_coef L_V - entropy_coef (1/n) sum entropy
+ * logp, entropy and values are gsm_policy_evaluate's (bit-identical).  grad = dL/dparams through the seeds
+ *   d_logp = -rho Abar / n where rho Abar <= clip(rho) Abar, else 0;  d_entropy = -entropy_coef / n;
+ *   d_v_h = value_coef (v_h - R_h) / n where (v_h - R_h)^2 >= (vc_h - R_h)^2, else value_coef (vc_h - R_h) / n
+ *   where |v_h - old_v_h| <= value_clip, else 0  (torch autograd of L except at exact ties);
+ * stats [GSM_PPO_STAT_FIELDS] = means over the n rows of: L_pi, L_V reward head, L_V cost head, entropy,
+ * rho, clipped (|rho - 1| > clip), approx KL (old_logp - logp), then L.  Deterministic (a fixed partition
+ * of the rows, fixed-order sums, no atomics); three launches with gsm_adam_step, no host sync. */
+#define GSM_PPO_STAT_FIELDS 8
+
+typedef struct gsm_ppo_loss_io {   /* DEVICE pointers */
+  uint32_t struct_size;          /* = sizeof(gsm_ppo_loss_io); checked                                */
+  int32_t reserved;              /* 0 */
+  const float* old_logp;         /* [src_rows]     the buffer's logp                                  */
+  const float* old_values;       /* [src_rows][2]  the buffer's values[:-1]                           */
+  const float* returns;          /* [src_rows][2]  gsm_gae returns                                    */
+  const float* advantages;       /* [src_rows][2]  gsm_gae advantages                                 */
+  const float* adv_moments;      /* [4] (mu_0, sigma_0, mu_1, sigma_1) over the whole rollout         */
+  const float* lagrange;         /* [1] lambda >= 0                                                   */
+  float* stats;                  /* [GSM_PPO_STAT_FIELDS] out                                         */
+  float clip;                    /* > 0 */
+  float value_clip;              /* > 0 */
+  float value_coef;              /* >= 0 */
+  float entropy_coef;            /* >= 0 */
+} gsm_ppo_loss_io;
+
+/* Workspace bytes gsm_ppo_backward(_gauss) needs (a function of n_rows and n_actions only);
+ * GSM_ERR_INVALID_ARG for n_rows < 0, GSM_ERR_UNSUPPORTED for n_actions not 5 or 9. */
+int64_t gsm_ppo_backward_workspace(int64_t n_rows, int32_t n_actions);
+int64_t gsm_ppo_backward_workspace_gauss(int64_t n_rows);
+
+/* GSM_ERR_ABI for a bad struct_size; GSM_ERR_INVALID_ARG for a missing pointer, a short workspace,
+ * clip <= 0, value_clip <= 0 or a negative coefficient.  n_rows == 0 leaves grad and stats untouched. */
+int gsm_ppo_backward(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace,
+                     size_t workspace_bytes, int device, void* stream);
+int gsm_ppo_backward_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss, float* grad,
+                           void* workspace, size_t workspace_bytes, int device, void* stream);
+
+/* torch.nn.utils.clip_grad_norm_(max_grad_norm) then torch.optim.Adam (no weight decay, no amsgrad), one
+ * launch over n floats:  norm = ||grad||_2 (fixed-order sum);  g = grad min(1, max_grad_norm / (norm + 1e-6));
+ * t = *step + 1;  m = beta1 m + (1 - beta1) g;  v = beta2 v + (1 - beta2) g^2;
+ * params -= (lr / (1 - beta1^t)) m / (sqrt(v) / sqrt(1 - beta2^t) + eps)  (bias corrections in fp64);
+ * *step = t;  *grad_norm = norm.  A non-finite norm skips the step: params, m, v and *step are left
+ * unchanged (torch would write NaN); *grad_norm is still written.  grad is not modified.  DEVICE pointers.
+ * GSM_ERR_INVALID_ARG for a missing pointer, n < 1, beta1 or beta2 outside [0, 1), lr < 0, eps < 0 or
+ * max_grad_norm <= 0. */
+int gsm_adam_step(float* params, const float* grad, float* m, float* v, int32_t* step, int64_t n, float lr,
+                  float beta1, float beta2, float eps, float max_grad_norm, float* grad_norm, int device,
+                  void* stream);
+
 /* n_steps of {actor forward + sampling, env step} enqueued on `stream` with no host sync (2
  * kernels per step; capturable into a CUDA graph).  io->obs / nbr_* / adj / assign point at slot 0
  * of [n_steps+1][...] tensors whose slot 0 already holds the current observation (gsm_reset,
