@@ -39,17 +39,20 @@ namespace gsm {
 
 constexpr int H = GSM_POLICY_HIDDEN;
 
-struct PolicyParams {                 // kernel-parameter image of gsm_policy_weights
+// The kernel-parameter image both heads share: the embedding and NH head rows.
+template <int NH> struct EmbedParams {
   float ego_w[H][GSM_OBS_DIM];
   float ego_b[H];
   float nbr_w[H][GSM_NBR_FEAT_DIM];
   float nbr_b[H];
   float att_w[H];
-  // rows 0..NA-1: action logits; rows NA, NA+1: the two critics (reward value, cost value)
-  float head_w[GSM_POLICY_MAX_ACTIONS + GSM_POLICY_VALUE_HEADS][2 * H];
-  float head_b[GSM_POLICY_MAX_ACTIONS + GSM_POLICY_VALUE_HEADS];
+  // rows 0..NA-1: the head (logits or means); rows NA, NA+1: the two critics (reward value, cost value)
+  float head_w[NH][2 * H];
+  float head_b[NH];
   float att_b;
 };
+// kernel-parameter image of gsm_policy_weights
+using PolicyParams = EmbedParams<GSM_POLICY_MAX_ACTIONS + GSM_POLICY_VALUE_HEADS>;
 
 // Head kinds (SPEC.md §10 / §10b).  The embedding h = [e; sum_r a_r m_r] and everything that computes
 // it are shared; the kind selects the weights' image, the action type and the epilogue.
@@ -59,18 +62,11 @@ struct PolicyParams {                 // kernel-parameter image of gsm_policy_we
 enum HeadKind { HEAD_CAT = 0, HEAD_GAUSS = 1 };
 constexpr int GD = GSM_POLICY_GAUSS_DIM;
 
-struct GaussParams {                  // kernel-parameter image of gsm_policy_gauss_weights
-  float ego_w[H][GSM_OBS_DIM];
-  float ego_b[H];
-  float nbr_w[H][GSM_NBR_FEAT_DIM];
-  float nbr_b[H];
-  float att_w[H];
-  // rows 0..GD-1: the means; rows GD, GD+1: the two critics
-  float head_w[GD + GSM_POLICY_VALUE_HEADS][2 * H];
-  float head_b[GD + GSM_POLICY_VALUE_HEADS];
-  float att_b;
+// kernel-parameter image of gsm_policy_gauss_weights: log_std right behind the shared part
+struct GaussParams : EmbedParams<GD + GSM_POLICY_VALUE_HEADS> {
   float log_std[GD];
 };
+static_assert(sizeof(GaussParams) == sizeof(EmbedParams<GD + GSM_POLICY_VALUE_HEADS>) + sizeof(float) * GD, "layout");
 
 template <int KIND> struct Head;
 template <> struct Head<HEAD_CAT> { using Params = PolicyParams; using Act = int32_t; };
@@ -85,8 +81,6 @@ template <int KIND> struct ActorIO {
   int64_t n_rows; uint64_t row_offset, seed, step;
   int K, greedy;
 };
-using PolicyIO = ActorIO<HEAD_CAT>;
-using GaussIO = ActorIO<HEAD_GAUSS>;
 
 __device__ __forceinline__ void philox_p(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                          uint32_t k0, uint32_t k1, uint32_t out[4]) {
@@ -101,7 +95,7 @@ __device__ __forceinline__ void philox_p(uint32_t c0, uint32_t c1, uint32_t c2, 
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 
-// the categorical sampler's map of a Philox word to (0, 1), below
+// a Philox word to (0, 1): 23 random bits + half a step, every value k * 2^-23 + 2^-24 is exact in fp32
 __device__ __forceinline__ float unit_open(uint32_t x) {
   return (float)(x >> 9) * 1.1920928955078125e-7f + 5.9604644775390625e-8f;
 }
@@ -337,9 +331,7 @@ graph_actor_kernel(const __grid_constant__ typename Head<KIND>::Params w, const 
       for (int q = 0; q < 4; q++) {
         const int a = 4 * b + q;
         if (a < NA) {
-          // 23 random bits + half a step: every value k * 2^-23 + 2^-24 is exact in fp32 and lies in (0, 1)
-          const float u = (float)(r[q] >> 9) * 1.1920928955078125e-7f + 5.9604644775390625e-8f;
-          const float v = z[a] - logf(-logf(u));
+          const float v = z[a] - logf(-logf(unit_open(r[q])));
           if (a == 0 || v > bv) { bv = v; best = a; zb = z[a]; }
         }
       }
@@ -402,7 +394,7 @@ __global__ void __launch_bounds__(256) gae_kernel(const __grid_constant__ GaePar
 // to what gsm_policy_act / gsm_collect wrote.  One row per thread instead of the actor's flattened
 // row items: simpler, divergent on nbr_cnt, and the learner pass is not the collect loop's hot path.
 //
-// Backward (policy_backward_kernel), with h = [e; g], g = sum_r a_r m_r, Z = [z; v], W = [W_h; W_v]:
+// Backward (backward_kernel), with h = [e; g], g = sum_r a_r m_r, Z = [z; v], W = [W_h; W_v]:
 //   dz = d_logp (onehot(a) - p) - d_entropy p o (log p + entropy),  dZ = [dz; d_values]
 //   dh = W^T dZ;  dW += dZ h^T;  de = dh[:H] o [e > 0];  dg = dh[H:]
 //   m_r . dg = dZ . hr_r with hr_r = W[:, H:] m_r, so ds_r = a_r (dZ . hr_r - dZ . (sum_r a_r hr_r))
@@ -634,20 +626,200 @@ __device__ __forceinline__ void ppo_seeds(const PpoArgs<KIND>& p, int64_t src, f
   st[3] = ent; st[4] = rho; st[5] = fabsf(rho - 1.f) > p.clip ? 1.f : 0.f; st[6] = olp - lp;
 }
 
-#define GSM_BWD_KERNEL policy_backward_kernel
-#define GSM_BWD_ARGS EvalArgs
-#define GSM_BWD_LOSS false
-#include "gsm_policy_backward.inl"
-#undef GSM_BWD_KERNEL
-#undef GSM_BWD_ARGS
-#undef GSM_BWD_LOSS
-#define GSM_BWD_KERNEL ppo_backward_kernel
-#define GSM_BWD_ARGS PpoArgs
-#define GSM_BWD_LOSS true
-#include "gsm_policy_backward.inl"
-#undef GSM_BWD_KERNEL
-#undef GSM_BWD_ARGS
-#undef GSM_BWD_LOSS
+// The backward kernel.  LOSS = false (gsm_policy_backward): the seeds d_logp, d_entropy, d_values are
+// inputs.  LOSS = true (gsm_ppo_backward): phase A computes them from the PPO-Lagrangian loss (ppo_seeds,
+// SPEC.md §14) and the block also sums the loss statistics.  The loss mode adds code only under
+// `if constexpr (LOSS)`, so the LOSS = false instances carry none of it.  (A __forceinline__ device function
+// shared by two thin kernels would not do: the inliner changes the optimisation pipeline and the SASS of
+// every instance.)
+template <int KIND, bool LOSS> using BwdArgs = std::conditional_t<LOSS, PpoArgs<KIND>, EvalArgs<KIND>>;
+template <int NA, int KIND, bool LOSS>
+using BwdSmemT = std::conditional_t<LOSS, PpoSmem<BwdSmemOf<NA, KIND>>, BwdSmemOf<NA, KIND>>;
+
+template <int NA, int KIND, bool LOSS>
+__global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant__ BwdArgs<KIND, LOSS> p) {
+  using P = PV<NA, KIND>;
+  constexpr int NZ = NA + V2, NP = P::N, WS = NP + (LOSS ? PPO_WS_STATS : 0);
+  __shared__ BwdSmemT<NA, KIND, LOSS> sm;
+  extern __shared__ float s_rows[];    // [BWD_AG][K][2]: (a_r, ds_r) of the valid rows; a float2 array
+                                       // would round every kernel's static shared memory in this file up to 16 B
+  const int tid = threadIdx.x;
+  for (int k = tid; k < NP; k += BWD_AG) sm.w[k] = p.params[k];
+  const float* W = sm.w;
+  // phase-B accumulators of hidden unit j = tid, live across the tiles
+  float gwe[GSM_OBS_DIM], gwn[GSM_NBR_FEAT_DIM], ghe[NZ], ghg[NZ];
+  float gbe = 0.f, gbn = 0.f, gwa = 0.f, gsc = 0.f;   // gsc: bias sum of dZ[tid] (tid < NZ) or db_a (tid = H-1)
+#pragma unroll
+  for (int k = 0; k < GSM_OBS_DIM; k++) { gwe[k] = 0.f; gwn[k] = 0.f; }
+#pragma unroll
+  for (int a = 0; a < NZ; a++) { ghe[a] = 0.f; ghg[a] = 0.f; }
+  if constexpr (LOSS) { if (tid < PPO_ROW_STATS) sm.stacc[tid] = 0.f; }
+  __syncthreads();
+
+  for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {   // block-uniform
+    const int64_t base = tile * BWD_AG;
+    const int nag = p.n_rows - base < BWD_AG ? (int)(p.n_rows - base) : BWD_AG;
+    // ---- phase A: thread = row ----
+    if (tid < nag) {
+      const int64_t i = base + tid;
+      const int64_t src = p.rows ? p.rows[i] : i;
+      const int cnt = clamp_cnt(p.nbr_cnt[src], p.K);
+      const float* o = p.obs + src * GSM_OBS_DIM;
+      const float* f = p.nbr_feat + src * p.K * GSM_NBR_FEAT_DIM;
+      float z[NZ], acc[NZ], mx, s;
+      row_forward<NA, KIND>(W, o, f, cnt, z, acc, mx, s);
+      // The categorical dz stays at this scope for BOTH kinds, on purpose: guarded by
+      // `if constexpr (KIND == HEAD_CAT)` (or nested in an if-constexpr / else) it changes the register
+      // allocation and SASS of the categorical instances, which must stay as they were.  For the
+      // Gaussian it is dead code: act is the constant 0, every dz[a < NA] it writes is rewritten by the
+      // Gaussian block below and nothing else reads its values, so the compiler removes it (same
+      // registers as the nested form).  Only dlp and dent are shared with the Gaussian block.
+      float zm, se;
+      const int act = KIND == HEAD_CAT ? (int)p.actions[src] : 0;
+      const float lp = row_logp<NA>(z, act, zm, se);
+      float dlp = 0.f, dent = 0.f, dvl[V2];
+      if constexpr (!LOSS) { dlp = p.d_logp ? p.d_logp[i] : 0.f; dent = p.d_entropy ? p.d_entropy[i] : 0.f; }
+      const float lse = zm + logf(se), inv_se = 1.f / se;
+      float pr[NA], ent = 0.f;
+#pragma unroll
+      for (int a = 0; a < NA; a++) { pr[a] = expf(z[a] - zm) * inv_se; ent = fmaf(pr[a], z[a] - zm, ent); }
+      ent = logf(se) - ent;
+      // the categorical loss: lp and ent are evaluate's (same row_logp, same entropy chain)
+      if constexpr (LOSS && KIND == HEAD_CAT) ppo_seeds(p, src, lp, ent, z + NA, dlp, dent, dvl, sm.st[tid]);
+      // an action outside [0, NA) has no one-hot: its NaN logp poisons the gradient it feeds
+      const float bad = (dlp != 0.f && lp != lp) ? __int_as_float(0x7fc00000) : 0.f;
+      float dz[NZ];
+#pragma unroll
+      for (int a = 0; a < NA; a++)
+        dz[a] = dlp * ((act == a ? 1.f : 0.f) - pr[a] + bad) - dent * pr[a] * ((z[a] - lse) + ent);
+      if constexpr (KIND == HEAD_GAUSS) {
+        // SPEC.md §12b: dmu_d = d_logp delta_d exp(-log_std_d);
+        // dlog_std_d = d_logp (delta_d^2 - 1) + d_entropy.  A non-finite action (NaN logp) gives a NaN
+        // gradient exactly where d_logp != 0; where d_logp == 0 the action does not enter it.
+        const float ls0 = W[P::LS], ls1 = W[P::LS + 1];
+        float d0, d1;
+        const float glp = gauss_logp(p.actions[src * GD], p.actions[src * GD + 1], z[0], z[1], ls0, ls1, d0, d1);
+        if constexpr (LOSS) ppo_seeds(p, src, glp, gauss_entropy(ls0, ls1), z + NA, dlp, dent, dvl, sm.st[tid]);
+        const bool use = dlp != 0.f;
+        const float gbad = (use && glp != glp) ? __int_as_float(0x7fc00000) : 0.f;
+        dz[0] = use ? dlp * d0 * expf(-ls0) + gbad : 0.f;
+        dz[1] = use ? dlp * d1 * expf(-ls1) + gbad : 0.f;
+        sm.dls[tid][0] = (use ? dlp * fmaf(d0, d0, -1.f) + gbad : 0.f) + dent;
+        sm.dls[tid][1] = (use ? dlp * fmaf(d1, d1, -1.f) + gbad : 0.f) + dent;
+      }
+#pragma unroll
+      for (int v = 0; v < V2; v++) {
+        if constexpr (LOSS) dz[NA + v] = dvl[v];
+        else dz[NA + v] = p.d_values ? p.d_values[i * V2 + v] : 0.f;
+      }
+      float dsum = 0.f;
+      if (cnt > 0) {
+        const float inv = 1.f / s;
+        float gdg = 0.f;                 // g . dg = dZ . sum_r a_r hr_r
+#pragma unroll
+        for (int a = 0; a < NZ; a++) gdg = fmaf(dz[a], acc[a] * inv, gdg);
+        float* pr_rows = s_rows + 2 * tid * p.K;
+        for (int r = 0; r < cnt; r++) {  // second pass: the same t_r, hr_r as the first
+          float hr[NZ];
+          const float t = nbr_row<NA, KIND>(W, f + r * GSM_NBR_FEAT_DIM, hr);
+          const float ar = expf(t - mx) * inv;
+          float q = 0.f;
+#pragma unroll
+          for (int a = 0; a < NZ; a++) q = fmaf(dz[a], hr[a], q);
+          const float ds = ar * (q - gdg);
+          pr_rows[2 * r] = ar; pr_rows[2 * r + 1] = ds;
+          dsum += ds;
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < GSM_OBS_DIM; k++) sm.obs[tid][k] = o[k];
+#pragma unroll
+      for (int a = 0; a < NZ; a++) sm.dz[tid][a] = dz[a];
+      sm.dsum[tid] = dsum;
+      sm.cnt[tid] = cnt;
+      sm.src[tid] = src;
+    }
+    __syncthreads();
+    // ---- phase B: thread = hidden unit j ----
+    {
+      const int j = tid;
+      float we[GSM_OBS_DIM], wn[GSM_NBR_FEAT_DIM], wh[NZ], wg[NZ];
+#pragma unroll
+      for (int k = 0; k < GSM_OBS_DIM; k++) { we[k] = W[P::EW + j * GSM_OBS_DIM + k]; wn[k] = W[P::NW + j * GSM_NBR_FEAT_DIM + k]; }
+#pragma unroll
+      for (int a = 0; a < NZ; a++) { wh[a] = W[P::row(a) + j]; wg[a] = W[P::row(a) + H + j]; }
+      const float be = W[P::EB + j], bn = W[P::NB + j], wa = W[P::AW + j];
+      for (int ag = 0; ag < nag; ag++) {
+        float dZ[NZ];
+#pragma unroll
+        for (int a = 0; a < NZ; a++) dZ[a] = sm.dz[ag][a];
+        float u = be;
+#pragma unroll
+        for (int k = 0; k < GSM_OBS_DIM; k++) u = fmaf(we[k], sm.obs[ag][k], u);
+        const float e = fmaxf(u, 0.f);
+        float dh = 0.f;
+#pragma unroll
+        for (int a = 0; a < NZ; a++) { dh = fmaf(wh[a], dZ[a], dh); ghe[a] = fmaf(dZ[a], e, ghe[a]); }
+        const float de = u > 0.f ? dh : 0.f;            // ReLU'(0) = 0, as in torch
+#pragma unroll
+        for (int k = 0; k < GSM_OBS_DIM; k++) gwe[k] = fmaf(de, sm.obs[ag][k], gwe[k]);
+        gbe += de;
+        const int c = sm.cnt[ag];                        // block-uniform: no divergence
+        if (c > 0) {
+          float dg = 0.f, g = 0.f;
+#pragma unroll
+          for (int a = 0; a < NZ; a++) dg = fmaf(wg[a], dZ[a], dg);
+          const float* f = p.nbr_feat + sm.src[ag] * p.K * GSM_NBR_FEAT_DIM;
+          const float* rr = s_rows + 2 * ag * p.K;
+          for (int r = 0; r < c; r++) {
+            float fr[GSM_NBR_FEAT_DIM];
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) fr[k] = __ldg(f + r * GSM_NBR_FEAT_DIM + k);
+            float um = bn;
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) um = fmaf(wn[k], fr[k], um);
+            const float m = fmaxf(um, 0.f);
+            const float ar = rr[2 * r], ds = rr[2 * r + 1];
+            g = fmaf(ar, m, g);
+            const float du = um > 0.f ? fmaf(ar, dg, ds * wa) : 0.f;
+#pragma unroll
+            for (int k = 0; k < GSM_NBR_FEAT_DIM; k++) gwn[k] = fmaf(du, fr[k], gwn[k]);
+            gbn += du;
+            gwa = fmaf(ds, m, gwa);
+          }
+#pragma unroll
+          for (int a = 0; a < NZ; a++) ghg[a] = fmaf(dZ[a], g, ghg[a]);
+        }
+        if (j < NZ) gsc += sm.dz[ag][j];
+        else if (j == H - 1) gsc += sm.dsum[ag];
+        else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) gsc += sm.dls[ag][j - NZ]; }
+      }
+    }
+    if constexpr (LOSS) {                // the tile's statistics, in row order
+      if (tid < PPO_ROW_STATS) {
+        float acc = sm.stacc[tid];
+        for (int ag = 0; ag < nag; ag++) acc += sm.st[ag][tid];
+        sm.stacc[tid] = acc;
+      }
+    }
+    __syncthreads();                     // before the next tile overwrites the row state
+  }
+  // ---- this block's partial gradient, in vector order (then its statistics) ----
+  float* out = p.ws + (int64_t)blockIdx.x * WS;
+  const int j = tid;
+#pragma unroll
+  for (int k = 0; k < GSM_OBS_DIM; k++) {
+    out[P::EW + j * GSM_OBS_DIM + k] = gwe[k];
+    out[P::NW + j * GSM_NBR_FEAT_DIM + k] = gwn[k];
+  }
+  out[P::EB + j] = gbe; out[P::NB + j] = gbn; out[P::AW + j] = gwa;
+#pragma unroll
+  for (int a = 0; a < NZ; a++) { out[P::row(a) + j] = ghe[a]; out[P::row(a) + H + j] = ghg[a]; }
+  if (j < NZ) out[j < NA ? P::HB + j : P::VB + (j - NA)] = gsc;
+  else if (j == H - 1) out[P::AB] = gsc;
+  else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) out[P::LS + (j - NZ)] = gsc; }
+  if constexpr (LOSS) { if (j < PPO_WS_STATS) out[NP + j] = j < PPO_ROW_STATS ? sm.stacc[j] : 0.f; }
+}
 
 // grad[k] = sum of the G partials in a fixed order: warp w sums partials w, w + 8, ... (lane = k),
 // then warp 0 adds the 8 warp sums in order.
@@ -671,7 +843,7 @@ __global__ void __launch_bounds__(256) policy_grad_reduce_kernel(const float* __
   }
 }
 
-// ppo_backward_kernel's partials: blocks 0 .. ceil(NP / 32) - 1 reduce the gradient exactly as
+// backward_kernel<..., true>'s partials: blocks 0 .. ceil(NP / 32) - 1 reduce the gradient exactly as
 // policy_grad_reduce_kernel does (partials of stride NP + PPO_WS_STATS); the last block reduces the
 // statistics in the same order, then lanes 0..6 write their means over the n rows and lane 0 adds
 // L = L_pi + c_v (L_V reward + L_V cost) - c_e entropy.  Counts (the clip fraction) are exact in fp32
@@ -761,75 +933,53 @@ static int64_t bwd_blocks(int64_t n_rows) {
   return tiles < BWD_MAX_BLOCKS ? tiles : BWD_MAX_BLOCKS;
 }
 
-static int n_params(int n_actions) { return n_actions == 5 ? PV<5, HEAD_CAT>::N : PV<9, HEAD_CAT>::N; }
+// f(std::integral_constant<int, NA>()) for the compiled instance of a head: NA = n_actions (5 or 9, checked
+// by the caller) for the categorical head, GD for the Gaussian
+template <int KIND, class F> static auto for_na(int n_actions, F f) {
+  if constexpr (KIND == HEAD_GAUSS) return f(std::integral_constant<int, GD>());
+  else return n_actions == 5 ? f(std::integral_constant<int, 5>()) : f(std::integral_constant<int, 9>());
+}
 
-static int launch_evaluate(const EvalArgs<HEAD_CAT>& a, int n_actions, cudaStream_t st) {
+template <int KIND>
+static int launch_actor(const typename Head<KIND>::Params& w, const ActorIO<KIND>& io, int n_actions, cudaStream_t st) {
+  if (io.n_rows == 0) return 0;
+  const unsigned grid = (unsigned)((io.n_rows + 127) / 128);   // 128 = AG, the agents a block owns
+  for_na<KIND>(n_actions, [&](auto na) {
+    constexpr int NA = decltype(na)::value;
+    if (io.values) graph_actor_kernel<NA, GSM_POLICY_VALUE_HEADS, KIND><<<grid, 128, 0, st>>>(w, io);
+    else graph_actor_kernel<NA, 0, KIND><<<grid, 128, 0, st>>>(w, io);
+  });
+  return (int)cudaGetLastError();
+}
+
+template <int KIND> static int launch_evaluate(const EvalArgs<KIND>& a, int n_actions, cudaStream_t st) {
   const unsigned grid = (unsigned)((a.n_rows + 127) / 128);
-  if (n_actions == 5) policy_eval_kernel<5, HEAD_CAT><<<grid, 128, 0, st>>>(a);
-  else policy_eval_kernel<9, HEAD_CAT><<<grid, 128, 0, st>>>(a);
+  for_na<KIND>(n_actions, [&](auto na) { policy_eval_kernel<decltype(na)::value, KIND><<<grid, 128, 0, st>>>(a); });
   return (int)cudaGetLastError();
 }
 
-static int launch_evaluate_gauss(const EvalArgs<HEAD_GAUSS>& a, cudaStream_t st) {
-  policy_eval_kernel<GD, HEAD_GAUSS><<<(unsigned)((a.n_rows + 127) / 128), 128, 0, st>>>(a);
-  return (int)cudaGetLastError();
-}
-
-template <int NA, int KIND>
-static int launch_backward_na(EvalArgs<KIND> a, float* grad, cudaStream_t st) {
+// the backward kernel, then the reduction of its G partials: the gradient (and, with the loss, the statistics)
+template <int NA, int KIND, bool LOSS>
+static int launch_backward(BwdArgs<KIND, LOSS> a, float* grad, float* stats, cudaStream_t st) {
+  constexpr int NP = PV<NA, KIND>::N;
   const int64_t G = bwd_blocks(a.n_rows);
   a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
+  if constexpr (LOSS) a.inv_n = 1.f / (float)a.n_rows;
   const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
-  if (sizeof(BwdSmemOf<NA, KIND>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
-    const cudaError_t e = cudaFuncSetAttribute(policy_backward_kernel<NA, KIND>,
+  if (sizeof(BwdSmemT<NA, KIND, LOSS>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
+    const cudaError_t e = cudaFuncSetAttribute(backward_kernel<NA, KIND, LOSS>,
                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) {            // max_nbrs beyond the block's shared memory: report it here and clear
       cudaGetLastError();              // it, or the next launch's cudaGetLastError() would report it again
       return (int)e;
     }
   }
-  policy_backward_kernel<NA, KIND><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
-  policy_grad_reduce_kernel<<<(PV<NA, KIND>::N + 31) / 32, 256, 0, st>>>(a.ws, (int)G, PV<NA, KIND>::N, grad);
-  return (int)cudaGetLastError();
-}
-
-template <int NA, int KIND>
-static int launch_ppo_na(PpoArgs<KIND> a, float* grad, float* stats, cudaStream_t st) {
-  const int64_t G = bwd_blocks(a.n_rows);
-  a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
-  a.inv_n = 1.f / (float)a.n_rows;
-  const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
-  if (sizeof(PpoSmem<BwdSmemOf<NA, KIND>>) + dyn > 48 * 1024) {
-    const cudaError_t e = cudaFuncSetAttribute(ppo_backward_kernel<NA, KIND>,
-                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
-  }
-  ppo_backward_kernel<NA, KIND><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
-  constexpr int NP = PV<NA, KIND>::N;
-  ppo_reduce_kernel<<<(NP + 31) / 32 + 1, 256, 0, st>>>(a.ws, (int)G, NP, grad, stats, (float)a.n_rows,
-                                                         a.value_coef, a.entropy_coef);
-  return (int)cudaGetLastError();
-}
-
-static int launch_actor(const PolicyParams& w, const PolicyIO& io, int n_actions, cudaStream_t st) {
-  if (io.n_rows == 0) return 0;
-  const int block = 128;            // = AG, the agents a block owns
-  const int64_t grid = (io.n_rows + block - 1) / block;
-  constexpr int V = GSM_POLICY_VALUE_HEADS;
-  const unsigned gd = (unsigned)grid;
-  if (n_actions == 5 && !io.values) graph_actor_kernel<5, 0, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 5) graph_actor_kernel<5, V, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 9 && !io.values) graph_actor_kernel<9, 0, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
-  else if (n_actions == 9) graph_actor_kernel<9, V, HEAD_CAT><<<gd, block, 0, st>>>(w, io);
-  else return -1;
-  return (int)cudaGetLastError();
-}
-
-static int launch_actor_gauss(const GaussParams& w, const GaussIO& io, cudaStream_t st) {
-  if (io.n_rows == 0) return 0;
-  const unsigned gd = (unsigned)((io.n_rows + 127) / 128);
-  if (!io.values) graph_actor_kernel<GD, 0, HEAD_GAUSS><<<gd, 128, 0, st>>>(w, io);
-  else graph_actor_kernel<GD, GSM_POLICY_VALUE_HEADS, HEAD_GAUSS><<<gd, 128, 0, st>>>(w, io);
+  backward_kernel<NA, KIND, LOSS><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
+  if constexpr (LOSS)
+    ppo_reduce_kernel<<<(NP + 31) / 32 + 1, 256, 0, st>>>(a.ws, (int)G, NP, grad, stats, (float)a.n_rows,
+                                                           a.value_coef, a.entropy_coef);
+  else
+    policy_grad_reduce_kernel<<<(NP + 31) / 32, 256, 0, st>>>(a.ws, (int)G, NP, grad);
   return (int)cudaGetLastError();
 }
 
@@ -842,21 +992,9 @@ int pfail(int status, const char* msg) {
   std::strncpy(g_policy_err, msg, sizeof(g_policy_err) - 1);
   return status;
 }
-int pack(const gsm_policy_weights* w, gsm::PolicyParams* p) {
-  if (!w) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy: weights is NULL");
-  if (w->struct_size != sizeof(gsm_policy_weights)) return pfail(GSM_ERR_ABI, "gsm_policy: weights.struct_size mismatch");
-  if (w->n_actions != 5 && w->n_actions != 9)
-    return pfail(GSM_ERR_UNSUPPORTED, "gsm_policy: compiled actor instances exist for n_actions 5 and 9 only");
-  static_assert(sizeof(p->ego_w) == sizeof(w->ego_w), "layout");
-  std::memcpy(p->ego_w, w->ego_w, sizeof(p->ego_w));   std::memcpy(p->ego_b, w->ego_b, sizeof(p->ego_b));
-  std::memcpy(p->nbr_w, w->nbr_w, sizeof(p->nbr_w));   std::memcpy(p->nbr_b, w->nbr_b, sizeof(p->nbr_b));
-  std::memcpy(p->att_w, w->att_w, sizeof(p->att_w));   p->att_b = w->att_b;
-  std::memset(p->head_w, 0, sizeof(p->head_w)); std::memset(p->head_b, 0, sizeof(p->head_b));
-  std::memcpy(p->head_w, w->head_w, sizeof(float) * 2 * GSM_POLICY_HIDDEN * w->n_actions);
-  std::memcpy(p->head_b, w->head_b, sizeof(float) * w->n_actions);
-  std::memcpy(p->head_w[w->n_actions], w->value_w, sizeof(w->value_w));   // critics right behind the logits' rows
-  std::memcpy(&p->head_b[w->n_actions], w->value_b, sizeof(w->value_b));
-  return GSM_OK;
+int pfailf(int status, const char* who, const char* msg) {
+  snprintf(g_policy_err, sizeof(g_policy_err), "%s: %s", who, msg);
+  return status;
 }
 struct DevGuard {
   int prev = -1;
@@ -881,12 +1019,62 @@ int check_device(int device, const char* who) {
   }
   return GSM_OK;
 }
-int pfailf(int status, const char* who, const char* msg) {
-  snprintf(g_policy_err, sizeof(g_policy_err), "%s: %s", who, msg);
-  return status;
+// check_device, then launch() (a cudaError_t) with `device` current; GSM_OK or the error status to return.
+template <class Launch> int on_device(int device, const char* who, Launch launch) {
+  if (const int ds = check_device(device, who)) return ds;
+  DevGuard guard(device);
+  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
+  const int e = launch();
+  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
+  return GSM_OK;
 }
+
+// the embedding and the critics, which follow the head's na rows
+template <class W, class P> void pack_embedding(const W* w, P* p, int na) {
+  static_assert(sizeof(p->ego_w) == sizeof(w->ego_w), "layout");
+  std::memcpy(p->ego_w, w->ego_w, sizeof(p->ego_w));   std::memcpy(p->ego_b, w->ego_b, sizeof(p->ego_b));
+  std::memcpy(p->nbr_w, w->nbr_w, sizeof(p->nbr_w));   std::memcpy(p->nbr_b, w->nbr_b, sizeof(p->nbr_b));
+  std::memcpy(p->att_w, w->att_w, sizeof(p->att_w));   p->att_b = w->att_b;
+  std::memcpy(p->head_w[na], w->value_w, sizeof(w->value_w));
+  std::memcpy(&p->head_b[na], w->value_b, sizeof(w->value_b));
+}
+int pack(const gsm_policy_weights* w, gsm::PolicyParams* p) {
+  if (!w) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy: weights is NULL");
+  if (w->struct_size != sizeof(gsm_policy_weights)) return pfail(GSM_ERR_ABI, "gsm_policy: weights.struct_size mismatch");
+  if (w->n_actions != 5 && w->n_actions != 9)
+    return pfail(GSM_ERR_UNSUPPORTED, "gsm_policy: compiled actor instances exist for n_actions 5 and 9 only");
+  std::memset(p->head_w, 0, sizeof(p->head_w)); std::memset(p->head_b, 0, sizeof(p->head_b));
+  pack_embedding(w, p, w->n_actions);
+  std::memcpy(p->head_w, w->head_w, sizeof(float) * 2 * GSM_POLICY_HIDDEN * w->n_actions);
+  std::memcpy(p->head_b, w->head_b, sizeof(float) * w->n_actions);
+  return GSM_OK;
+}
+int pack(const gsm_policy_gauss_weights* w, gsm::GaussParams* p) {
+  if (!w) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_gauss: weights is NULL");
+  if (w->struct_size != sizeof(gsm_policy_gauss_weights))
+    return pfail(GSM_ERR_ABI, "gsm_policy_gauss: weights.struct_size mismatch");
+  static_assert(sizeof(p->log_std) == sizeof(w->log_std), "layout");
+  pack_embedding(w, p, gsm::GD);
+  std::memcpy(p->head_w, w->mean_w, sizeof(w->mean_w));
+  std::memcpy(p->head_b, w->mean_b, sizeof(w->mean_b));
+  std::memcpy(p->log_std, w->log_std, sizeof(p->log_std));
+  return GSM_OK;
+}
+
+// the head rows of the instance that serves a call
+int n_actions(const gsm_policy_weights* w) { return w->n_actions; }
+int n_actions(const gsm_policy_gauss_weights*) { return gsm::GD; }
+int n_actions(const gsm_policy_eval_io* io) { return io->n_actions; }
+int n_actions(const gsm_policy_gauss_eval_io*) { return gsm::GD; }
+
+template <class IO> int check_rows(const IO* io, const char* who) {
+  if (io->n_rows < 0 || io->max_nbrs < 1) return pfailf(GSM_ERR_INVALID_ARG, who, "bad n_rows / max_nbrs");
+  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfailf(GSM_ERR_INVALID_ARG, who, "n_rows too large");
+  return GSM_OK;
+}
+
 // The checks the evaluate and backward entry points of both heads share; none touches the device.
-template <class IO> int check_eval_io_t(const IO* io, const char* who) {
+template <class IO> int check_eval_io(const IO* io, const char* who) {
   if (!io) return pfailf(GSM_ERR_INVALID_ARG, who, "io is NULL");
   if (io->struct_size != sizeof(IO)) return pfailf(GSM_ERR_ABI, who, "io.struct_size mismatch");
   if constexpr (std::is_same_v<IO, gsm_policy_eval_io>) {
@@ -898,32 +1086,14 @@ template <class IO> int check_eval_io_t(const IO* io, const char* who) {
   }
   if (!io->params || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
     return pfailf(GSM_ERR_INVALID_ARG, who, "params, obs, nbr_feat, nbr_cnt and actions are required");
-  if (io->n_rows < 0 || io->max_nbrs < 1) return pfailf(GSM_ERR_INVALID_ARG, who, "bad n_rows / max_nbrs");
-  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfailf(GSM_ERR_INVALID_ARG, who, "n_rows too large");
-  return GSM_OK;
+  return check_rows(io, who);
 }
-int check_eval_io(const gsm_policy_eval_io* io, const char* who) { return check_eval_io_t(io, who); }
 template <int KIND, class IO> gsm::EvalArgs<KIND> eval_args(const IO* io) {
   gsm::EvalArgs<KIND> a{};
   a.params = io->params; a.obs = io->obs; a.nbr_feat = io->nbr_feat; a.nbr_cnt = io->nbr_cnt;
   a.actions = io->actions; a.rows = io->rows;
   a.n_rows = io->n_rows; a.K = io->max_nbrs;
   return a;
-}
-int pack_gauss(const gsm_policy_gauss_weights* w, gsm::GaussParams* p) {
-  if (!w) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_gauss: weights is NULL");
-  if (w->struct_size != sizeof(gsm_policy_gauss_weights))
-    return pfail(GSM_ERR_ABI, "gsm_policy_gauss: weights.struct_size mismatch");
-  static_assert(sizeof(p->ego_w) == sizeof(w->ego_w) && sizeof(p->log_std) == sizeof(w->log_std), "layout");
-  std::memcpy(p->ego_w, w->ego_w, sizeof(p->ego_w));   std::memcpy(p->ego_b, w->ego_b, sizeof(p->ego_b));
-  std::memcpy(p->nbr_w, w->nbr_w, sizeof(p->nbr_w));   std::memcpy(p->nbr_b, w->nbr_b, sizeof(p->nbr_b));
-  std::memcpy(p->att_w, w->att_w, sizeof(p->att_w));   p->att_b = w->att_b;
-  std::memcpy(p->head_w, w->mean_w, sizeof(w->mean_w));                        // means, then the critics
-  std::memcpy(p->head_w[GSM_POLICY_GAUSS_DIM], w->value_w, sizeof(w->value_w));
-  std::memcpy(p->head_b, w->mean_b, sizeof(w->mean_b));
-  std::memcpy(&p->head_b[GSM_POLICY_GAUSS_DIM], w->value_b, sizeof(w->value_b));
-  std::memcpy(p->log_std, w->log_std, sizeof(p->log_std));
-  return GSM_OK;
 }
 int check_loss_io(const gsm_ppo_loss_io* l, const char* who) {
   if (!l) return pfailf(GSM_ERR_INVALID_ARG, who, "loss is NULL");
@@ -936,195 +1106,139 @@ int check_loss_io(const gsm_ppo_loss_io* l, const char* who) {
     return pfailf(GSM_ERR_INVALID_ARG, who, "value_coef and entropy_coef must be >= 0");
   return GSM_OK;
 }
-template <int KIND> void set_loss(gsm::PpoArgs<KIND>& a, const gsm_ppo_loss_io* l) {
-  a.old_logp = l->old_logp; a.old_values = l->old_values; a.returns = l->returns; a.adv = l->advantages;
-  a.adv_moments = l->adv_moments; a.lagrange = l->lagrange;
-  a.clip = l->clip; a.value_clip = l->value_clip; a.value_coef = l->value_coef; a.entropy_coef = l->entropy_coef;
+
+template <int KIND, class W, class IO> int act_t(const W* w, const IO* io, int device, void* stream, const char* who) {
+  typename gsm::Head<KIND>::Params p;
+  if (const int st = pack(w, &p)) return st;
+  if (!io || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
+    return pfailf(GSM_ERR_INVALID_ARG, who, "obs, nbr_feat, nbr_cnt and actions are required");
+  if (const int st = check_rows(io, who)) return st;
+  gsm::ActorIO<KIND> k;
+  k.obs = io->obs; k.nbr_feat = io->nbr_feat; k.nbr_cnt = io->nbr_cnt;
+  k.actions = io->actions; k.logp = io->logp; k.values = io->values;
+  if constexpr (KIND == gsm::HEAD_CAT) k.dist = io->logits; else k.dist = io->mean;
+  k.n_rows = io->n_rows; k.row_offset = io->row_offset; k.seed = io->seed; k.step = io->step;
+  k.K = io->max_nbrs; k.greedy = io->greedy;
+  return on_device(device, who, [&] { return gsm::launch_actor<KIND>(p, k, n_actions(w), (cudaStream_t)stream); });
 }
-// the argument checks and the launch of both heads; need: the workspace bytes for io->n_rows
-template <int KIND, class IO, class Launch>
-int ppo_backward_t(const IO* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace, size_t workspace_bytes,
-                   int device, void* stream, const char* who, int64_t (*need_fn)(const IO*), Launch launch) {
-  if (const int st = check_eval_io_t(io, who)) return st;
-  if (const int st = check_loss_io(loss, who)) return st;
-  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
-  const int64_t need = need_fn(io);
-  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
-    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than the ppo backward workspace for n_rows");
+
+template <int KIND, class IO> int evaluate_t(const IO* io, int device, void* stream, const char* who) {
+  if (const int st = check_eval_io(io, who)) return st;
   if (io->n_rows == 0) return GSM_OK;
-  if (const int ds = check_device(device, who)) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
-  gsm::PpoArgs<KIND> a{};
+  gsm::EvalArgs<KIND> a = eval_args<KIND>(io);
+  a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
+  return on_device(device, who, [&] { return gsm::launch_evaluate<KIND>(a, n_actions(io), (cudaStream_t)stream); });
+}
+
+// the *_workspace entry points; n_actions is checked for the categorical head only (the Gaussian passes GD)
+template <int KIND, bool LOSS> int64_t workspace_t(int64_t n_rows, int n_actions, const char* who) {
+  if (KIND == gsm::HEAD_CAT && n_actions != 5 && n_actions != 9)
+    return pfailf(GSM_ERR_UNSUPPORTED, who, "n_actions must be 5 or 9");
+  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, who, "n_rows < 0");
+  return gsm::for_na<KIND>(n_actions, [&](auto na) {   // per block: its partial gradient (then its statistics)
+    constexpr int WS = gsm::PV<decltype(na)::value, KIND>::N + (LOSS ? gsm::PPO_WS_STATS : 0);
+    return gsm::bwd_blocks(n_rows) * WS * (int64_t)sizeof(float);
+  });
+}
+
+// gsm_policy_backward(_gauss) (LOSS = false: d_logp, d_entropy and d_values are the seeds) and
+// gsm_ppo_backward(_gauss) (LOSS: `loss` computes the seeds); ws_msg: the error for a short workspace
+template <int KIND, bool LOSS, class IO>
+int backward_t(const IO* io, const gsm_ppo_loss_io* loss, const float* d_logp, const float* d_entropy,
+               const float* d_values, float* grad, void* workspace, size_t workspace_bytes, int device, void* stream,
+               const char* who, const char* ws_msg) {
+  if (const int st = check_eval_io(io, who)) return st;
+  if constexpr (LOSS) { if (const int st = check_loss_io(loss, who)) return st; }
+  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
+  const int64_t need = workspace_t<KIND, LOSS>(io->n_rows, n_actions(io), who);
+  if (need > 0 && (!workspace || workspace_bytes < (size_t)need)) return pfailf(GSM_ERR_INVALID_ARG, who, ws_msg);
+  if (io->n_rows == 0) return GSM_OK;
+  gsm::BwdArgs<KIND, LOSS> a{};
   static_cast<gsm::EvalArgs<KIND>&>(a) = eval_args<KIND>(io);
-  set_loss(a, loss);
+  float* stats = nullptr;
+  if constexpr (LOSS) {
+    a.old_logp = loss->old_logp; a.old_values = loss->old_values; a.returns = loss->returns; a.adv = loss->advantages;
+    a.adv_moments = loss->adv_moments; a.lagrange = loss->lagrange;
+    a.clip = loss->clip; a.value_clip = loss->value_clip;
+    a.value_coef = loss->value_coef; a.entropy_coef = loss->entropy_coef;
+    stats = loss->stats;
+  } else {
+    a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
+  }
   a.ws = (float*)workspace;
-  const int e = launch(a, grad, loss->stats, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
+  return on_device(device, who, [&] {
+    return gsm::for_na<KIND>(n_actions(io), [&](auto na) {
+      return gsm::launch_backward<decltype(na)::value, KIND, LOSS>(a, grad, stats, (cudaStream_t)stream);
+    });
+  });
 }
 }  // namespace
 
 extern "C" {
 
+const char* gsm_policy_last_error(void) { return g_policy_err; }
+
+int gsm_policy_act(const gsm_policy_weights* w, const gsm_policy_io* io, int device, void* stream) {
+  return act_t<gsm::HEAD_CAT>(w, io, device, stream, "gsm_policy_act");
+}
+
+int gsm_policy_act_gauss(const gsm_policy_gauss_weights* w, const gsm_policy_gauss_io* io, int device,
+                         void* stream) {
+  return act_t<gsm::HEAD_GAUSS>(w, io, device, stream, "gsm_policy_act_gauss");
+}
+
 int gsm_policy_evaluate(const gsm_policy_eval_io* io, int device, void* stream) {
-  if (const int st = check_eval_io(io, "gsm_policy_evaluate")) return st;
-  if (io->n_rows == 0) return GSM_OK;
-  if (const int ds = check_device(device, "gsm_policy_evaluate")) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_evaluate: cudaSetDevice failed");
-  gsm::EvalArgs<gsm::HEAD_CAT> a = eval_args<gsm::HEAD_CAT>(io);
-  a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
-  const int e = gsm::launch_evaluate(a, io->n_actions, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
+  return evaluate_t<gsm::HEAD_CAT>(io, device, stream, "gsm_policy_evaluate");
+}
+
+int gsm_policy_evaluate_gauss(const gsm_policy_gauss_eval_io* io, int device, void* stream) {
+  return evaluate_t<gsm::HEAD_GAUSS>(io, device, stream, "gsm_policy_evaluate_gauss");
 }
 
 int64_t gsm_policy_backward_workspace(int64_t n_rows, int32_t n_actions) {
-  if (n_actions != 5 && n_actions != 9)
-    return pfailf(GSM_ERR_UNSUPPORTED, "gsm_policy_backward_workspace", "n_actions must be 5 or 9");
-  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_policy_backward_workspace", "n_rows < 0");
-  return gsm::bwd_blocks(n_rows) * gsm::n_params(n_actions) * (int64_t)sizeof(float);
+  return workspace_t<gsm::HEAD_CAT, false>(n_rows, n_actions, "gsm_policy_backward_workspace");
+}
+
+int64_t gsm_policy_backward_workspace_gauss(int64_t n_rows) {
+  return workspace_t<gsm::HEAD_GAUSS, false>(n_rows, gsm::GD, "gsm_policy_backward_workspace_gauss");
 }
 
 int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const float* d_entropy,
                         const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                         int device, void* stream) {
-  const char* who = "gsm_policy_backward";
-  if (const int st = check_eval_io(io, who)) return st;
-  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
-  const int64_t need = gsm_policy_backward_workspace(io->n_rows, io->n_actions);
-  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
-    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than gsm_policy_backward_workspace(n_rows, n_actions)");
-  if (io->n_rows == 0) return GSM_OK;
-  if (const int ds = check_device(device, who)) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_backward: cudaSetDevice failed");
-  gsm::EvalArgs<gsm::HEAD_CAT> a = eval_args<gsm::HEAD_CAT>(io);
-  a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
-  a.ws = (float*)workspace;
-  const int e = io->n_actions == 5 ? gsm::launch_backward_na<5, gsm::HEAD_CAT>(a, grad, (cudaStream_t)stream)
-                                   : gsm::launch_backward_na<9, gsm::HEAD_CAT>(a, grad, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
-}
-
-const char* gsm_policy_last_error(void) { return g_policy_err; }
-
-int gsm_policy_act(const gsm_policy_weights* w, const gsm_policy_io* io, int device, void* stream) {
-  gsm::PolicyParams p;
-  int st = pack(w, &p);
-  if (st) return st;
-  if (!io || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
-    return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act: obs, nbr_feat, nbr_cnt and actions are required");
-  if (io->n_rows < 0 || io->max_nbrs < 1) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act: bad n_rows / max_nbrs");
-  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act: n_rows too large");
-  if (const int ds = check_device(device, "gsm_policy_act")) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_act: cudaSetDevice failed");
-  gsm::PolicyIO k;
-  k.obs = io->obs; k.nbr_feat = io->nbr_feat; k.nbr_cnt = io->nbr_cnt;
-  k.actions = io->actions; k.logp = io->logp; k.dist = io->logits; k.values = io->values;
-  k.n_rows = io->n_rows; k.row_offset = io->row_offset; k.seed = io->seed; k.step = io->step;
-  k.K = io->max_nbrs; k.greedy = io->greedy;
-  const int e = gsm::launch_actor(p, k, w->n_actions, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
-}
-
-int gsm_policy_act_gauss(const gsm_policy_gauss_weights* w, const gsm_policy_gauss_io* io, int device,
-                         void* stream) {
-  gsm::GaussParams p;
-  int st = pack_gauss(w, &p);
-  if (st) return st;
-  if (!io || !io->obs || !io->nbr_feat || !io->nbr_cnt || !io->actions)
-    return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: obs, nbr_feat, nbr_cnt and actions are required");
-  if (io->n_rows < 0 || io->max_nbrs < 1) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: bad n_rows / max_nbrs");
-  if (io->n_rows > ((int64_t)1 << 31) * 128 - 128) return pfail(GSM_ERR_INVALID_ARG, "gsm_policy_act_gauss: n_rows too large");
-  if (const int ds = check_device(device, "gsm_policy_act_gauss")) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_act_gauss: cudaSetDevice failed");
-  gsm::GaussIO k;
-  k.obs = io->obs; k.nbr_feat = io->nbr_feat; k.nbr_cnt = io->nbr_cnt;
-  k.actions = io->actions; k.logp = io->logp; k.dist = io->mean; k.values = io->values;
-  k.n_rows = io->n_rows; k.row_offset = io->row_offset; k.seed = io->seed; k.step = io->step;
-  k.K = io->max_nbrs; k.greedy = io->greedy;
-  const int e = gsm::launch_actor_gauss(p, k, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
-}
-
-int gsm_policy_evaluate_gauss(const gsm_policy_gauss_eval_io* io, int device, void* stream) {
-  const char* who = "gsm_policy_evaluate_gauss";
-  if (const int st = check_eval_io_t(io, who)) return st;
-  if (io->n_rows == 0) return GSM_OK;
-  if (const int ds = check_device(device, who)) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_evaluate_gauss: cudaSetDevice failed");
-  gsm::EvalArgs<gsm::HEAD_GAUSS> a = eval_args<gsm::HEAD_GAUSS>(io);
-  a.logp = io->logp; a.entropy = io->entropy; a.values = io->values;
-  const int e = gsm::launch_evaluate_gauss(a, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
-}
-
-int64_t gsm_policy_backward_workspace_gauss(int64_t n_rows) {
-  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_policy_backward_workspace_gauss", "n_rows < 0");
-  return gsm::bwd_blocks(n_rows) * GSM_POLICY_GAUSS_N_PARAMS * (int64_t)sizeof(float);
+  return backward_t<gsm::HEAD_CAT, false>(io, nullptr, d_logp, d_entropy, d_values, grad, workspace, workspace_bytes,
+                                          device, stream, "gsm_policy_backward",
+                                          "workspace smaller than gsm_policy_backward_workspace(n_rows, n_actions)");
 }
 
 int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d_logp, const float* d_entropy,
                               const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                               int device, void* stream) {
-  const char* who = "gsm_policy_backward_gauss";
-  if (const int st = check_eval_io_t(io, who)) return st;
-  if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
-  const int64_t need = gsm_policy_backward_workspace_gauss(io->n_rows);
-  if (need > 0 && (!workspace || workspace_bytes < (size_t)need))
-    return pfailf(GSM_ERR_INVALID_ARG, who, "workspace smaller than gsm_policy_backward_workspace_gauss(n_rows)");
-  if (io->n_rows == 0) return GSM_OK;
-  if (const int ds = check_device(device, who)) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_policy_backward_gauss: cudaSetDevice failed");
-  gsm::EvalArgs<gsm::HEAD_GAUSS> a = eval_args<gsm::HEAD_GAUSS>(io);
-  a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
-  a.ws = (float*)workspace;
-  const int e = gsm::launch_backward_na<gsm::GD, gsm::HEAD_GAUSS>(a, grad, (cudaStream_t)stream);
-  if (e) return pfail(GSM_ERR_CUDA, cudaGetErrorString((cudaError_t)e));
-  return GSM_OK;
+  return backward_t<gsm::HEAD_GAUSS, false>(io, nullptr, d_logp, d_entropy, d_values, grad, workspace,
+                                            workspace_bytes, device, stream, "gsm_policy_backward_gauss",
+                                            "workspace smaller than gsm_policy_backward_workspace_gauss(n_rows)");
 }
 
 int64_t gsm_ppo_backward_workspace(int64_t n_rows, int32_t n_actions) {
-  if (n_actions != 5 && n_actions != 9)
-    return pfailf(GSM_ERR_UNSUPPORTED, "gsm_ppo_backward_workspace", "n_actions must be 5 or 9");
-  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_ppo_backward_workspace", "n_rows < 0");
-  return gsm::bwd_blocks(n_rows) * (gsm::n_params(n_actions) + gsm::PPO_WS_STATS) * (int64_t)sizeof(float);
+  return workspace_t<gsm::HEAD_CAT, true>(n_rows, n_actions, "gsm_ppo_backward_workspace");
 }
 
 int64_t gsm_ppo_backward_workspace_gauss(int64_t n_rows) {
-  if (n_rows < 0) return pfailf(GSM_ERR_INVALID_ARG, "gsm_ppo_backward_workspace_gauss", "n_rows < 0");
-  return gsm::bwd_blocks(n_rows) * (GSM_POLICY_GAUSS_N_PARAMS + gsm::PPO_WS_STATS) * (int64_t)sizeof(float);
+  return workspace_t<gsm::HEAD_GAUSS, true>(n_rows, gsm::GD, "gsm_ppo_backward_workspace_gauss");
 }
 
 int gsm_ppo_backward(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace,
                      size_t workspace_bytes, int device, void* stream) {
-  return ppo_backward_t<gsm::HEAD_CAT>(
-      io, loss, grad, workspace, workspace_bytes, device, stream, "gsm_ppo_backward",
-      +[](const gsm_policy_eval_io* q) { return gsm_ppo_backward_workspace(q->n_rows, q->n_actions); },
-      [&](const gsm::PpoArgs<gsm::HEAD_CAT>& a, float* g, float* st, cudaStream_t s) {
-        return io->n_actions == 5 ? gsm::launch_ppo_na<5, gsm::HEAD_CAT>(a, g, st, s)
-                                  : gsm::launch_ppo_na<9, gsm::HEAD_CAT>(a, g, st, s);
-      });
+  return backward_t<gsm::HEAD_CAT, true>(io, loss, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes, device,
+                                         stream, "gsm_ppo_backward",
+                                         "workspace smaller than the ppo backward workspace for n_rows");
 }
 
 int gsm_ppo_backward_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss, float* grad,
                            void* workspace, size_t workspace_bytes, int device, void* stream) {
-  return ppo_backward_t<gsm::HEAD_GAUSS>(
-      io, loss, grad, workspace, workspace_bytes, device, stream, "gsm_ppo_backward_gauss",
-      +[](const gsm_policy_gauss_eval_io* q) { return gsm_ppo_backward_workspace_gauss(q->n_rows); },
-      [](const gsm::PpoArgs<gsm::HEAD_GAUSS>& a, float* g, float* st, cudaStream_t s) {
-        return gsm::launch_ppo_na<gsm::GD, gsm::HEAD_GAUSS>(a, g, st, s);
-      });
+  return backward_t<gsm::HEAD_GAUSS, true>(io, loss, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes,
+                                           device, stream, "gsm_ppo_backward_gauss",
+                                           "workspace smaller than the ppo backward workspace for n_rows");
 }
 
 int gsm_adam_step(float* params, const float* grad, float* m, float* v, int32_t* step, int64_t n, float lr,
@@ -1138,14 +1252,11 @@ int gsm_adam_step(float* params, const float* grad, float* m, float* v, int32_t*
     return pfailf(GSM_ERR_INVALID_ARG, who, "beta1 and beta2 must lie in [0, 1)");
   if (!(lr >= 0.f) || !(eps >= 0.f) || !(max_grad_norm > 0.f))
     return pfailf(GSM_ERR_INVALID_ARG, who, "lr and eps must be >= 0 and max_grad_norm > 0");
-  if (const int ds = check_device(device, who)) return ds;
-  DevGuard guard(device);
-  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
   const gsm::AdamArgs a{params, grad, m, v, step, grad_norm, n, lr, beta1, beta2, eps, max_grad_norm};
-  gsm::adam_step_kernel<<<1, gsm::ADAM_THREADS, 0, (cudaStream_t)stream>>>(a);
-  const cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return pfail(GSM_ERR_CUDA, cudaGetErrorString(e));
-  return GSM_OK;
+  return on_device(device, who, [&] {
+    gsm::adam_step_kernel<<<1, gsm::ADAM_THREADS, 0, (cudaStream_t)stream>>>(a);
+    return (int)cudaGetLastError();
+  });
 }
 
 int gsm_gae(const float* reward, const float* cost, const float* values, const uint8_t* done, int32_t n_steps,

@@ -26,7 +26,7 @@ import ctypes as C
 import torch
 
 from . import abi
-from .policy import GaussianGraphActor, GraphAttentionActor, _check, _eval_io, _CAT_LEARNER, _GAUSS_LEARNER
+from .policy import GaussianGraphActor, GraphAttentionActor, _check, _eval_io
 
 # the columns of `update`'s result: the GSM_PPO_STAT_FIELDS loss statistics, then the gradient norm
 STAT_FIELDS = ("policy_loss", "value_loss_reward", "value_loss_cost", "entropy", "ratio", "clip_fraction",
@@ -40,16 +40,10 @@ class LagrangianPPO:
 
     def __init__(self, actor, *, clip, value_clip, value_coef, entropy_coef, lr, betas, eps, max_grad_norm,
                  ppo_epoch, num_mini_batch, lagrangian_lr, cost_limit, lagrangian_init=0.0, seed):
-        if isinstance(actor, GraphAttentionActor):
-            self._head, self._act_tail, self._act_dtype = _CAT_LEARNER[actor.n_actions], (), torch.int32
-            self._backward, self._workspace = "gsm_ppo_backward", lambda lib, n: lib.gsm_ppo_backward_workspace(
-                n, actor.n_actions)
-        elif isinstance(actor, GaussianGraphActor):
-            self._head, self._act_tail, self._act_dtype = _GAUSS_LEARNER, (abi.GSM_POLICY_GAUSS_DIM,), torch.float32
-            self._backward, self._workspace = "gsm_ppo_backward_gauss", lambda lib, n: \
-                lib.gsm_ppo_backward_workspace_gauss(n)
-        else:
+        if not isinstance(actor, (GraphAttentionActor, GaussianGraphActor)):
             raise TypeError("LagrangianPPO trains a GraphAttentionActor or a GaussianGraphActor")
+        self._head = actor._desc
+        self._act_dtype, self._act_tail = self._head.act_dtype, self._head.act_tail
         b1, b2 = (float(b) for b in betas)
         if not (clip > 0 and value_clip > 0):
             raise ValueError("clip and value_clip must be > 0")
@@ -119,7 +113,7 @@ class LagrangianPPO:
         lib = abi.load_library()
         dev = self.device
         n = rows.numel() if rows is not None else x["cnt"].numel()
-        need = self._workspace(lib, n)
+        need = getattr(lib, self._head.ppo_workspace)(n, *self._head.ws_args)
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
         io = _eval_io(self._head, self.params, x["obs"], x["feat"], x["cnt"], x["act"], rows)
@@ -131,8 +125,9 @@ class LagrangianPPO:
                                                        stats.data_ptr())
         loss.clip, loss.value_clip = self.clip, self.value_clip
         loss.value_coef, loss.entropy_coef = self.value_coef, self.entropy_coef
-        _check(lib, getattr(lib, self._backward)(C.byref(io), C.byref(loss), self.grad.data_ptr(), self._ws.data_ptr(),
-                                                 self._ws.numel(), dev.index or 0, self._stream()))
+        _check(lib, getattr(lib, self._head.ppo_backward)(C.byref(io), C.byref(loss), self.grad.data_ptr(),
+                                                          self._ws.data_ptr(), self._ws.numel(), dev.index or 0,
+                                                          self._stream()))
 
     def adam_step(self, grad_norm):
         """gsm_adam_step on (self.params, self.grad, self.m, self.v, self.step); grad_norm: a device float [1]."""

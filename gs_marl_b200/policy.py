@@ -23,6 +23,7 @@ worlds (SPEC.md §10b / §12b): mean = W_mu h + b_mu, a state-independent log_st
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 
 import numpy as np
 import torch
@@ -44,10 +45,39 @@ def _seeded_linear(g):
     return lin
 
 
+@dataclasses.dataclass(frozen=True)
+class _Head:
+    """The C side of one head, the one place that names it: the entry points, the io structs and the
+    action tensors' dtype and trailing shape.  The workspace functions take n_rows, then ws_args."""
+    act: str
+    act_io: type
+    dist_field: str           # act_io's field for the logits / the means
+    evaluate: str
+    backward: str
+    workspace: str
+    ppo_backward: str
+    ppo_workspace: str
+    ws_args: tuple
+    eval_io: type
+    head_field: str
+    head_value: int           # n_actions or action_dim: also the width of the logits / the means
+    act_dtype: torch.dtype
+    act_tail: tuple
+
+
+_CAT_HEADS = {a: _Head("gsm_policy_act", abi.GsmPolicyIO, "logits", "gsm_policy_evaluate", "gsm_policy_backward",
+                       "gsm_policy_backward_workspace", "gsm_ppo_backward", "gsm_ppo_backward_workspace", (a,),
+                       abi.GsmPolicyEvalIO, "n_actions", a, torch.int32, ()) for a in (5, 9)}
+_GAUSS_HEAD = _Head("gsm_policy_act_gauss", abi.GsmPolicyGaussIO, "mean", "gsm_policy_evaluate_gauss",
+                    "gsm_policy_backward_gauss", "gsm_policy_backward_workspace_gauss", "gsm_ppo_backward_gauss",
+                    "gsm_ppo_backward_workspace_gauss", (), abi.GsmPolicyGaussEvalIO, "action_dim",
+                    abi.GSM_POLICY_GAUSS_DIM, torch.float32, (abi.GSM_POLICY_GAUSS_DIM,))
+
+
 class _GraphEmbedding(torch.nn.Module):
     """What both actors share: the embedding h = [e; sum_r a_r m_r] in plain torch, the packing of its
-    weights and the input checks of the kernel paths.  Subclasses register ego, nbr, att, their head
-    and value, in that order (parameters_to_vector order is the learner's vector layout)."""
+    weights and the kernel paths.  Subclasses register ego, nbr, att, their head and value, in that
+    order (parameters_to_vector order is the learner's vector layout), and set `_desc`, their _Head."""
 
     def _put_embedding(self, w, put):
         put("ego_w", self.ego.weight); put("ego_b", self.ego.bias)
@@ -59,6 +89,52 @@ class _GraphEmbedding(torch.nn.Module):
     def packed(self):
         """The last `pack()` (call `pack()` again after an optimizer step)."""
         return self._packed if self._packed is not None else self.pack()
+
+    @torch.no_grad()
+    def _act(self, obs, graph, seed, step, row_offset, greedy, want_dist, want_values, out):
+        d = self._desc
+        lib = abi.load_library()
+        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
+        lead = _check_act_inputs(obs, feat, cnt)
+        dev = obs.device
+        if out is None:
+            actions = torch.empty(lead + d.act_tail, dtype=d.act_dtype, device=dev)
+            logp = torch.empty(lead, dtype=torch.float32, device=dev)
+        else:
+            actions, logp = out
+        dist = torch.empty(lead + (d.head_value,), dtype=torch.float32, device=dev) if want_dist else None
+        values = (torch.empty(lead + (abi.GSM_POLICY_VALUE_HEADS,), dtype=torch.float32, device=dev)
+                  if want_values else None)
+        io = d.act_io()
+        io.obs, io.nbr_feat, io.nbr_cnt = obs.data_ptr(), feat.data_ptr(), cnt.data_ptr()
+        io.actions, io.logp, io.values = actions.data_ptr(), logp.data_ptr(), _ptr(values)
+        setattr(io, d.dist_field, _ptr(dist))
+        io.n_rows, io.row_offset, io.seed, io.step = cnt.numel(), int(row_offset), int(seed), int(step)
+        io.max_nbrs, io.greedy = int(feat.shape[-2]), int(bool(greedy))
+        _check(lib, getattr(lib, d.act)(C.byref(self.packed()), C.byref(io), dev.index or 0,
+                                        C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        return (actions, logp) + ((dist,) if want_dist else ()) + ((values,) if want_values else ())
+
+    # ---- learner pass: two kernels, differentiable ----------------------------------------------
+    def evaluate_actions(self, obs, graph, actions, rows=None):
+        """log pi(actions), entropy and the two critics, differentiable w.r.t. the parameters.
+
+        obs [..., 6], graph['nbr_feat'] [..., K, 6], graph['nbr_cnt'] [...] and actions (int32 [...]
+        for the categorical head, float32 [..., 2] for the Gaussian; contiguous CUDA tensors on the
+        parameters' device) are the source rows.  rows: optional int64 1-D index into the flattened
+        source rows (a shuffled minibatch read straight out of the rollout buffer, no gather of
+        nbr_feat).  Returns logp [n], entropy [n] and values [n, 2] with n = the source shape, or
+        [len(rows)].  logp and values are bit-identical to what `act` / `collect_fused` wrote for the
+        same rows and actions.  The range check on `rows` synchronises and is skipped while a CUDA
+        graph is being captured."""
+        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
+        params = torch.nn.utils.parameters_to_vector(self.parameters())
+        rows = _check_eval_inputs(params, obs, feat, cnt, actions, rows, self._desc.act_dtype, self._desc.act_tail)
+        return _EvaluateActions.apply(params, obs, feat, cnt, actions, rows, self._desc)
+
+    # ---- the same function in plain torch (reference formulation; not used by the kernels) ----
+    def values_autograd(self, obs, graph):
+        return self.value(self.embed_autograd(obs, graph))
 
     def embed_autograd(self, obs, graph):
         feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
@@ -139,6 +215,7 @@ class GraphAttentionActor(_GraphEmbedding):
         self.head = lin(n_actions, 2 * H)
         self.value = lin(abi.GSM_POLICY_VALUE_HEADS, 2 * H)     # [0] reward critic, [1] cost critic
         self._packed = None
+        self._desc = _CAT_HEADS[n_actions]
 
     # ---- weights -> the C struct (host memory; they ride in the kernel's parameter space) ----
     def pack(self) -> abi.GsmPolicyWeights:
@@ -152,60 +229,16 @@ class GraphAttentionActor(_GraphEmbedding):
         return w
 
     # ---- collect path: one kernel ------------------------------------------------------------
-    @torch.no_grad()
     def act(self, obs, graph, seed: int = 0, step: int = 0, row_offset: int = 0, greedy: bool = False,
             want_logits: bool = False, want_values: bool = False, out=None):
         """obs [..., 6], graph['nbr_feat'] [..., K, 6], graph['nbr_cnt'] [...] (fp32 / int32 CUDA
         tensors, contiguous) -> actions int32 [...], logp fp32 [...], then logits [..., n_actions] if
         want_logits, then values [..., 2] (reward critic, cost critic) if want_values."""
-        lib = abi.load_library()
-        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
-        lead = _check_act_inputs(obs, feat, cnt)
-        n_rows = cnt.numel()
-        dev = obs.device
-        if out is None:
-            actions = torch.empty(lead, dtype=torch.int32, device=dev)
-            logp = torch.empty(lead, dtype=torch.float32, device=dev)
-        else:
-            actions, logp = out
-        logits = torch.empty(lead + (self.n_actions,), dtype=torch.float32, device=dev) if want_logits else None
-        io = abi.GsmPolicyIO()
-        io.obs, io.nbr_feat, io.nbr_cnt = obs.data_ptr(), feat.data_ptr(), cnt.data_ptr()
-        io.actions, io.logp = actions.data_ptr(), logp.data_ptr()
-        io.logits = logits.data_ptr() if want_logits else None
-        values = (torch.empty(lead + (abi.GSM_POLICY_VALUE_HEADS,), dtype=torch.float32, device=dev)
-                  if want_values else None)
-        io.values = values.data_ptr() if want_values else None
-        io.n_rows, io.row_offset, io.seed, io.step = n_rows, int(row_offset), int(seed), int(step)
-        io.max_nbrs, io.greedy = int(feat.shape[-2]), int(bool(greedy))
-        st = lib.gsm_policy_act(C.byref(self.packed()), C.byref(io), dev.index or 0,
-                                C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
-        if st != 0:
-            raise abi.GsmError(f"{lib.gsm_status_string(st).decode()}: {lib.gsm_policy_last_error().decode()}")
-        return (actions, logp) + ((logits,) if want_logits else ()) + ((values,) if want_values else ())
-
-    # ---- learner pass: two kernels, differentiable ----------------------------------------------
-    def evaluate_actions(self, obs, graph, actions, rows=None):
-        """log pi(actions), entropy and the two critics, differentiable w.r.t. the parameters.
-
-        obs [..., 6], graph['nbr_feat'] [..., K, 6], graph['nbr_cnt'] [...] and actions [...]
-        (fp32 / int32 contiguous CUDA tensors on the parameters' device) are the source rows.  rows:
-        optional int64 1-D index into the flattened source rows (a shuffled minibatch read straight
-        out of the rollout buffer, no gather of nbr_feat).  Returns logp [n], entropy [n] and values
-        [n, 2] with n = the source shape, or [len(rows)].  logp and values are bit-identical to what
-        `act` / `collect_fused` wrote for the same rows and actions.  The range check on `rows`
-        synchronises and is skipped while a CUDA graph is being captured."""
-        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
-        params = torch.nn.utils.parameters_to_vector(self.parameters())
-        rows = _check_eval_inputs(params, obs, feat, cnt, actions, rows, torch.int32, ())
-        return _EvaluateActions.apply(params, obs, feat, cnt, actions, rows, _CAT_LEARNER[self.n_actions])
+        return self._act(obs, graph, seed, step, row_offset, greedy, want_logits, want_values, out)
 
     # ---- the same function in plain torch (reference formulation; not used by the kernels) ----
     def logits_autograd(self, obs, graph):
         return self.head(self.embed_autograd(obs, graph))
-
-    def values_autograd(self, obs, graph):
-        return self.value(self.embed_autograd(obs, graph))
 
 
 class _LogStd(torch.nn.Module):
@@ -225,6 +258,7 @@ class GaussianGraphActor(_GraphEmbedding):
     (SPEC.md §10b): ego, nbr, att, head = Linear(2H, 2) (the mean), log_std (initialised to 0), value.
     Actions are float32 [..., 2], not clipped or squashed."""
     action_mode = "continuous"
+    _desc = _GAUSS_HEAD
 
     def __init__(self, seed: int = 0):
         super().__init__()
@@ -246,41 +280,12 @@ class GaussianGraphActor(_GraphEmbedding):
         self._packed = w
         return w
 
-    @torch.no_grad()
     def act(self, obs, graph, seed: int = 0, step: int = 0, row_offset: int = 0, greedy: bool = False,
             want_mean: bool = False, want_values: bool = False, out=None):
         """obs [..., 6], graph['nbr_feat'] [..., K, 6], graph['nbr_cnt'] [...] (fp32 / int32 CUDA
         tensors, contiguous) -> actions float32 [..., 2], logp fp32 [...], then the mean [..., 2] if
         want_mean, then values [..., 2] (reward critic, cost critic) if want_values.  greedy: the mean."""
-        lib = abi.load_library()
-        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
-        lead = _check_act_inputs(obs, feat, cnt)
-        dev = obs.device
-        D = abi.GSM_POLICY_GAUSS_DIM
-        if out is None:
-            actions = torch.empty(lead + (D,), dtype=torch.float32, device=dev)
-            logp = torch.empty(lead, dtype=torch.float32, device=dev)
-        else:
-            actions, logp = out
-        mean = torch.empty(lead + (D,), dtype=torch.float32, device=dev) if want_mean else None
-        values = (torch.empty(lead + (abi.GSM_POLICY_VALUE_HEADS,), dtype=torch.float32, device=dev)
-                  if want_values else None)
-        io = abi.GsmPolicyGaussIO()
-        io.obs, io.nbr_feat, io.nbr_cnt = obs.data_ptr(), feat.data_ptr(), cnt.data_ptr()
-        io.actions, io.logp, io.mean, io.values = actions.data_ptr(), logp.data_ptr(), _ptr(mean), _ptr(values)
-        io.n_rows, io.row_offset, io.seed, io.step = cnt.numel(), int(row_offset), int(seed), int(step)
-        io.max_nbrs, io.greedy = int(feat.shape[-2]), int(bool(greedy))
-        _check(lib, lib.gsm_policy_act_gauss(C.byref(self.packed()), C.byref(io), dev.index or 0,
-                                             C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
-        return (actions, logp) + ((mean,) if want_mean else ()) + ((values,) if want_values else ())
-
-    def evaluate_actions(self, obs, graph, actions, rows=None):
-        """log pi(actions), entropy and the two critics, differentiable w.r.t. the parameters, as
-        `GraphAttentionActor.evaluate_actions` with float32 actions [..., 2]."""
-        feat, cnt = graph["nbr_feat"], graph["nbr_cnt"]
-        params = torch.nn.utils.parameters_to_vector(self.parameters())
-        rows = _check_eval_inputs(params, obs, feat, cnt, actions, rows, torch.float32, (abi.GSM_POLICY_GAUSS_DIM,))
-        return _EvaluateActions.apply(params, obs, feat, cnt, actions, rows, _GAUSS_LEARNER)
+        return self._act(obs, graph, seed, step, row_offset, greedy, want_mean, want_values, out)
 
     # ---- the same function in plain torch (reference formulation; not used by the kernels) ----
     def dist_autograd(self, obs, graph):
@@ -288,28 +293,10 @@ class GaussianGraphActor(_GraphEmbedding):
         mean = self.head(self.embed_autograd(obs, graph))
         return torch.distributions.Normal(mean, self.log_std().exp().expand_as(mean))
 
-    def values_autograd(self, obs, graph):
-        return self.value(self.embed_autograd(obs, graph))
-
-
-class _Learner:
-    """The learner entry points of one head: the eval-io struct and its head field, the C functions."""
-
-    def __init__(self, io_cls, head_field, head_value, evaluate, backward, workspace):
-        self.io_cls, self.head_field, self.head_value = io_cls, head_field, head_value
-        self.evaluate, self.backward, self.workspace = evaluate, backward, workspace
-
-
-_CAT_LEARNER = {a: _Learner(abi.GsmPolicyEvalIO, "n_actions", a, "gsm_policy_evaluate", "gsm_policy_backward",
-                            lambda lib, n, a=a: lib.gsm_policy_backward_workspace(n, a)) for a in (5, 9)}
-_GAUSS_LEARNER = _Learner(abi.GsmPolicyGaussEvalIO, "action_dim", abi.GSM_POLICY_GAUSS_DIM,
-                          "gsm_policy_evaluate_gauss", "gsm_policy_backward_gauss",
-                          lambda lib, n: lib.gsm_policy_backward_workspace_gauss(n))
-
 
 def _eval_io(head, params, obs, feat, cnt, actions, rows):
-    io = head.io_cls()
-    io.struct_size = C.sizeof(head.io_cls)
+    io = head.eval_io()
+    io.struct_size = C.sizeof(head.eval_io)
     setattr(io, head.head_field, head.head_value)
     io.params, io.obs, io.nbr_feat = params.data_ptr(), obs.data_ptr(), feat.data_ptr()
     io.nbr_cnt, io.actions = cnt.data_ptr(), actions.data_ptr()
@@ -354,7 +341,7 @@ class _EvaluateActions(torch.autograd.Function):
         if not io.n_rows:
             return torch.zeros_like(params), None, None, None, None, None, None
         grad = torch.empty_like(params)
-        ws = torch.empty(ctx.head.workspace(lib, io.n_rows), dtype=torch.uint8, device=dev)
+        ws = torch.empty(getattr(lib, ctx.head.workspace)(io.n_rows, *ctx.head.ws_args), dtype=torch.uint8, device=dev)
         d = [g.contiguous() if g is not None else None for g in (d_logp, d_entropy, d_values)]
         _check(lib, getattr(lib, ctx.head.backward)(C.byref(io), _ptr(d[0]), _ptr(d[1]), _ptr(d[2]), grad.data_ptr(),
                                             ws.data_ptr(), ws.numel(), dev.index or 0,

@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE — fp64 numpy restatement of the PPO-Lagrangian loss (SPEC.md §14) that
-gs_marl_b200/csrc/gsm_policy.cu fuses into ppo_backward_kernel: the seeds d_logp, d_entropy, d_values the loss
+gs_marl_b200/csrc/gsm_policy.cu fuses into backward_kernel<NA, KIND, true>: the seeds d_logp, d_entropy, d_values the loss
 passes into the §12 chain, the loss statistics, and the gradient through tests/_learner_oracle.py or
 tests/_gauss_oracle.py `evaluate_backward`.  numpy only; pinned to torch autograd of the §14 formula by
 tests/test_ppo_update.py.
