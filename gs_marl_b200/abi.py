@@ -8,7 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-GSM_ABI_VERSION = 7
+GSM_ABI_VERSION = 8
 GSM_OBS_DIM = 6
 GSM_NBR_FEAT_DIM = 6
 GSM_MAX_DISCRETE = 16
@@ -160,6 +160,16 @@ class GsmPpoLossIO(C.Structure):
     ]
 
 
+class GsmValueNormIO(C.Structure):
+    """gsm_value_norm_io: one epoch of value-normaliser updates (SPEC.md §15); DEVICE pointers."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("reserved", C.c_int32),
+        ("state", C.c_void_p), ("affine", C.c_void_p), ("returns", C.c_void_p), ("rows", C.c_void_p),
+        ("mb", C.c_int64), ("n_mini_batch", C.c_int64),
+        ("beta", C.c_double), ("epsilon", C.c_double), ("var_floor", C.c_double),
+    ]
+
+
 def policy_n_params(n_actions: int) -> int:
     """GSM_POLICY_N_PARAMS: length of the learner's parameter vector."""
     return 961 + 129 * n_actions + 2 * (2 * GSM_POLICY_HIDDEN + 1)
@@ -222,6 +232,16 @@ SYMBOLS = {
                                          C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gsm_adam_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
                                 C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_int, C.c_void_p]),
+    "gsm_gae_normalized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64,
+                                     C.c_int64, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                     C.c_void_p]),
+    "gsm_ppo_backward_normalized": (C.c_int, [C.POINTER(GsmPolicyEvalIO), C.POINTER(GsmPpoLossIO), C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gsm_ppo_backward_normalized_gauss": (C.c_int, [C.POINTER(GsmPolicyGaussEvalIO), C.POINTER(GsmPpoLossIO),
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int,
+                                                    C.c_void_p]),
+    "gsm_value_norm_update_workspace": (C.c_int64, [C.c_int64, C.c_int64]),
+    "gsm_value_norm_update": (C.c_int, [C.POINTER(GsmValueNormIO), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gsm_episode_stats_workspace": (C.c_int64, [C.c_int64, C.c_int32]),
     "gsm_episode_stats": (C.c_int, [C.POINTER(GsmEpisodeIO), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
 }

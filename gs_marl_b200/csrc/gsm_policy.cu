@@ -359,19 +359,30 @@ struct GaeParams {
   int T;
   float gamma, lam;
 };
-__global__ void __launch_bounds__(256) gae_kernel(const __grid_constant__ GaeParams p) {
+// NORM (SPEC.md §15, gsm_gae_normalized): the critics' values are normalised; every V_h[t] is denormalised
+// as fmaf(V, sigma_h, mu_h) with the [2][2] affine (mu_h, sigma_h) before the recursion.
+struct GaeNormParams : GaeParams {
+  const float* affine;
+};
+template <bool NORM> using GaeArgs = std::conditional_t<NORM, GaeNormParams, GaeParams>;
+template <bool NORM>
+__global__ void __launch_bounds__(256) gae_kernel(const __grid_constant__ GaeArgs<NORM> p) {
   constexpr int V = GSM_POLICY_VALUE_HEADS;
   const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= p.n_rows * V) return;
   const int64_t row = g / V;
   const int head = (int)(g - row * V);
   const float* rw = head == 0 ? p.reward : p.cost;
+  float mu = 0.f, sd = 1.f;
+  if constexpr (NORM) { mu = p.affine[2 * head]; sd = p.affine[2 * head + 1]; }
   float gae = 0.f;
   float v_next = p.values[((int64_t)p.T * p.slot_rows + row) * V + head];
+  if constexpr (NORM) v_next = fmaf(v_next, sd, mu);
   for (int t = p.T - 1; t >= 0; t--) {
     const int64_t o = (int64_t)t * p.slot_rows + row;
     const float mask = p.done[o] ? 0.f : 1.f;      // done at step t: slot t+1 starts a new episode
-    const float v = p.values[o * V + head];
+    float v = p.values[o * V + head];
+    if constexpr (NORM) v = fmaf(v, sd, mu);
     const float delta = rw[o] + p.gamma * v_next * mask - v;
     gae = delta + p.gamma * p.lam * mask * gae;
     if (p.adv) p.adv[o * V + head] = gae;
@@ -591,17 +602,29 @@ template <int KIND> struct PpoArgs : EvalArgs<KIND> {
   const float* adv_moments; const float* lagrange;                                          // device scalars
   float clip, value_clip, value_coef, entropy_coef, inv_n;
 };
+// SPEC.md §15 (gsm_ppo_backward_normalized): the minibatch's value-normaliser affine [2][2] (mu_h, sigma_h)
+template <int KIND> struct PpoNormArgs : PpoArgs<KIND> {
+  const float* value_affine;
+};
 template <class Base> struct PpoSmem : Base {
   float st[BWD_AG][PPO_ROW_STATS];     // the tile's per-row statistics
   float stacc[PPO_ROW_STATS];          // the block's sums over its tiles (thread k owns entry k)
 };
 
+// backward_kernel's LOSS modes: the seeds are inputs (gsm_policy_backward); the §14 loss computes them
+// (gsm_ppo_backward); the §14 loss on normalised value targets, R_h -> (R_h - mu_h) / sigma_h (§15,
+// gsm_ppo_backward_normalized)
+constexpr int LOSS_NONE = 0, LOSS_PPO = 1, LOSS_PPO_VNORM = 2;
+template <int KIND, int LOSS>
+using BwdArgs = std::conditional_t<LOSS == LOSS_NONE, EvalArgs<KIND>,
+                                   std::conditional_t<LOSS == LOSS_PPO, PpoArgs<KIND>, PpoNormArgs<KIND>>>;
+
 // SPEC.md §14 for one row: the seeds d_logp, d_entropy, d_values of the §12 chain and the row's statistics.
 // A comparison with a NaN operand is false, so a NaN log-prob (an action outside the head's range)
 // reaches d_logp and poisons the gradient, as in gsm_policy_backward.
-template <int KIND>
-__device__ __forceinline__ void ppo_seeds(const PpoArgs<KIND>& p, int64_t src, float lp, float ent, const float* v,
-                                          float& dlp, float& dent, float (&dv)[V2], float* st) {
+template <int KIND, int LOSS>
+__device__ __forceinline__ void ppo_seeds(const BwdArgs<KIND, LOSS>& p, int64_t src, float lp, float ent,
+                                          const float* v, float& dlp, float& dent, float (&dv)[V2], float* st) {
   const float* mom = p.adv_moments;
   const float a0 = (p.adv[src * V2] - mom[0]) / (mom[1] + 1e-5f);
   const float a1 = (p.adv[src * V2 + 1] - mom[2]) / (mom[3] + 1e-5f);
@@ -613,7 +636,9 @@ __device__ __forceinline__ void ppo_seeds(const PpoArgs<KIND>& p, int64_t src, f
   st[0] = -(s2 < s1 ? s2 : s1);
 #pragma unroll
   for (int h = 0; h < V2; h++) {
-    const float ov = p.old_values[src * V2 + h], R = p.returns[src * V2 + h];
+    const float ov = p.old_values[src * V2 + h];
+    float R = p.returns[src * V2 + h];
+    if constexpr (LOSS == LOSS_PPO_VNORM) R = (R - p.value_affine[2 * h]) / p.value_affine[2 * h + 1];
     const float dov = v[h] - ov;
     const float vc = ov + fminf(fmaxf(dov, -p.value_clip), p.value_clip);
     const float e1 = v[h] - R, e2 = vc - R, q1 = e1 * e1, q2 = e2 * e2;
@@ -626,20 +651,25 @@ __device__ __forceinline__ void ppo_seeds(const PpoArgs<KIND>& p, int64_t src, f
   st[3] = ent; st[4] = rho; st[5] = fabsf(rho - 1.f) > p.clip ? 1.f : 0.f; st[6] = olp - lp;
 }
 
-// The backward kernel.  LOSS = false (gsm_policy_backward): the seeds d_logp, d_entropy, d_values are
-// inputs.  LOSS = true (gsm_ppo_backward): phase A computes them from the PPO-Lagrangian loss (ppo_seeds,
-// SPEC.md §14) and the block also sums the loss statistics.  The loss mode adds code only under
-// `if constexpr (LOSS)`, so the LOSS = false instances carry none of it.  (A __forceinline__ device function
+// The backward kernel.  LOSS_NONE (gsm_policy_backward): the seeds d_logp, d_entropy, d_values are
+// inputs.  LOSS_PPO (gsm_ppo_backward): phase A computes them from the PPO-Lagrangian loss (ppo_seeds,
+// SPEC.md §14) and the block also sums the loss statistics; LOSS_PPO_VNORM normalises the value targets
+// first.  The loss modes add code only under `if constexpr`, so the LOSS_NONE instances carry none of it.  (A __forceinline__ device function
 // shared by two thin kernels would not do: the inliner changes the optimisation pipeline and the SASS of
 // every instance.)
-template <int KIND, bool LOSS> using BwdArgs = std::conditional_t<LOSS, PpoArgs<KIND>, EvalArgs<KIND>>;
-template <int NA, int KIND, bool LOSS>
-using BwdSmemT = std::conditional_t<LOSS, PpoSmem<BwdSmemOf<NA, KIND>>, BwdSmemOf<NA, KIND>>;
+template <int NA, int KIND, int LOSS>
+using BwdSmemT = std::conditional_t<LOSS != LOSS_NONE, PpoSmem<BwdSmemOf<NA, KIND>>, BwdSmemOf<NA, KIND>>;
 
-template <int NA, int KIND, bool LOSS>
-__global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant__ BwdArgs<KIND, LOSS> p) {
+// The normalised <9, CAT> instance names a minimum of one block per SM: left to its own occupancy target,
+// ptxas caps it at 168 registers and spills one value.  A bound of 0 is no bound: every other instance
+// compiles as it does without one (the bound on <5, CAT> and <2, GAUSS> would raise their registers and cost
+// occupancy).
+template <int NA, int KIND, int LOSS>
+__global__ void __launch_bounds__(BWD_AG, LOSS == LOSS_PPO_VNORM && NA == 9 ? 1 : 0)
+    backward_kernel(const __grid_constant__ BwdArgs<KIND, LOSS> p) {
   using P = PV<NA, KIND>;
-  constexpr int NZ = NA + V2, NP = P::N, WS = NP + (LOSS ? PPO_WS_STATS : 0);
+  constexpr bool PPO = LOSS != LOSS_NONE;
+  constexpr int NZ = NA + V2, NP = P::N, WS = NP + (PPO ? PPO_WS_STATS : 0);
   __shared__ BwdSmemT<NA, KIND, LOSS> sm;
   extern __shared__ float s_rows[];    // [BWD_AG][K][2]: (a_r, ds_r) of the valid rows; a float2 array
                                        // would round every kernel's static shared memory in this file up to 16 B
@@ -653,7 +683,7 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
   for (int k = 0; k < GSM_OBS_DIM; k++) { gwe[k] = 0.f; gwn[k] = 0.f; }
 #pragma unroll
   for (int a = 0; a < NZ; a++) { ghe[a] = 0.f; ghg[a] = 0.f; }
-  if constexpr (LOSS) { if (tid < PPO_ROW_STATS) sm.stacc[tid] = 0.f; }
+  if constexpr (PPO) { if (tid < PPO_ROW_STATS) sm.stacc[tid] = 0.f; }
   __syncthreads();
 
   for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {   // block-uniform
@@ -678,14 +708,14 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
       const int act = KIND == HEAD_CAT ? (int)p.actions[src] : 0;
       const float lp = row_logp<NA>(z, act, zm, se);
       float dlp = 0.f, dent = 0.f, dvl[V2];
-      if constexpr (!LOSS) { dlp = p.d_logp ? p.d_logp[i] : 0.f; dent = p.d_entropy ? p.d_entropy[i] : 0.f; }
+      if constexpr (!PPO) { dlp = p.d_logp ? p.d_logp[i] : 0.f; dent = p.d_entropy ? p.d_entropy[i] : 0.f; }
       const float lse = zm + logf(se), inv_se = 1.f / se;
       float pr[NA], ent = 0.f;
 #pragma unroll
       for (int a = 0; a < NA; a++) { pr[a] = expf(z[a] - zm) * inv_se; ent = fmaf(pr[a], z[a] - zm, ent); }
       ent = logf(se) - ent;
       // the categorical loss: lp and ent are evaluate's (same row_logp, same entropy chain)
-      if constexpr (LOSS && KIND == HEAD_CAT) ppo_seeds(p, src, lp, ent, z + NA, dlp, dent, dvl, sm.st[tid]);
+      if constexpr (PPO && KIND == HEAD_CAT) ppo_seeds<KIND, LOSS>(p, src, lp, ent, z + NA, dlp, dent, dvl, sm.st[tid]);
       // an action outside [0, NA) has no one-hot: its NaN logp poisons the gradient it feeds
       const float bad = (dlp != 0.f && lp != lp) ? __int_as_float(0x7fc00000) : 0.f;
       float dz[NZ];
@@ -699,7 +729,7 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
         const float ls0 = W[P::LS], ls1 = W[P::LS + 1];
         float d0, d1;
         const float glp = gauss_logp(p.actions[src * GD], p.actions[src * GD + 1], z[0], z[1], ls0, ls1, d0, d1);
-        if constexpr (LOSS) ppo_seeds(p, src, glp, gauss_entropy(ls0, ls1), z + NA, dlp, dent, dvl, sm.st[tid]);
+        if constexpr (PPO) ppo_seeds<KIND, LOSS>(p, src, glp, gauss_entropy(ls0, ls1), z + NA, dlp, dent, dvl, sm.st[tid]);
         const bool use = dlp != 0.f;
         const float gbad = (use && glp != glp) ? __int_as_float(0x7fc00000) : 0.f;
         dz[0] = use ? dlp * d0 * expf(-ls0) + gbad : 0.f;
@@ -709,7 +739,7 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
       }
 #pragma unroll
       for (int v = 0; v < V2; v++) {
-        if constexpr (LOSS) dz[NA + v] = dvl[v];
+        if constexpr (PPO) dz[NA + v] = dvl[v];
         else dz[NA + v] = p.d_values ? p.d_values[i * V2 + v] : 0.f;
       }
       float dsum = 0.f;
@@ -795,7 +825,7 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
         else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) gsc += sm.dls[ag][j - NZ]; }
       }
     }
-    if constexpr (LOSS) {                // the tile's statistics, in row order
+    if constexpr (PPO) {                 // the tile's statistics, in row order
       if (tid < PPO_ROW_STATS) {
         float acc = sm.stacc[tid];
         for (int ag = 0; ag < nag; ag++) acc += sm.st[ag][tid];
@@ -818,7 +848,7 @@ __global__ void __launch_bounds__(BWD_AG) backward_kernel(const __grid_constant_
   if (j < NZ) out[j < NA ? P::HB + j : P::VB + (j - NA)] = gsc;
   else if (j == H - 1) out[P::AB] = gsc;
   else if constexpr (KIND == HEAD_GAUSS) { if (j < NZ + GD) out[P::LS + (j - NZ)] = gsc; }
-  if constexpr (LOSS) { if (j < PPO_WS_STATS) out[NP + j] = j < PPO_ROW_STATS ? sm.stacc[j] : 0.f; }
+  if constexpr (PPO) { if (j < PPO_WS_STATS) out[NP + j] = j < PPO_ROW_STATS ? sm.stacc[j] : 0.f; }
 }
 
 // grad[k] = sum of the G partials in a fixed order: warp w sums partials w, w + 8, ... (lane = k),
@@ -843,7 +873,7 @@ __global__ void __launch_bounds__(256) policy_grad_reduce_kernel(const float* __
   }
 }
 
-// backward_kernel<..., true>'s partials: blocks 0 .. ceil(NP / 32) - 1 reduce the gradient exactly as
+// the loss modes' backward_kernel partials: blocks 0 .. ceil(NP / 32) - 1 reduce the gradient exactly as
 // policy_grad_reduce_kernel does (partials of stride NP + PPO_WS_STATS); the last block reduces the
 // statistics in the same order, then lanes 0..6 write their means over the n rows and lane 0 adds
 // L = L_pi + c_v (L_V reward + L_V cost) - c_e entropy.  Counts (the clip fraction) are exact in fp32
@@ -959,12 +989,12 @@ template <int KIND> static int launch_evaluate(const EvalArgs<KIND>& a, int n_ac
 }
 
 // the backward kernel, then the reduction of its G partials: the gradient (and, with the loss, the statistics)
-template <int NA, int KIND, bool LOSS>
+template <int NA, int KIND, int LOSS>
 static int launch_backward(BwdArgs<KIND, LOSS> a, float* grad, float* stats, cudaStream_t st) {
   constexpr int NP = PV<NA, KIND>::N;
   const int64_t G = bwd_blocks(a.n_rows);
   a.n_tiles = (a.n_rows + BWD_AG - 1) / BWD_AG;
-  if constexpr (LOSS) a.inv_n = 1.f / (float)a.n_rows;
+  if constexpr (LOSS != LOSS_NONE) a.inv_n = 1.f / (float)a.n_rows;
   const size_t dyn = 2 * sizeof(float) * BWD_AG * (size_t)a.K;
   if (sizeof(BwdSmemT<NA, KIND, LOSS>) + dyn > 48 * 1024) {      // large max_nbrs: opt in to more shared memory
     const cudaError_t e = cudaFuncSetAttribute(backward_kernel<NA, KIND, LOSS>,
@@ -975,7 +1005,7 @@ static int launch_backward(BwdArgs<KIND, LOSS> a, float* grad, float* stats, cud
     }
   }
   backward_kernel<NA, KIND, LOSS><<<(unsigned)G, BWD_AG, dyn, st>>>(a);
-  if constexpr (LOSS)
+  if constexpr (LOSS != LOSS_NONE)
     ppo_reduce_kernel<<<(NP + 31) / 32 + 1, 256, 0, st>>>(a.ws, (int)G, NP, grad, stats, (float)a.n_rows,
                                                            a.value_coef, a.entropy_coef);
   else
@@ -1141,27 +1171,33 @@ template <int KIND, bool LOSS> int64_t workspace_t(int64_t n_rows, int n_actions
   });
 }
 
-// gsm_policy_backward(_gauss) (LOSS = false: d_logp, d_entropy and d_values are the seeds) and
-// gsm_ppo_backward(_gauss) (LOSS: `loss` computes the seeds); ws_msg: the error for a short workspace
-template <int KIND, bool LOSS, class IO>
-int backward_t(const IO* io, const gsm_ppo_loss_io* loss, const float* d_logp, const float* d_entropy,
-               const float* d_values, float* grad, void* workspace, size_t workspace_bytes, int device, void* stream,
-               const char* who, const char* ws_msg) {
+// gsm_policy_backward(_gauss) (LOSS_NONE: d_logp, d_entropy and d_values are the seeds),
+// gsm_ppo_backward(_gauss) (LOSS_PPO: `loss` computes the seeds) and gsm_ppo_backward_normalized(_gauss)
+// (LOSS_PPO_VNORM: on targets normalised with value_affine); ws_msg: the error for a short workspace
+template <int KIND, int LOSS, class IO>
+int backward_t(const IO* io, const gsm_ppo_loss_io* loss, const float* value_affine, const float* d_logp,
+               const float* d_entropy, const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
+               int device, void* stream, const char* who, const char* ws_msg) {
+  constexpr bool PPO = LOSS != gsm::LOSS_NONE;
   if (const int st = check_eval_io(io, who)) return st;
-  if constexpr (LOSS) { if (const int st = check_loss_io(loss, who)) return st; }
+  if constexpr (PPO) { if (const int st = check_loss_io(loss, who)) return st; }
+  if constexpr (LOSS == gsm::LOSS_PPO_VNORM) {
+    if (!value_affine) return pfailf(GSM_ERR_INVALID_ARG, who, "value_affine is required");
+  }
   if (!grad) return pfailf(GSM_ERR_INVALID_ARG, who, "grad is required");
-  const int64_t need = workspace_t<KIND, LOSS>(io->n_rows, n_actions(io), who);
+  const int64_t need = workspace_t<KIND, PPO>(io->n_rows, n_actions(io), who);
   if (need > 0 && (!workspace || workspace_bytes < (size_t)need)) return pfailf(GSM_ERR_INVALID_ARG, who, ws_msg);
   if (io->n_rows == 0) return GSM_OK;
   gsm::BwdArgs<KIND, LOSS> a{};
   static_cast<gsm::EvalArgs<KIND>&>(a) = eval_args<KIND>(io);
   float* stats = nullptr;
-  if constexpr (LOSS) {
+  if constexpr (PPO) {
     a.old_logp = loss->old_logp; a.old_values = loss->old_values; a.returns = loss->returns; a.adv = loss->advantages;
     a.adv_moments = loss->adv_moments; a.lagrange = loss->lagrange;
     a.clip = loss->clip; a.value_clip = loss->value_clip;
     a.value_coef = loss->value_coef; a.entropy_coef = loss->entropy_coef;
     stats = loss->stats;
+    if constexpr (LOSS == gsm::LOSS_PPO_VNORM) a.value_affine = value_affine;
   } else {
     a.d_logp = d_logp; a.d_entropy = d_entropy; a.d_values = d_values;
   }
@@ -1171,6 +1207,30 @@ int backward_t(const IO* io, const gsm_ppo_loss_io* loss, const float* d_logp, c
       return gsm::launch_backward<decltype(na)::value, KIND, LOSS>(a, grad, stats, (cudaStream_t)stream);
     });
   });
+}
+
+// gsm_gae (NORM = false) and gsm_gae_normalized (NORM: the values are denormalised with `affine`)
+template <bool NORM>
+int gae_t(const float* reward, const float* cost, const float* values, const uint8_t* done, int32_t n_steps,
+          int64_t n_rows, int64_t slot_rows, float gamma, float lam, float* returns, float* advantages,
+          const float* affine, int device, void* stream, const char* who) {
+  if (!reward || !cost || !values || !done || !returns)
+    return pfailf(GSM_ERR_INVALID_ARG, who, "reward, cost, values, done and returns are required");
+  if constexpr (NORM) { if (!affine) return pfailf(GSM_ERR_INVALID_ARG, who, "value_affine is required"); }
+  if (n_steps < 1 || n_rows < 0 || slot_rows < n_rows) return pfailf(GSM_ERR_INVALID_ARG, who, "bad sizes");
+  if (const int ds = check_device(device, who)) return ds;
+  if (n_rows == 0) return GSM_OK;
+  DevGuard guard(device);
+  if (!guard.ok) return pfailf(GSM_ERR_CUDA, who, "cudaSetDevice failed");
+  gsm::GaeArgs<NORM> p{};
+  static_cast<gsm::GaeParams&>(p) = {reward, cost, values, done, returns, advantages, n_rows, slot_rows, n_steps,
+                                     gamma, lam};
+  if constexpr (NORM) p.affine = affine;
+  const int64_t threads = n_rows * GSM_POLICY_VALUE_HEADS;
+  gsm::gae_kernel<NORM><<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return pfail(GSM_ERR_CUDA, cudaGetErrorString(e));
+  return GSM_OK;
 }
 }  // namespace
 
@@ -1206,7 +1266,7 @@ int64_t gsm_policy_backward_workspace_gauss(int64_t n_rows) {
 int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const float* d_entropy,
                         const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                         int device, void* stream) {
-  return backward_t<gsm::HEAD_CAT, false>(io, nullptr, d_logp, d_entropy, d_values, grad, workspace, workspace_bytes,
+  return backward_t<gsm::HEAD_CAT, gsm::LOSS_NONE>(io, nullptr, nullptr, d_logp, d_entropy, d_values, grad, workspace, workspace_bytes,
                                           device, stream, "gsm_policy_backward",
                                           "workspace smaller than gsm_policy_backward_workspace(n_rows, n_actions)");
 }
@@ -1214,7 +1274,7 @@ int gsm_policy_backward(const gsm_policy_eval_io* io, const float* d_logp, const
 int gsm_policy_backward_gauss(const gsm_policy_gauss_eval_io* io, const float* d_logp, const float* d_entropy,
                               const float* d_values, float* grad, void* workspace, size_t workspace_bytes,
                               int device, void* stream) {
-  return backward_t<gsm::HEAD_GAUSS, false>(io, nullptr, d_logp, d_entropy, d_values, grad, workspace,
+  return backward_t<gsm::HEAD_GAUSS, gsm::LOSS_NONE>(io, nullptr, nullptr, d_logp, d_entropy, d_values, grad, workspace,
                                             workspace_bytes, device, stream, "gsm_policy_backward_gauss",
                                             "workspace smaller than gsm_policy_backward_workspace_gauss(n_rows)");
 }
@@ -1229,14 +1289,14 @@ int64_t gsm_ppo_backward_workspace_gauss(int64_t n_rows) {
 
 int gsm_ppo_backward(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss, float* grad, void* workspace,
                      size_t workspace_bytes, int device, void* stream) {
-  return backward_t<gsm::HEAD_CAT, true>(io, loss, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes, device,
+  return backward_t<gsm::HEAD_CAT, gsm::LOSS_PPO>(io, loss, nullptr, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes, device,
                                          stream, "gsm_ppo_backward",
                                          "workspace smaller than the ppo backward workspace for n_rows");
 }
 
 int gsm_ppo_backward_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss, float* grad,
                            void* workspace, size_t workspace_bytes, int device, void* stream) {
-  return backward_t<gsm::HEAD_GAUSS, true>(io, loss, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes,
+  return backward_t<gsm::HEAD_GAUSS, gsm::LOSS_PPO>(io, loss, nullptr, nullptr, nullptr, nullptr, grad, workspace, workspace_bytes,
                                            device, stream, "gsm_ppo_backward_gauss",
                                            "workspace smaller than the ppo backward workspace for n_rows");
 }
@@ -1262,19 +1322,32 @@ int gsm_adam_step(float* params, const float* grad, float* m, float* v, int32_t*
 int gsm_gae(const float* reward, const float* cost, const float* values, const uint8_t* done, int32_t n_steps,
             int64_t n_rows, int64_t slot_rows, float gamma, float lam, float* returns, float* advantages,
             int device, void* stream) {
-  if (!reward || !cost || !values || !done || !returns)
-    return pfail(GSM_ERR_INVALID_ARG, "gsm_gae: reward, cost, values, done and returns are required");
-  if (n_steps < 1 || n_rows < 0 || slot_rows < n_rows) return pfail(GSM_ERR_INVALID_ARG, "gsm_gae: bad sizes");
-  if (const int ds = check_device(device, "gsm_gae")) return ds;
-  if (n_rows == 0) return GSM_OK;
-  DevGuard guard(device);
-  if (!guard.ok) return pfail(GSM_ERR_CUDA, "gsm_gae: cudaSetDevice failed");
-  gsm::GaeParams p{reward, cost, values, done, returns, advantages, n_rows, slot_rows, n_steps, gamma, lam};
-  const int64_t threads = n_rows * GSM_POLICY_VALUE_HEADS;
-  gsm::gae_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p);
-  const cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return pfail(GSM_ERR_CUDA, cudaGetErrorString(e));
-  return GSM_OK;
+  return gae_t<false>(reward, cost, values, done, n_steps, n_rows, slot_rows, gamma, lam, returns, advantages,
+                      nullptr, device, stream, "gsm_gae");
+}
+
+int gsm_gae_normalized(const float* reward, const float* cost, const float* values, const uint8_t* done,
+                       int32_t n_steps, int64_t n_rows, int64_t slot_rows, float gamma, float lam, float* returns,
+                       float* advantages, const float* value_affine, int device, void* stream) {
+  return gae_t<true>(reward, cost, values, done, n_steps, n_rows, slot_rows, gamma, lam, returns, advantages,
+                     value_affine, device, stream, "gsm_gae_normalized");
+}
+
+int gsm_ppo_backward_normalized(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss, const float* value_affine,
+                                float* grad, void* workspace, size_t workspace_bytes, int device, void* stream) {
+  return backward_t<gsm::HEAD_CAT, gsm::LOSS_PPO_VNORM>(io, loss, value_affine, nullptr, nullptr, nullptr, grad,
+                                                        workspace, workspace_bytes, device, stream,
+                                                        "gsm_ppo_backward_normalized",
+                                                        "workspace smaller than the ppo backward workspace for n_rows");
+}
+
+int gsm_ppo_backward_normalized_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss,
+                                      const float* value_affine, float* grad, void* workspace,
+                                      size_t workspace_bytes, int device, void* stream) {
+  return backward_t<gsm::HEAD_GAUSS, gsm::LOSS_PPO_VNORM>(io, loss, value_affine, nullptr, nullptr, nullptr, grad,
+                                                          workspace, workspace_bytes, device, stream,
+                                                          "gsm_ppo_backward_normalized_gauss",
+                                                          "workspace smaller than the ppo backward workspace for n_rows");
 }
 
 }  // extern "C"

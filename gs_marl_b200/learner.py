@@ -18,15 +18,119 @@ clipping and Adam; lambda follows the team episode cost against a limit.
 
 Per minibatch: `gsm_ppo_backward(_gauss)` (the §12 backward with the loss seeds computed in its phase A,
 no separate forward) and `gsm_adam_step` (clip_grad_norm_ + Adam in one launch): three kernels.
+
+With a value normaliser (SPEC.md §15, the lineage's `use_valuenorm`) the critics are trained on, and output,
+normalised values:
+
+    vnorm = ValueNorm(device, **presets.UNVERIFIED_VALUE_NORM)
+    trainer = LagrangianPPO(actor, **presets.UNVERIFIED_PPO_LAG, value_norm=vnorm, seed=0)
+    ...
+        buf.compute_returns(gamma, lam, value_norm=vnorm)   # denormalises the collected values
+        stats = trainer.update(buf)                         # one normaliser pass per epoch
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import torch
 
 from . import abi
 from .policy import GaussianGraphActor, GraphAttentionActor, _check, _eval_io
+
+class ValueNorm:
+    """The lineage's ValueNorm (utils/popart.py), one independent normaliser per critic head (SPEC.md §15).
+    Owns `state` (fp64 [2, 3]: running mean, running mean of squares, debiasing term per head, from 0) and
+    `affine` (fp32 [2, 2]: (mu_h, sigma_h) of the state), both on `device`.  Every hyper-parameter is a
+    required keyword (`presets.UNVERIFIED_VALUE_NORM` holds the lineage's values)."""
+
+    def __init__(self, device, *, beta, epsilon, var_floor):
+        if not (0 <= beta < 1) or not (epsilon > 0 and var_floor > 0):
+            raise ValueError("beta must lie in [0, 1), epsilon and var_floor must be > 0")
+        self.beta, self.epsilon, self.var_floor = float(beta), float(epsilon), float(var_floor)
+        dev = torch.device(device)
+        if dev.type != "cuda":
+            raise abi.GsmError("ValueNorm lives on a CUDA device: gs_marl_b200 has no CPU fallback")
+        self.device = dev if dev.index is not None else torch.device("cuda", torch.cuda.current_device())
+        self.state = torch.zeros(2, 3, dtype=torch.float64, device=self.device)
+        # affine snapshots [n_mini_batch + 1, 2, 2] of the last update; `affine` is its last entry
+        self._snaps = torch.tensor([[0.0, math.sqrt(self.var_floor)]] * 2, dtype=torch.float32,
+                                   device=self.device)[None]
+        self._ws = None
+
+    @property
+    def affine(self) -> torch.Tensor:
+        """(mu_h, sigma_h) [2, 2] of the current state; a view that the next `update` rewrites."""
+        return self._snaps[-1]
+
+    def mean_std(self):
+        """(mu [2], sigma [2]), fp32, per head (0: reward, 1: cost)."""
+        return self.affine[:, 0], self.affine[:, 1]
+
+    def normalize(self, x: torch.Tensor) -> torch.Tensor:
+        """(x - mu_h) / sigma_h over x [..., 2], fp32: the rounding of the normalised backward's targets."""
+        mu, sd = self.mean_std()
+        return (x.float() - mu) / sd
+
+    def denormalize(self, v: torch.Tensor) -> torch.Tensor:
+        """fmaf(v, sigma_h, mu_h) over v [..., 2] (critic outputs to raw units): the rounding of
+        gsm_gae_normalized.  The product is exact in fp64; the sum is rounded to odd there, which makes the
+        final rounding to fp32 the single rounding of fmaf."""
+        mu, sd = (t.double() for t in self.mean_std())
+        p = v.double() * sd
+        s = p + mu
+        bp = s - mu
+        err = (p - bp) + (mu - (s - bp))                      # s + err == p + mu exactly (TwoSum)
+        even = (s.view(torch.int64) & 1) == 0
+        toward = torch.where(err > 0, torch.full_like(s, math.inf), torch.full_like(s, -math.inf))
+        return torch.where((err != 0) & even, torch.nextafter(s, toward), s).float()
+
+    def update(self, returns: torch.Tensor, rows: torch.Tensor, num_mini_batch: int) -> torch.Tensor:
+        """One epoch of updates: minibatch b = rows[b mb:(b + 1) mb], mb = len(rows) // num_mini_batch (the
+        remainder is left out), in order.  Returns the affine snapshots [num_mini_batch, 2, 2], snapshot b
+        taken after minibatch b's update; they stay valid until the next call.  Two launches, no host sync."""
+        nmb = int(num_mini_batch)
+        if returns.dtype != torch.float32 or returns.shape[-1] != 2 or not returns.is_contiguous():
+            raise ValueError("returns must be a contiguous float32 [..., 2] tensor")
+        if rows.dtype != torch.int64 or rows.dim() != 1 or not rows.is_contiguous():
+            raise ValueError("rows must be a contiguous int64 vector")
+        if returns.device != self.device or rows.device != self.device:
+            raise ValueError(f"returns and rows must be on {self.device}")
+        if nmb < 1 or rows.numel() < nmb:
+            raise ValueError(f"{rows.numel()} rows cannot make {nmb} minibatches")
+        mb = rows.numel() // nmb
+        lib = abi.load_library()
+        if self._snaps.shape[0] != nmb + 1:
+            snaps = torch.empty(nmb + 1, 2, 2, dtype=torch.float32, device=self.device)
+            snaps[-1] = self.affine
+            self._snaps = snaps
+        need = lib.gsm_value_norm_update_workspace(mb, nmb)
+        if need < 0:
+            raise ValueError(f"gsm_value_norm_update_workspace({mb}, {nmb}) = {need}")
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        io = abi.GsmValueNormIO()
+        io.struct_size = C.sizeof(abi.GsmValueNormIO)
+        io.state, io.affine = self.state.data_ptr(), self._snaps.data_ptr()
+        io.returns, io.rows = returns.data_ptr(), rows.data_ptr()
+        io.mb, io.n_mini_batch = mb, nmb
+        io.beta, io.epsilon, io.var_floor = self.beta, self.epsilon, self.var_floor
+        st = lib.gsm_value_norm_update(C.byref(io), self._ws.data_ptr(), self._ws.numel(), self.device.index or 0,
+                                       C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
+        if st != 0:
+            raise abi.GsmError(f"gsm_value_norm_update: {lib.gsm_status_string(st).decode()}")
+        return self._snaps[:nmb]
+
+    def state_dict(self) -> dict:
+        return {"state": self.state.clone(), "affine": self.affine.clone()}
+
+    def load_state_dict(self, sd: dict):
+        for k, shape, dt in (("state", (2, 3), torch.float64), ("affine", (2, 2), torch.float32)):
+            if tuple(sd[k].shape) != shape or sd[k].dtype != dt:
+                raise ValueError(f"value_norm {k}: {tuple(sd[k].shape)} {sd[k].dtype}, expected {shape} {dt}")
+        self.state.copy_(sd["state"])
+        self.affine.copy_(sd["affine"])
+
 
 # the columns of `update`'s result: the GSM_PPO_STAT_FIELDS loss statistics, then the gradient norm
 STAT_FIELDS = ("policy_loss", "value_loss_reward", "value_loss_cost", "entropy", "ratio", "clip_fraction",
@@ -36,10 +140,15 @@ STAT_FIELDS = ("policy_loss", "value_loss_reward", "value_loss_cost", "entropy",
 class LagrangianPPO:
     """Owns the flat parameter vector (parameters_to_vector order), Adam's m, v and step, and lambda, all on
     the actor's device.  Every hyper-parameter is a required keyword (`presets.UNVERIFIED_PPO_LAG` holds
-    lineage-typical values); the library has no defaults."""
+    lineage-typical values); the library has no defaults.
+
+    value_norm: a `ValueNorm` (SPEC.md §15) or None.  With one, each epoch first updates it once per minibatch
+    and each minibatch's value loss regresses the critics on normalize(R) under its snapshot; the buffer's
+    returns must come from `compute_returns(..., value_norm=...)`.  The value-loss statistics are then in
+    normalised units."""
 
     def __init__(self, actor, *, clip, value_clip, value_coef, entropy_coef, lr, betas, eps, max_grad_norm,
-                 ppo_epoch, num_mini_batch, lagrangian_lr, cost_limit, lagrangian_init=0.0, seed):
+                 ppo_epoch, num_mini_batch, lagrangian_lr, cost_limit, lagrangian_init=0.0, seed, value_norm=None):
         if not isinstance(actor, (GraphAttentionActor, GaussianGraphActor)):
             raise TypeError("LagrangianPPO trains a GraphAttentionActor or a GaussianGraphActor")
         self._head = actor._desc
@@ -76,6 +185,9 @@ class LagrangianPPO:
         self.generator = torch.Generator(device=dev)
         self.generator.manual_seed(int(seed))
         self._ws = None
+        if value_norm is not None and (not isinstance(value_norm, ValueNorm) or value_norm.device != dev):
+            raise ValueError(f"value_norm must be a ValueNorm on {dev}")
+        self.value_norm = value_norm
 
     # ---- the pieces of one update -------------------------------------------------------------------
     def inputs(self, buf):
@@ -107,9 +219,11 @@ class LagrangianPPO:
         sd = (a - mu).square().mean(0).sqrt()
         self.adv_moments.copy_(torch.stack([mu[0], sd[0], mu[1], sd[1]]).float())
 
-    def backward(self, x, rows, stats):
+    def backward(self, x, rows, stats, value_affine=None):
         """gsm_ppo_backward(_gauss) over the source rows `rows` (int64 [n], or None for all of x): self.grad =
-        dL/dparams of the §14 loss at self.params, stats [8] = its statistics.  Two launches, no host sync."""
+        dL/dparams of the §14 loss at self.params, stats [8] = its statistics.  With value_affine (a device
+        fp32 [2, 2] (mu_h, sigma_h)), gsm_ppo_backward_normalized(_gauss): the value targets are normalised
+        with it (§15).  Two launches, no host sync."""
         lib = abi.load_library()
         dev = self.device
         n = rows.numel() if rows is not None else x["cnt"].numel()
@@ -125,9 +239,14 @@ class LagrangianPPO:
                                                        stats.data_ptr())
         loss.clip, loss.value_clip = self.clip, self.value_clip
         loss.value_coef, loss.entropy_coef = self.value_coef, self.entropy_coef
-        _check(lib, getattr(lib, self._head.ppo_backward)(C.byref(io), C.byref(loss), self.grad.data_ptr(),
-                                                          self._ws.data_ptr(), self._ws.numel(), dev.index or 0,
-                                                          self._stream()))
+        if value_affine is None:
+            _check(lib, getattr(lib, self._head.ppo_backward)(C.byref(io), C.byref(loss), self.grad.data_ptr(),
+                                                              self._ws.data_ptr(), self._ws.numel(), dev.index or 0,
+                                                              self._stream()))
+        else:
+            _check(lib, getattr(lib, self._head.ppo_backward_normalized)(
+                C.byref(io), C.byref(loss), value_affine.data_ptr(), self.grad.data_ptr(), self._ws.data_ptr(),
+                self._ws.numel(), dev.index or 0, self._stream()))
 
     def adam_step(self, grad_norm):
         """gsm_adam_step on (self.params, self.grad, self.m, self.v, self.step); grad_norm: a device float [1]."""
@@ -137,9 +256,9 @@ class LagrangianPPO:
                                       self.betas[0], self.betas[1], self.eps, self.max_grad_norm,
                                       grad_norm.data_ptr(), self.device.index or 0, self._stream()))
 
-    def minibatch_step(self, x, rows, stats):
+    def minibatch_step(self, x, rows, stats, value_affine=None):
         """backward then adam_step; stats [9]: the loss statistics, then the gradient norm.  Three launches."""
-        self.backward(x, rows, stats)
+        self.backward(x, rows, stats, value_affine)
         self.adam_step(stats[abi.GSM_PPO_STAT_FIELDS:])
 
     def _stream(self):
@@ -149,7 +268,8 @@ class LagrangianPPO:
     def update(self, buf) -> torch.Tensor:
         """ppo_epoch x num_mini_batch minibatch steps over the buffer filled by collect + compute_returns.
         Minibatches: a seeded device permutation of the T * n_envs * N rows per epoch, cut into
-        num_mini_batch parts of rows // num_mini_batch (the remainder is left out, as in the lineage).
+        num_mini_batch parts of rows // num_mini_batch (the remainder is left out, as in the lineage).  With a
+        value normaliser, one `value_norm.update` over the epoch's permutation precedes its minibatches.
         Returns stats [ppo_epoch * num_mini_batch, 9] (STAT_FIELDS) on the device.  No host sync between the
         first and the last launch; call `actor.pack()` afterwards for the collect kernels."""
         x = self.inputs(buf)
@@ -165,9 +285,15 @@ class LagrangianPPO:
             k = 0
             for _ in range(self.ppo_epoch):
                 perm = torch.randperm(n, generator=self.generator, device=dev)
-                for b in range(self.num_mini_batch):
-                    self.minibatch_step(x, perm[b * mb:(b + 1) * mb], out[k])
-                    k += 1
+                if self.value_norm is None:
+                    for b in range(self.num_mini_batch):
+                        self.minibatch_step(x, perm[b * mb:(b + 1) * mb], out[k])
+                        k += 1
+                else:
+                    snaps = self.value_norm.update(x["ret"], perm, self.num_mini_batch)
+                    for b in range(self.num_mini_batch):
+                        self.minibatch_step(x, perm[b * mb:(b + 1) * mb], out[k], snaps[b])
+                        k += 1
             self.write_back()
         return out
 
@@ -193,11 +319,16 @@ class LagrangianPPO:
 
     # ---- checkpoints ----------------------------------------------------------------------------------
     def state_dict(self) -> dict:
-        return {"params": self.params.clone(), "m": self.m.clone(), "v": self.v.clone(), "step": self.step.clone(),
-                "lagrange": self.lagrange.clone(), "adv_moments": self.adv_moments.clone(),
-                "generator": self.generator.get_state()}
+        sd = {"params": self.params.clone(), "m": self.m.clone(), "v": self.v.clone(), "step": self.step.clone(),
+              "lagrange": self.lagrange.clone(), "adv_moments": self.adv_moments.clone(),
+              "generator": self.generator.get_state()}
+        if self.value_norm is not None:
+            sd["value_norm"] = self.value_norm.state_dict()
+        return sd
 
     def load_state_dict(self, sd: dict):
+        if ("value_norm" in sd) != (self.value_norm is not None):
+            raise ValueError("the checkpoint and this trainer disagree on having a value normaliser")
         for k in ("params", "m", "v", "step", "lagrange", "adv_moments"):
             dst = getattr(self, k)
             if tuple(sd[k].shape) != tuple(dst.shape) or sd[k].dtype != dst.dtype:
@@ -205,4 +336,6 @@ class LagrangianPPO:
             dst.copy_(sd[k])
         if "generator" in sd:
             self.generator.set_state(sd["generator"])
+        if self.value_norm is not None:
+            self.value_norm.load_state_dict(sd["value_norm"])
         self.write_back()

@@ -57,6 +57,7 @@ class _Head:
     workspace: str
     ppo_backward: str
     ppo_workspace: str
+    ppo_backward_normalized: str
     ws_args: tuple
     eval_io: type
     head_field: str
@@ -66,11 +67,13 @@ class _Head:
 
 
 _CAT_HEADS = {a: _Head("gsm_policy_act", abi.GsmPolicyIO, "logits", "gsm_policy_evaluate", "gsm_policy_backward",
-                       "gsm_policy_backward_workspace", "gsm_ppo_backward", "gsm_ppo_backward_workspace", (a,),
+                       "gsm_policy_backward_workspace", "gsm_ppo_backward", "gsm_ppo_backward_workspace",
+                       "gsm_ppo_backward_normalized", (a,),
                        abi.GsmPolicyEvalIO, "n_actions", a, torch.int32, ()) for a in (5, 9)}
 _GAUSS_HEAD = _Head("gsm_policy_act_gauss", abi.GsmPolicyGaussIO, "mean", "gsm_policy_evaluate_gauss",
                     "gsm_policy_backward_gauss", "gsm_policy_backward_workspace_gauss", "gsm_ppo_backward_gauss",
-                    "gsm_ppo_backward_workspace_gauss", (), abi.GsmPolicyGaussEvalIO, "action_dim",
+                    "gsm_ppo_backward_workspace_gauss", "gsm_ppo_backward_normalized_gauss", (),
+                    abi.GsmPolicyGaussEvalIO, "action_dim",
                     abi.GSM_POLICY_GAUSS_DIM, torch.float32, (abi.GSM_POLICY_GAUSS_DIM,))
 
 

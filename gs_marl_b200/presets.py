@@ -55,3 +55,7 @@ UNVERIFIED_PPO_LAG = dict(
     lagrangian_lr=1e-2,
     cost_limit=0.0,
 )
+
+# The lineage's value normaliser (utils/popart.py / ValueNorm: beta 0.99999, epsilon 1e-5, a variance floor of
+# 1e-2); `learner.ValueNorm` takes each as a required keyword.
+UNVERIFIED_VALUE_NORM = dict(beta=0.99999, epsilon=1e-5, var_floor=1e-2)

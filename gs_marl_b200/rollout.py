@@ -94,21 +94,29 @@ class GraphRolloutBuffer:
             sh.lib.gsm_reset(sh._h, sh._seed, None, 1, C.byref(self._io_reset[j]), st)))
         self.step = 0
 
-    def compute_returns(self, gamma: float = 0.99, gae_lambda: float = 0.95):
+    def compute_returns(self, gamma: float = 0.99, gae_lambda: float = 0.95, value_norm=None):
         """buffer.compute_returns + compute_cost_returns of the lineage (GAE, SPEC.md §11), one kernel
         for both critics: fills `returns` and `advantages` [T, n_envs, N, 2] from reward / cost / done
-        and `values` (slot T must hold the bootstrap prediction for the last observation)."""
+        and `values` (slot T must hold the bootstrap prediction for the last observation).  With a
+        `learner.ValueNorm` (SPEC.md §15) the values are the critics' normalised outputs: every one is
+        denormalised with the normaliser's current affine first (`gsm_gae_normalized`), so returns and
+        advantages are in raw units."""
         d, e = self.data, self.env
         for k in ("returns", "advantages"):
             if k not in d:
                 d[k] = torch.zeros_like(d["values"][:-1])
         lib = abi.load_library()
         rows = d["reward"][0].numel()
+        args = (d["reward"].data_ptr(), d["cost"].data_ptr(), d["values"].data_ptr(), d["done"].data_ptr(), self.T,
+                rows, rows, float(gamma), float(gae_lambda), d["returns"].data_ptr(), d["advantages"].data_ptr())
         with torch.cuda.device(e.device):
-            st = lib.gsm_gae(d["reward"].data_ptr(), d["cost"].data_ptr(), d["values"].data_ptr(),
-                             d["done"].data_ptr(), self.T, rows, rows, float(gamma), float(gae_lambda),
-                             d["returns"].data_ptr(), d["advantages"].data_ptr(), e.device.index or 0,
-                             C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream))
+            stream = C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)
+            if value_norm is None:
+                st = lib.gsm_gae(*args, e.device.index or 0, stream)
+            else:
+                if value_norm.affine.device != d["values"].device:
+                    raise ValueError(f"value_norm must live on {d['values'].device}")
+                st = lib.gsm_gae_normalized(*args, value_norm.affine.data_ptr(), e.device.index or 0, stream)
         if st != 0:
             raise abi.GsmError(f"{lib.gsm_status_string(st).decode()}: {lib.gsm_policy_last_error().decode()}")
         return d["returns"], d["advantages"]

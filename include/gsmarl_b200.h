@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define GSM_ABI_VERSION 7
+#define GSM_ABI_VERSION 8
 
 #define GSM_OBS_DIM 6        /* vx, vy, px, py, target_dx, target_dy          (SPEC.md §6) */
 #define GSM_NBR_FEAT_DIM 6   /* dx, dy, dvx, dvy, dist, (real)entity_type     (SPEC.md §6) */
@@ -511,6 +511,60 @@ int gsm_collect_gauss(gsm_env* h, const gsm_policy_gauss_weights* w, int32_t n_s
 int gsm_gae(const float* reward, const float* cost, const float* values, const uint8_t* done,
             int32_t n_steps, int64_t n_rows, int64_t slot_rows, float gamma, float lam,
             float* returns, float* advantages, int device, void* stream);
+
+/* ---- value normalisation (SPEC.md §15): the lineage's ValueNorm (utils/popart.py), one per critic head ----
+ * The critics then output normalised values.  Per head h (0: reward, 1: cost) the state (m_h, s_h, d_h) is
+ * fp64 and starts at 0; the affine (mu_h, sigma_h), fp64 rounded to fp32, is
+ *   mu_h = m_h / max(d_h, epsilon);  sigma_h = sqrt(max(s_h / max(d_h, epsilon) - mu_h^2, var_floor))
+ * (a fresh normaliser: mu = 0, sigma = sqrt(var_floor)).  value_affine arguments are DEVICE float [2][2]
+ * (mu_0, sigma_0, mu_1, sigma_1). */
+
+/* gsm_gae with every V_h[t] (slot T included) denormalised first: V = fmaf(V, sigma_h, mu_h); returns and
+ * advantages are in raw units.  Errors as gsm_gae, plus GSM_ERR_INVALID_ARG for a NULL value_affine. */
+int gsm_gae_normalized(const float* reward, const float* cost, const float* values, const uint8_t* done,
+                       int32_t n_steps, int64_t n_rows, int64_t slot_rows, float gamma, float lam,
+                       float* returns, float* advantages, const float* value_affine, int device, void* stream);
+
+/* gsm_ppo_backward(_gauss) with the value loss on normalised targets: R_h -> (R_h - mu_h) / sigma_h (fp32)
+ * before the unchanged §14 value terms; old_values and the values stay in normalised units, and so does
+ * value_clip.  Workspace: gsm_ppo_backward_workspace(_gauss).  Errors as gsm_ppo_backward, plus
+ * GSM_ERR_INVALID_ARG for a NULL value_affine. */
+int gsm_ppo_backward_normalized(const gsm_policy_eval_io* io, const gsm_ppo_loss_io* loss,
+                                const float* value_affine, float* grad, void* workspace, size_t workspace_bytes,
+                                int device, void* stream);
+int gsm_ppo_backward_normalized_gauss(const gsm_policy_gauss_eval_io* io, const gsm_ppo_loss_io* loss,
+                                      const float* value_affine, float* grad, void* workspace,
+                                      size_t workspace_bytes, int device, void* stream);
+
+/* One epoch of normaliser updates, one per minibatch b = 0 .. n_mini_batch - 1 over the returns of its rows
+ * rows[b mb .. (b + 1) mb), in this order:
+ *   m_h = beta m_h + (1 - beta) mean(R_h);  s_h = beta s_h + (1 - beta) mean(R_h^2);  d_h = beta d_h + (1 - beta)
+ * (fp64, batch sums in a fixed order), then affine[b] = the affine of the updated state.  affine[n_mini_batch]
+ * and `state` end as the final affine and state.  Two launches, no atomics (bit-identical across calls,
+ * streams and devices), no host sync. */
+typedef struct gsm_value_norm_io {   /* DEVICE pointers */
+  uint32_t struct_size;          /* = sizeof(gsm_value_norm_io); checked                              */
+  int32_t reserved;              /* 0 */
+  double* state;                 /* [2][3] in/out: (m_h, s_h, d_h) per head                           */
+  float* affine;                 /* [n_mini_batch + 1][2][2] out                                      */
+  const float* returns;          /* [src_rows][2]  gsm_gae(_normalized) returns                       */
+  const int64_t* rows;           /* [n_mini_batch * mb] source rows, each in [0, src_rows)            */
+  int64_t mb;                    /* rows per minibatch >= 1                                           */
+  int64_t n_mini_batch;          /* >= 1                                                              */
+  double beta;                   /* in [0, 1)                                                         */
+  double epsilon;                /* > 0                                                               */
+  double var_floor;              /* > 0                                                               */
+} gsm_value_norm_io;
+
+/* Workspace bytes gsm_value_norm_update needs (a function of mb and n_mini_batch only);
+ * GSM_ERR_INVALID_ARG for mb < 1 or n_mini_batch < 1. */
+int64_t gsm_value_norm_update_workspace(int64_t mb, int64_t n_mini_batch);
+
+/* GSM_ERR_ABI for a bad struct_size; GSM_ERR_INVALID_ARG for a missing pointer, mb or n_mini_batch < 1,
+ * beta outside [0, 1), epsilon <= 0, var_floor <= 0 or a workspace smaller than
+ * gsm_value_norm_update_workspace. */
+int gsm_value_norm_update(const gsm_value_norm_io* io, void* workspace, size_t workspace_bytes, int device,
+                          void* stream);
 
 /* ---- episode statistics (SPEC.md §13): the runner's per-episode logging over the buffer slots --------
  * Episode return, cost and length per agent row and per team, across calls: rollouts shorter or longer
